@@ -8,13 +8,16 @@ quantizator Linear at Lossless and at Medium.  One *step* = for q in (Lossless, 
 Encoder::encode over the batch, then Decoder::decode over the batch.  `value` counts every pixel
 once per encode+decode round trip: Mpixel/s = n_gpus * 2 * frames * 1920*1080 / step_time.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Timed with CUDA events on the launching stream after W warm-up steps, barrier + synchronize on
 both sides, max over ranks.  The working set (8.5 GB per plane set) is far larger than the 126 MB
 L2, so no flush is needed between iterations.  `e2e` is the same metric through the host-pointer
 C-ABI calls (pinned host buffers, H2D + D2H inside the timed region).  `--impl reference` times
 the CPU restatement of the reference (oracle/, all host threads) on a bounded sample.
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0's grids and decoded planes at both quantizers)
+as float32 .npy files: a fixed, seeded sample, so two builds run with the same arguments compare output for output.
 """
 import argparse
 import json
@@ -262,6 +265,31 @@ def oracle_parity(frames, encs, dec, ctx, n_check=64):
             "mismatches": bad, "checker": "oracle/hgi_oracle.c (grid bytes and decoded planes, every byte)"}
 
 
+DUMP_SEED, DUMP_PIXELS = 20261020, 1 << 20
+
+
+def dump_positions(n):
+    """What --dump-outputs keeps of a batch of n frames: one frame index, and DUMP_PIXELS flat (frame, y, x) indices
+    over the whole batch.  Seeded, so the same arguments give the same positions in every run and every build."""
+    import numpy as np
+    rng = np.random.default_rng(DUMP_SEED)
+    return int(rng.integers(n)), np.sort(rng.integers(0, n * H * W, DUMP_PIXELS))
+
+
+def dump_outputs(out_dir, outputs):
+    """`outputs`: name -> (n, H, W) uint8 CUDA tensor.  Writes <name>_frame.npy (the chosen frame in full) and
+    <name>_sample.npy (the sampled pixels) as float32: 12.5 MB per output at 1080p, 50 MB for the four."""
+    import numpy as np
+    import torch
+    first = next(iter(outputs.values()))
+    frame, pix = dump_positions(first.shape[0])
+    pix = torch.from_numpy(pix).to(first.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, f"{name}_frame.npy"), t[frame].cpu().numpy().astype(np.float32))
+        np.save(os.path.join(out_dir, f"{name}_sample.npy"), t.reshape(-1)[pix].cpu().numpy().astype(np.float32))
+
+
 def time_events(fn, stream, reps, warm=3):
     import torch
     for _ in range(warm):
@@ -418,8 +446,9 @@ def run_ours(args, rank, world, local_rank):
     for k0 in range(0, frames_n, 256):
         k = torch.arange(first + k0, first + min(k0 + 256, frames_n), device=dev, dtype=torch.int32)[:, None, None]
         frames[k0:k0 + k.shape[0]] = ((xx * yy + 31 * k) & 255).to(torch.uint8)
-    grids = torch.empty_like(frames)
-    back = torch.empty_like(frames)
+    # one grid and one decoded batch per quantizer, so that the last step leaves every output it computed intact
+    grids = [torch.empty_like(frames) for _ in QLEVELS]
+    backs = [torch.empty_like(frames) for _ in QLEVELS]
     stream = torch.cuda.current_stream(dev)
 
     ev = lambda: torch.cuda.Event(enable_timing=True)
@@ -430,10 +459,10 @@ def run_ours(args, rank, world, local_rank):
         if record:
             row[0].record(stream)
         for i, enc in enumerate(encs):
-            enc.encode_device(frames, grids_out=grids)
+            enc.encode_device(frames, grids_out=grids[i])
             if record:
                 row[2 * i + 1].record(stream)
-            dec.decode_device(LEVELS, grids, images_out=back)
+            dec.decode_device(LEVELS, grids[i], images_out=backs[i])
             if record:
                 row[2 * i + 2].record(stream)
         if record:
@@ -468,15 +497,19 @@ def run_ours(args, rank, world, local_rank):
     names = ["encode_lossless", "decode_lossless", "encode_medium", "decode_medium"]
     per = {n: statistics.mean(r[i].elapsed_time(r[i + 1]) for r in marks) for i, n in enumerate(names)}
 
-    # sanity: the timed outputs are real (last pass was Medium): bounded error, seeds raw
-    err = int((back[:8].to(torch.int16) - frames[:8].to(torch.int16)).abs().max().item())
-    assert err <= 20 and torch.equal(back[:8, ::16, ::16], frames[:8, ::16, ::16]), "bench output failed sanity"
+    # sanity: the timed outputs are real (Medium): bounded error, seeds raw
+    err = int((backs[1][:8].to(torch.int16) - frames[:8].to(torch.int16)).abs().max().item())
+    assert err <= 20 and torch.equal(backs[1][:8, ::16, ::16], frames[:8, ::16, ::16]), "bench output failed sanity"
+
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {f"{kind}_{qname}": t for qname, g, b in zip(("lossless", "medium"), grids, backs)
+                                         for kind, t in (("grid", g), ("decoded", b))})
 
     # ---- strong scaling of the workload as BASELINE configs[4] words it: 4096 frames in total, 4096 / N per rank ----
     strong = None
     if world > 1 and not args.no_extra:
         share = max(1, frames_n // world)
-        fs, gs, bs = frames[:share], grids[:share], back[:share]
+        fs, gs, bs = frames[:share], grids[1][:share], backs[1][:share]
 
         def strong_step():
             for enc in encs:
@@ -498,9 +531,8 @@ def run_ours(args, rank, world, local_rank):
 
     extra = None
     if not args.no_extra:
-        encs[1].encode_device(frames, grids_out=grids)             # Medium grids for the histogram block
         try:
-            extra = extra_block(hgi, ctx, dev, rank, world, dist, measured_peak()[0], grids, barrier)
+            extra = extra_block(hgi, ctx, dev, rank, world, dist, measured_peak()[0], grids[1], barrier)
         except Exception as exc:                                   # the headline line must survive a failing side measurement
             if world > 1:
                 raise                                              # ranks would lose step with each other: fail loudly instead
@@ -511,7 +543,7 @@ def run_ours(args, rank, world, local_rank):
     # ---- e2e: host-pointer C-ABI calls, pinned host memory, copies inside the timed region ----
     e2e = None
     if not args.no_e2e:
-        del back
+        del backs
         torch.cuda.empty_cache()
         n_e = min(args.e2e_frames or 1024, frames_n)        # pinned buffer size (frames); see e2e_step
         n_sub = -(-frames_n // n_e)                         # sub-batches per step: the whole workload streams through
@@ -602,7 +634,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra block (single planes, config 4, histogram, strong scaling)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's outputs to DIR "
+                                                          "as float32 .npy files (50 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     world = int(os.environ.get("WORLD_SIZE", "1"))

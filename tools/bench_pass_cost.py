@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0,'/root/repo')
+import os, sys, torch
+sys.path.insert(0,os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import rustyhgi_b200 as hgi
 def t(fn,n=30):
     for _ in range(5): fn()
