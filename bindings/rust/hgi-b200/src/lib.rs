@@ -130,4 +130,39 @@ impl<I: Interpolator> Decoder<I> {
         assert_eq!(rc, HGI_OK, "hgi_decode_u8: {}", strerror(rc));
         image
     }
+
+    /// Scalable decode (not in the reference): `decode(..)` at 1/2^scale_log2 resolution -- every 2^k-th pixel of
+    /// every 2^k-th row -- cut to `region` (x, y, width, height in those scaled coordinates; None = all of it).
+    /// Only the grid rows the region depends on are decoded.  An empty or out-of-image region is an error.
+    pub fn decode_region(&mut self, (width, height): (u32, u32), levels: usize, grid: &Grid, scale_log2: u32,
+                         region: Option<(u32, u32, u32, u32)>) -> Result<GrayImage, String> {
+        if grid.buffer.len() != width as usize * height as usize {
+            return Err("grid size does not match dimensions".into());
+        }
+        let plan = plan_region(width, height, levels as u32, scale_log2, region)?;
+        let (rw, rh) = region.map_or((plan.scaled_width, plan.scaled_height), |r| (r.2, r.3));
+        let rect = region.map(|(x, y, w, h)| hgi_rect_t { x, y, width: w, height: h });
+        let mut image = GrayImage::new(rw, rh);
+        let params = hgi_params_t { levels: levels as u32, interp: I::ID, quant_kind: HGI_QUANT_NOOP, quant_level: 0 };
+        let rc = unsafe {
+            hgi_decode_region_u8(ctx(), grid.buffer.as_ptr(), width, height, &params, scale_log2,
+                                 rect.as_ref().map_or(ptr::null(), |r| r as *const hgi_rect_t), image.as_mut_ptr())
+        };
+        if rc != HGI_OK { return Err(format!("hgi_decode_region_u8: {}", strerror(rc))); }
+        Ok(image)
+    }
+}
+
+/// `hgi_plan_region`: the window of the grid a scalable decode of `region` reads (pure host arithmetic).
+pub fn plan_region(width: u32, height: u32, levels: u32, scale_log2: u32, region: Option<(u32, u32, u32, u32)>)
+                   -> Result<hgi_region_plan_t, String> {
+    let rect = region.map(|(x, y, w, h)| hgi_rect_t { x, y, width: w, height: h });
+    let mut plan = hgi_region_plan_t { scaled_width: 0, scaled_height: 0, levels: 0,
+                                       window: hgi_rect_t { x: 0, y: 0, width: 0, height: 0 }, crop_x: 0, crop_y: 0 };
+    let rc = unsafe {
+        hgi_plan_region(width, height, levels, scale_log2, rect.as_ref().map_or(ptr::null(), |r| r as *const hgi_rect_t),
+                        &mut plan)
+    };
+    if rc != HGI_OK { return Err(format!("hgi_plan_region: {}", strerror(rc))); }
+    Ok(plan)
 }

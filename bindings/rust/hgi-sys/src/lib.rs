@@ -21,6 +21,28 @@ pub struct hgi_band_t {
     pub in_y1: u32,
 }
 
+/// A rectangle of the scaled image of a scalable decode (scaled coordinates).
+#[repr(C)]
+#[derive(Clone, Copy, Debug, PartialEq, Eq)]
+pub struct hgi_rect_t {
+    pub x: u32,
+    pub y: u32,
+    pub width: u32,
+    pub height: u32,
+}
+
+/// `hgi_plan_region`: the scaled size, the levels decoded on the window, the window and the region's origin in it.
+#[repr(C)]
+#[derive(Clone, Copy, Debug, PartialEq, Eq)]
+pub struct hgi_region_plan_t {
+    pub scaled_width: u32,
+    pub scaled_height: u32,
+    pub levels: u32,
+    pub window: hgi_rect_t,
+    pub crop_x: u32,
+    pub crop_y: u32,
+}
+
 pub const HGI_ABI_VERSION: c_int = 2;
 pub const HGI_OK: c_int = 0;
 pub const HGI_ERR_INVALID_ARG: c_int = -1;
@@ -102,6 +124,14 @@ extern "C" {
                              d_hist_out: *mut u32, stream: *mut c_void) -> c_int;
     pub fn hgi_error_metrics_dev(ctx: *mut hgi_ctx_t, d_before: *const u8, d_after: *const u8, n: usize,
                                  d_out: *mut u64, stream: *mut c_void) -> c_int;
+    pub fn hgi_plan_region(width: u32, height: u32, levels: u32, scale_log2: u32, region: *const hgi_rect_t,
+                           plan_out: *mut hgi_region_plan_t) -> c_int;
+    pub fn hgi_decode_region_dev(ctx: *mut hgi_ctx_t, d_grids: *const u8, n_images: u32, width: u32, height: u32,
+                                 pitch: u32, params: *const hgi_params_t, scale_log2: u32, region: *const hgi_rect_t,
+                                 d_out: *mut u8, out_pitch: u32, stream: *mut c_void) -> c_int;
+    pub fn hgi_decode_region_u8(ctx: *mut hgi_ctx_t, grid: *const u8, width: u32, height: u32,
+                                params: *const hgi_params_t, scale_log2: u32, region: *const hgi_rect_t,
+                                image_out: *mut u8) -> c_int;
     pub fn hgi_pool_create(devices: *const c_int, n_devices: c_int, pool_out: *mut *mut hgi_pool_t) -> c_int;
     pub fn hgi_pool_destroy(pool: *mut hgi_pool_t);
     pub fn hgi_pool_size(pool: *const hgi_pool_t) -> c_int;

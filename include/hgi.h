@@ -199,6 +199,40 @@ int hgi_decode_dev_pitched(hgi_ctx_t *ctx, const uint8_t *d_grids, uint32_t n_im
 int hgi_error_metrics_dev(hgi_ctx_t *ctx, const uint8_t *d_before, const uint8_t *d_after,
                           size_t n, uint64_t *d_out, void *stream);
 
+/* ---- scalable decode: reduced resolution and region of interest ---------------------------- */
+/* The grid is a pyramid: for scale_log2 = k the *scaled image* is ws x hs = ceil(width / 2^k) x ceil(height / 2^k)
+   with scaled[v][u] = decode(grid)[v * 2^k][u * 2^k], and it equals the decode of the grid decimated by 2^k with
+   L' = max(levels - k, 0) levels.  A region is a rectangle of the scaled image (scaled coordinates, inside it; NULL =
+   the whole scaled image).  Because every dependency stays inside a coarse cell and its right / down neighbour, the
+   region is decoded from a window of the decimated grid (DESIGN.md "Scalable decode"), byte-identical to slicing
+   Decoder::decode (src/decoder.rs:18-46). */
+typedef struct {
+    uint32_t x, y, width, height;
+} hgi_rect_t;
+typedef struct {
+    uint32_t scaled_width, scaled_height; /* ws, hs */
+    uint32_t levels;                      /* L' = max(levels - scale_log2, 0): levels decoded on the window */
+    hgi_rect_t window;                    /* decoded window of the scaled image (scaled coordinates) */
+    uint32_t crop_x, crop_y;              /* the region's origin inside the window */
+} hgi_region_plan_t;
+/* The window of `region`: x0 = floor(u0 / A) * A with S' = 2^L', A = max(S', 16); x1 = min(ws, floor((u1 - 1) / S') * S'
+   + 2 S' + 1); rows the same with A = S'.  Pure host arithmetic, no device needed.  HGI_ERR_INVALID_ARG: levels or
+   scale_log2 > HGI_MAX_LEVELS, an empty region or one outside the scaled image, a NULL plan_out. */
+int hgi_plan_region(uint32_t width, uint32_t height, uint32_t levels, uint32_t scale_log2, const hgi_rect_t *region,
+                    hgi_region_plan_t *plan_out);
+/* `n_images` grid planes (rows `pitch` bytes apart, as hgi_decode_dev_pitched) -> the region of each one's scaled
+   image: d_out rows are `out_pitch` bytes apart (>= region width), planes out_pitch * region height apart, and no byte
+   outside the rectangles is written.  Enqueued on `stream` like every *_dev call.  Not on HGI_PATH_PER_LEVEL
+   (-> HGI_ERR_UNSUPPORTED). */
+int hgi_decode_region_dev(hgi_ctx_t *ctx, const uint8_t *d_grids, uint32_t n_images, uint32_t width, uint32_t height,
+                          uint32_t pitch, const hgi_params_t *params, uint32_t scale_log2, const hgi_rect_t *region,
+                          uint8_t *d_out, uint32_t out_pitch, void *stream);
+/* One host plane: only the window's grid rows (every 2^k-th row, the window's column span) go to the device and only
+   the region (packed, region width x height bytes) comes back. */
+int hgi_decode_region_u8(hgi_ctx_t *ctx, const uint8_t *grid, uint32_t width, uint32_t height,
+                         const hgi_params_t *params, uint32_t scale_log2, const hgi_rect_t *region,
+                         uint8_t *image_out);
+
 /* ---- pool: the GPUs of one box behind one handle ------------------------------------------ */
 /* The reference encodes one image per call on one thread (benches/bench.rs:54-110, src/main.rs:41-71); the path
    shards with no exchange between the shards (SURVEY.md 8e), so a pool drives one context per GPU from the calling

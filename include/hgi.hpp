@@ -231,6 +231,25 @@ public:
               "hgi_decode_u8");
         return image;
     }
+
+    // Scalable decode (not in the reference): decode(...) at 1/2^scale_log2 resolution -- every 2^k-th pixel of every
+    // 2^k-th row -- cut to `region` (scaled coordinates; nullptr = all of it), from the grid rows it depends on only.
+    GrayImage decode_region(std::pair<uint32_t, uint32_t> dimensions, size_t levels, const Grid& grid,
+                            uint32_t scale_log2, const hgi_rect_t* region = nullptr)
+    {
+        if (grid.buffer.size() != (size_t)dimensions.first * dimensions.second)
+            throw Error(HGI_ERR_INVALID_ARG, "Decoder::decode_region");
+        hgi_region_plan_t plan;
+        check(hgi_plan_region(dimensions.first, dimensions.second, (uint32_t)levels, scale_log2, region, &plan),
+              "hgi_plan_region");
+        GrayImage image(region ? region->width : plan.scaled_width, region ? region->height : plan.scaled_height,
+                        GrayImage::Uninitialized{});
+        const hgi_params_t p{(uint32_t)levels, I::id, HGI_QUANT_NOOP, 0};
+        check(hgi_decode_region_u8(ctx_->get(), grid.buffer.data(), dimensions.first, dimensions.second, &p, scale_log2,
+                                   region, image.data.data()),
+              "hgi_decode_region_u8");
+        return image;
+    }
 private:
     std::shared_ptr<Context> ctx_;
 };

@@ -27,6 +27,15 @@ class BandStruct(ctypes.Structure):
     _fields_ = [("y0", ctypes.c_uint32), ("y1", ctypes.c_uint32), ("in_y1", ctypes.c_uint32)]
 
 
+class RectStruct(ctypes.Structure):
+    _fields_ = [("x", ctypes.c_uint32), ("y", ctypes.c_uint32), ("width", ctypes.c_uint32), ("height", ctypes.c_uint32)]
+
+
+class RegionPlanStruct(ctypes.Structure):
+    _fields_ = [("scaled_width", ctypes.c_uint32), ("scaled_height", ctypes.c_uint32), ("levels", ctypes.c_uint32),
+                ("window", RectStruct), ("crop_x", ctypes.c_uint32), ("crop_y", ctypes.c_uint32)]
+
+
 class MetadataStruct(ctypes.Structure):
     _fields_ = [("quantization_level", ctypes.c_uint32), ("interpolation", ctypes.c_uint32),
                 ("width", ctypes.c_uint32), ("height", ctypes.c_uint32),
@@ -36,6 +45,7 @@ class MetadataStruct(ctypes.Structure):
 _vp, _u32, _u64, _sz, _int = ctypes.c_void_p, ctypes.c_uint32, ctypes.c_uint64, ctypes.c_size_t, ctypes.c_int
 _pp = ctypes.POINTER(Params)
 _pm = ctypes.POINTER(MetadataStruct)
+_pr = ctypes.POINTER(RectStruct)
 
 # name -> (restype, argtypes); every function declared in include/hgi.h
 PROTOTYPES = {
@@ -69,6 +79,9 @@ PROTOTYPES = {
     "hgi_decode_dev_pitched": (_int, [_vp, _vp, _u32, _u32, _u32, _u32, _pp, _vp, _vp]),
     "hgi_histogram_dev": (_int, [_vp, _vp, _sz, _u32, _vp, _vp]),
     "hgi_error_metrics_dev": (_int, [_vp, _vp, _vp, _sz, _vp, _vp]),
+    "hgi_plan_region": (_int, [_u32, _u32, _u32, _u32, _pr, ctypes.POINTER(RegionPlanStruct)]),
+    "hgi_decode_region_dev": (_int, [_vp, _vp, _u32, _u32, _u32, _u32, _pp, _u32, _pr, _vp, _u32, _vp]),
+    "hgi_decode_region_u8": (_int, [_vp, _vp, _u32, _u32, _pp, _u32, _pr, _vp]),
     "hgi_pool_create": (_int, [_vp, _int, ctypes.POINTER(_vp)]),
     "hgi_pool_destroy": (None, [_vp]),
     "hgi_pool_size": (_int, [_vp]),

@@ -8,6 +8,7 @@ Names, argument meaning and error behaviour follow the reference:
   Archive{metadata, grid}.serialize_to_writer / deserialize_from_reader         src/archive.rs:24-55
 All compute happens in libhgi_b200.so on the GPU; numpy arrays are only containers here.
 """
+import collections
 import ctypes
 import enum
 import threading
@@ -15,7 +16,7 @@ import threading
 import numpy as np
 
 from . import _lib
-from ._lib import HgiError, Params, MetadataStruct
+from ._lib import HgiError, Params, MetadataStruct, RectStruct, RegionPlanStruct
 
 
 class QuantizationLevel(enum.IntEnum):      # src/quantizator.rs:3-8
@@ -427,6 +428,74 @@ class Decoder:
         rc = _lib.lib().hgi_decode_dev_pitched(ctx._h, t.data_ptr(), n, w, h, pitch, ctypes.byref(p), images_out.data_ptr(), st)
         ctx.check(rc, "hgi_decode_dev_pitched")
         return images_out if images_out.dim() == grids.dim() else images_out[0]
+
+    def decode_region(self, dimensions, levels, grid, region=None, scale_log2=0):
+        """Scalable decode of one host grid: `decode(dimensions, levels, grid)[::2^k, ::2^k]` cut to `region` =
+        (x, y, width, height) in those scaled coordinates (None: the whole scaled image), byte for byte, computed from
+        the window of grid rows the region depends on (hgi_decode_region_u8)."""
+        width, height = int(dimensions[0]), int(dimensions[1])
+        buf = grid.buffer if isinstance(grid, Grid) else _host_planes(grid, "grid").reshape(-1)
+        if buf.size != width * height:
+            raise ValueError("grid size does not match dimensions")
+        rw, rh = _region_size(width, height, levels, scale_log2, region)
+        out = np.empty((rh, rw), np.uint8)
+        p = _params(levels, self._interp)
+        rc = _lib.lib().hgi_decode_region_u8(self.ctx._h, buf.ctypes.data, width, height, ctypes.byref(p), int(scale_log2),
+                                             _rect(region), out.ctypes.data)
+        self.ctx.check(rc, "hgi_decode_region_u8")
+        return out
+
+    def decode_region_device(self, levels, grids, region=None, scale_log2=0, out=None, stream=None):
+        """The same for CUDA grids (n, h, w) or (h, w), packed or with padded rows (hgi_decode_region_dev): the result
+        is (n, rh, rw) (or (rh, rw)); `out` may be such a tensor with padded rows, whose padding is left untouched."""
+        import torch
+        t, n, h, w, pitch = _dev_planes(grids, "grids")
+        ctx = _ctx_for(self._ctx, t)
+        rw, rh = _region_size(w, h, levels, scale_log2, region)
+        if out is None:
+            out = torch.empty((n, rh, rw) if grids.dim() == 3 else (rh, rw), dtype=torch.uint8, device=t.device)
+        o, on, oh, ow, out_pitch = _dev_planes(out, "out")
+        if (on, oh, ow) != (n, rh, rw) or o.device != t.device:
+            raise ValueError(f"out must be ({n}, {rh}, {rw}) on {t.device}")
+        st = _stream_handle(stream, t.device)
+        p = _params(levels, self._interp)
+        rc = _lib.lib().hgi_decode_region_dev(ctx._h, t.data_ptr(), n, w, h, pitch, ctypes.byref(p), int(scale_log2),
+                                              _rect(region), o.data_ptr(), out_pitch, st)
+        ctx.check(rc, "hgi_decode_region_dev")
+        return out
+
+
+RegionPlan = collections.namedtuple("RegionPlan", "scaled_width scaled_height levels window crop_x crop_y")
+RegionPlan.__doc__ = """hgi_region_plan_t: the scaled image's size, the levels decoded on the window (L' = max(L - k, 0)),
+the window (x, y, width, height) in scaled coordinates and the region's origin inside it."""
+
+
+def _rect(region):
+    """hgi_rect_t* for an (x, y, width, height) region; None = the whole scaled image (NULL)."""
+    if region is None:
+        return None
+    x, y, w, h = (int(v) for v in region)
+    if min(x, y, w, h) < 0:
+        raise ValueError("region must be (x, y, width, height) with non-negative values")
+    return ctypes.byref(RectStruct(x, y, w, h))
+
+
+def plan_region(width, height, levels, scale_log2=0, region=None):
+    """hgi_plan_region: the window a scalable decode of `region` (scaled coordinates; None = the whole scaled image)
+    reads.  Pure host arithmetic."""
+    p = RegionPlanStruct()
+    rc = _lib.lib().hgi_plan_region(int(width), int(height), int(levels), int(scale_log2), _rect(region), ctypes.byref(p))
+    if rc:
+        raise HgiError(rc, "hgi_plan_region")
+    w = p.window
+    return RegionPlan(p.scaled_width, p.scaled_height, p.levels, (w.x, w.y, w.width, w.height), p.crop_x, p.crop_y)
+
+
+def _region_size(width, height, levels, scale_log2, region):
+    if region is not None:
+        return int(region[2]), int(region[3])
+    pl = plan_region(width, height, levels, scale_log2)
+    return pl.scaled_width, pl.scaled_height
 
 
 def histogram(grid, ctx=None):

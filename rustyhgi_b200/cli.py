@@ -1,7 +1,7 @@
 """`hgi` command line with the reference's sub-commands and flags (src/options.rs:13-64, src/main.rs:41-134):
 
     hgi encode -i <image> -o <archive.hgi> [-l 4] [-q medium]
-    hgi decode -i <archive.hgi> -o <image>
+    hgi decode -i <archive.hgi> -o <image> [--scale K] [--region X,Y,W,H]
     hgi test <image> [-s suffix] [-l 4] [-q medium]
 
 Always Crossed + Linear like the reference (src/main.rs:43-45,67,76-78).  File decoding/encoding is PIL
@@ -44,6 +44,23 @@ def _encoding_options(p):
     p.add_argument("--entropy", choices=("rle", "deflate", "huffman"), default="rle")
 
 
+def _scale(text):
+    k = int(text)
+    if not 0 <= k <= 31:
+        raise argparse.ArgumentTypeError("scale must be 0..31")
+    return k
+
+
+def _region(text):
+    try:
+        v = tuple(int(t) for t in text.split(","))
+    except ValueError:
+        v = ()
+    if len(v) != 4 or min(v) < 0:
+        raise argparse.ArgumentTypeError("region must be X,Y,W,H (non-negative integers)")
+    return v
+
+
 def build_parser():
     ap = argparse.ArgumentParser(prog="hgi", description="Hierarchical Grid Interpolation codec (B200)")
     sub = ap.add_subparsers(dest="cmd", required=True)
@@ -54,6 +71,13 @@ def build_parser():
     dec = sub.add_parser("decode")
     dec.add_argument("-i", "--input", required=True)
     dec.add_argument("-o", "--output", required=True)
+    # not in the reference: scalable decode.  The archive's DEFLATE payload is in raster order, so it is still
+    # inflated whole on the host; only the GPU decode is limited to the rows and columns the output depends on.
+    dec.add_argument("--scale", type=_scale, default=0,
+                     help="write the image at 1/2^K resolution (every 2^K-th pixel of every 2^K-th row); the "
+                          "archive is still inflated whole")
+    dec.add_argument("--region", type=_region, default=None, metavar="X,Y,W,H",
+                     help="write only this rectangle, in the coordinates of the (scaled) image")
     tst = sub.add_parser("test")
     tst.add_argument("input")
     tst.add_argument("-s", "--suffix", default="")                              # src/options.rs:34-35
@@ -75,7 +99,10 @@ def decode(a):                                            # src/main.rs:63-71
     with open(a.input, "rb") as f:
         arch = api.Archive.deserialize_from_reader(f)
     m = arch.metadata
-    image = api.Decoder(api.Crossed).decode((m.width, m.height), m.scale_level, arch.grid)
+    if a.scale or a.region is not None:
+        image = api.Decoder(api.Crossed).decode_region((m.width, m.height), m.scale_level, arch.grid, a.region, a.scale)
+    else:
+        image = api.Decoder(api.Crossed).decode((m.width, m.height), m.scale_level, arch.grid)
     Image.fromarray(image, "L").save(a.output)
 
 

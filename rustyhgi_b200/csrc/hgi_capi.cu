@@ -58,6 +58,7 @@ struct Scratch {
     DevBuf compact[4];   // ping-pong {recon, q} compact planes of the coarse passes
     DevBuf dec_in;       // decimated source of a coarse pass
     DevBuf level_recon;  // per-level path: reconstruction planes when the caller gives none
+    DevBuf region_in, region_out;   // scalable decode: the gathered window of the grid, and the decoded window
     // fork/join of the independent split launches of the quantizing encode (hgi_kernels.h PassArgs::side_stream)
     cudaStream_t side = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
@@ -191,6 +192,8 @@ void free_scratch(Scratch& sc)
     for (auto& b : sc.compact) if (b.p) { cudaFree(b.p); b = DevBuf{}; }
     if (sc.dec_in.p) { cudaFree(sc.dec_in.p); sc.dec_in = DevBuf{}; }
     if (sc.level_recon.p) { cudaFree(sc.level_recon.p); sc.level_recon = DevBuf{}; }
+    if (sc.region_in.p) { cudaFree(sc.region_in.p); sc.region_in = DevBuf{}; }
+    if (sc.region_out.p) { cudaFree(sc.region_out.p); sc.region_out = DevBuf{}; }
     if (sc.side) { cudaStreamDestroy(sc.side); sc.side = nullptr; }
     if (sc.ev_fork) { cudaEventDestroy(sc.ev_fork); sc.ev_fork = nullptr; }
     if (sc.ev_join) { cudaEventDestroy(sc.ev_join); sc.ev_join = nullptr; }
@@ -653,6 +656,75 @@ int run_host(hgi_ctx* ctx, int mode, const uint8_t* in, uint32_t n_images, uint3
     }
     if (rc != HGI_OK) (void)cudaGetLastError();
     return rc;
+}
+
+// Window of a scalable decode (DESIGN.md "Scalable decode"): the region [u0, u1) of the scaled image is decoded from
+// the window [x0, x1) with L' = max(L - k, 0) levels, x0 aligned down to S' = 2^L' (to max(S', 16) on the column axis:
+// whole 16-byte chunks for the gather's 128-bit loads) and x1 = min(ws, floor((u1 - 1) / S') * S' + 2 S' + 1) -- the
+// band rule y1 + S + 1 after aligning the end outwards to S'.  `r_out` receives the region (NULL: the scaled image).
+int plan_region(uint32_t w, uint32_t h, uint32_t levels, uint32_t k, const hgi_rect_t* region, hgi_region_plan_t* p,
+                hgi_rect_t* r_out)
+{
+    if (levels > HGI_MAX_LEVELS || k > HGI_MAX_LEVELS) return HGI_ERR_INVALID_ARG;
+    const uint32_t ws = ceil_shift(w, k), hs = ceil_shift(h, k);
+    const hgi_rect_t r = region ? *region : hgi_rect_t{0, 0, ws, hs};
+    if (r.width == 0 || r.height == 0 || (uint64_t)r.x + r.width > ws || (uint64_t)r.y + r.height > hs)
+        return HGI_ERR_INVALID_ARG;
+    const uint32_t lp = levels > k ? levels - k : 0;
+    const uint64_t S = 1ull << lp, A = S > 16 ? S : 16;
+    auto end = [S](uint64_t u1, uint64_t n) {
+        const uint64_t e = (u1 - 1) / S * S + 2 * S + 1;
+        return e < n ? e : n;
+    };
+    const uint64_t x0 = r.x / A * A, y0 = r.y / S * S;
+    const uint64_t x1 = end((uint64_t)r.x + r.width, ws), y1 = end((uint64_t)r.y + r.height, hs);
+    *p = hgi_region_plan_t{ws, hs, lp, hgi_rect_t{(uint32_t)x0, (uint32_t)y0, (uint32_t)(x1 - x0), (uint32_t)(y1 - y0)},
+                           (uint32_t)(r.x - x0), (uint32_t)(r.y - y0)};
+    *r_out = r;
+    return HGI_OK;
+}
+
+// Argument checks shared by the region entry points: decode's, plus the region.
+int check_region(hgi_ctx* ctx, const hgi_params_t* prm, uint32_t w, uint32_t h, uint32_t n_images, uint32_t pitch,
+                 uint32_t k, const hgi_rect_t* region, hgi_region_plan_t* pl, hgi_rect_t* r)
+{
+    if (!ctx) return HGI_ERR_INVALID_ARG;
+    int rc = check_params(prm, false);
+    if (rc) return rc;
+    if (!plane_size_ok(w, h, n_images, pitch)) return HGI_ERR_INVALID_ARG;
+    rc = plan_region(w, h, prm->levels, k, region, pl, r);
+    if (rc) return rc;
+    if (ctx->path == HGI_PATH_PER_LEVEL) return HGI_ERR_UNSUPPORTED;   // the window decode is a tile path
+    return HGI_OK;
+}
+
+// Scalable decode of `n_images` planes: gather the window lattice (src + img * plane_stride + v * row_step + (u << k),
+// see launch_region_gather) into dense planes, decode them on the tile path with L' levels, crop the region into
+// d_out.  Launches plainly: region chains are not graph-cached.
+int run_region(hgi_ctx* ctx, Scratch& sc, const uint8_t* src, uint64_t row_step, uint64_t plane_stride, bool vec,
+               uint64_t row_avail, uint32_t k, uint32_t n_images, const hgi_region_plan_t& pl, const hgi_rect_t& r,
+               const hgi_params_t* prm, uint8_t* d_out, uint32_t out_pitch, cudaStream_t st)
+{
+    const uint32_t ww = pl.window.width, wh = pl.window.height, wpitch = align16(ww);
+    const size_t bytes = (size_t)n_images * wpitch * wh;
+    const uint32_t levels = effective_levels(pl.levels, ww, wh);   // 0: the window of the grid is the image
+    int rc = reserve(ctx, sc, sc.region_in, bytes);
+    if (!rc && levels) rc = reserve(ctx, sc, sc.region_out, bytes);
+    if (rc) return rc;
+    HGI_CUDA(ctx, hgi::launch_region_gather(src, row_step, plane_stride, k, ww, wh, wpitch, n_images, vec, row_avail,
+                                            sc.region_in.p, st));
+    ctx->launches++;
+    const uint8_t* win = sc.region_in.p;
+    if (levels) {
+        rc = run_tile_path(ctx, sc, hgi::kModeDecode, sc.region_in.p, n_images, ww, wh, wpitch, levels, prm, nullptr,
+                           sc.region_out.p, st);
+        if (rc) return rc;
+        win = sc.region_out.p;
+    }
+    HGI_CUDA(ctx, hgi::launch_region_crop(win, wpitch, wh, pl.crop_x, pl.crop_y, r.width, r.height, n_images, d_out,
+                                          out_pitch, st));
+    ctx->launches++;
+    return HGI_OK;
 }
 
 }  // namespace
@@ -1123,6 +1195,73 @@ int hgi_error_metrics_u8(hgi_ctx_t* ctx, const uint8_t* before, const uint8_t* a
     return HGI_OK;
 }
 
+
+int hgi_plan_region(uint32_t width, uint32_t height, uint32_t levels, uint32_t scale_log2, const hgi_rect_t* region,
+                    hgi_region_plan_t* plan_out)
+{
+    if (!plan_out) return HGI_ERR_INVALID_ARG;
+    hgi_rect_t r;
+    return plan_region(width, height, levels, scale_log2, region, plan_out, &r);
+}
+
+int hgi_decode_region_dev(hgi_ctx_t* ctx, const uint8_t* d_grids, uint32_t n_images, uint32_t width, uint32_t height,
+                          uint32_t pitch, const hgi_params_t* params, uint32_t scale_log2, const hgi_rect_t* region,
+                          uint8_t* d_out, uint32_t out_pitch, void* stream)
+{
+    hgi_region_plan_t pl;
+    hgi_rect_t r;
+    int rc = check_region(ctx, params, width, height, n_images, pitch, scale_log2, region, &pl, &r);
+    if (rc) return rc;
+    if (out_pitch < r.width) return HGI_ERR_INVALID_ARG;
+    if (n_images == 0) return HGI_OK;
+    if (!d_grids || !d_out) return HGI_ERR_INVALID_ARG;
+    // the whole image into packed rows is a plain decode (with padded rows that one may write the padding)
+    if (scale_log2 == 0 && r.width == width && r.height == height && out_pitch == pitch && pitch == width)
+        return hgi_decode_dev_pitched(ctx, d_grids, n_images, width, height, pitch, params, d_out, stream);
+    DeviceGuard g(ctx);
+    if (!g.ok) return HGI_ERR_CUDA;
+    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+    Scratch* sc = scratch_for(ctx, st);
+    if (!sc) return HGI_ERR_ALLOC;
+    const uint32_t k = scale_log2;
+    const uint8_t* src = d_grids + ((size_t)pl.window.y << k) * pitch + ((size_t)pl.window.x << k);
+    const uint64_t row_step = (uint64_t)pitch << k, plane_stride = (uint64_t)pitch * height;
+    const bool vec = aligned16(src) && row_step % 16 == 0 && (n_images == 1 || plane_stride % 16 == 0);
+    // the last row of the last plane ends at its pitch: no 128-bit load may reach past that
+    const uint64_t row_avail = pitch - ((uint64_t)pl.window.x << k);
+    return run_region(ctx, *sc, src, row_step, plane_stride, vec, row_avail, k, n_images, pl, r, params, d_out, out_pitch, st);
+}
+
+int hgi_decode_region_u8(hgi_ctx_t* ctx, const uint8_t* grid, uint32_t width, uint32_t height, const hgi_params_t* params,
+                         uint32_t scale_log2, const hgi_rect_t* region, uint8_t* image_out)
+{
+    hgi_region_plan_t pl;
+    hgi_rect_t r;
+    int rc = check_region(ctx, params, width, height, 1, width, scale_log2, region, &pl, &r);
+    if (rc) return rc;
+    if (!grid || !image_out) return HGI_ERR_INVALID_ARG;
+    DeviceGuard g(ctx);
+    if (!g.ok) return HGI_ERR_CUDA;
+    const uint32_t k = scale_log2, ww = pl.window.width, wh = pl.window.height;
+    // Stage the window's grid rows (every 2^k-th row, its column span) with one 2D copy.  Rows of the staging buffer
+    // are readable up to (ww << k) bytes for k <= 3, so the gather's 128-bit loads never leave a row.
+    const uint64_t span = ((uint64_t)(ww - 1) << k) + 1;
+    const uint64_t spitch = ((k <= 3 ? (uint64_t)ww << k : span) + 15) & ~(uint64_t)15;
+    const size_t out_bytes = (size_t)r.width * r.height;
+    Slot& sl = ctx->slots[0];
+    if (!sl.stream) HGI_CUDA(ctx, cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
+    rc = reserve(ctx, sl.in, (size_t)spitch * wh);
+    if (!rc) rc = reserve(ctx, sl.out, out_bytes);
+    if (rc) return rc;
+    const uint8_t* src = grid + ((size_t)pl.window.y << k) * width + ((size_t)pl.window.x << k);
+    const size_t src_pitch = wh > 1 ? (size_t)width << k : (size_t)spitch;
+    rc = cuda_rc(ctx, cudaMemcpy2DAsync(sl.in.p, spitch, src, src_pitch, span, wh, cudaMemcpyHostToDevice, sl.stream));
+    if (!rc) rc = run_region(ctx, sl.scratch, sl.in.p, spitch, 0, true, spitch, k, 1, pl, r, params, sl.out.p, r.width, sl.stream);
+    if (!rc) rc = cuda_rc(ctx, cudaMemcpyAsync(image_out, sl.out.p, out_bytes, cudaMemcpyDeviceToHost, sl.stream));
+    const cudaError_t e = cudaStreamSynchronize(sl.stream);   // nothing may still write into image_out on return
+    if (e != cudaSuccess && rc == HGI_OK) rc = fail(ctx, e);
+    return rc;
+}
 
 /* ---- pool: several GPUs behind one handle -------------------------------------------------------------------- */
 }  // extern "C"

@@ -79,6 +79,16 @@ struct LevelArgs {
 // dense planes (dpitch x hD each, zero padded), so that the pass itself runs on contiguous rows.
 cudaError_t launch_decimate(const uint8_t* src, uint32_t pitch, uint32_t h, uint32_t d_log2, uint32_t wD, uint32_t hD,
                             uint32_t dpitch, uint32_t n_images, uint8_t* dst, cudaStream_t stream);
+// Scalable decode (hgi_region.cu).  Gather: dst[img][v][u] = src[img * plane_stride + v * row_step + (u << k)] for the
+// ww x wh window of `n_images` planes, rows of dst `dpitch` (16-byte multiple) apart, zero padded; `vec`: src, row_step
+// and plane_stride are 16-byte aligned and every source row is readable for `row_avail` bytes (128-bit loads).
+cudaError_t launch_region_gather(const uint8_t* src, uint64_t row_step, uint64_t plane_stride, uint32_t k, uint32_t ww,
+                                 uint32_t wh, uint32_t dpitch, uint32_t n_images, bool vec, uint64_t row_avail,
+                                 uint8_t* dst, cudaStream_t stream);
+// Crop: out[img][r][j] = win[img][cy + r][cx + j] (window planes wpitch x wh) for the rw x rh rectangle; output rows
+// out_pitch apart, planes out_pitch * rh apart; no byte outside the rectangle is written.
+cudaError_t launch_region_crop(const uint8_t* win, uint32_t wpitch, uint32_t wh, uint32_t cx, uint32_t cy, uint32_t rw,
+                               uint32_t rh, uint32_t n_images, uint8_t* out, uint32_t out_pitch, cudaStream_t stream);
 cudaError_t launch_seed(int mode, const uint8_t* src, uint8_t* dst, uint32_t w, uint32_t h,
                         uint32_t levels, uint32_t n_images, cudaStream_t stream);
 cudaError_t launch_level(int mode, int interp, const LevelArgs& args, cudaStream_t stream);
