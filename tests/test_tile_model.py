@@ -34,6 +34,33 @@ def test_small_tiles_many_passes():
         assert (tm.decode(g, levels, True, tw=32, th=16) == r).all()
 
 
+@pytest.mark.parametrize("args,kw,want", [
+    (("enc", 20, 1920, 1080, True, 4, 4096), {"hist": True}, 4),   # the bench shape: interior + right column + bottom row + histogram
+    (("enc", 20, 1920, 1080, True, 4, 23), {}, 1),                 # 23 * 255 tiles = 5865 < 5920: one launch
+    (("enc", 20, 1920, 1080, True, 4, 24), {}, 3),                 # 24 * 255 = 6120 tiles split
+    (("enc", 0, 1920, 1080, True, 4, 4096), {}, 1),                # Lossless never splits
+    (("enc", 20, 1920, 1080, False, 4, 4096), {}, 1),              # nor the unaligned instantiation
+    (("dec", 0, 1920, 1080, True, 4, 4096), {}, 1),
+    (("enc", 20, 160, 96, True, 4, 1), {"split_min": 1}, 3),       # one interior tile, one right column (PART 2), one bottom row
+    (("enc", 20, 256, 145, True, 4, 1), {"split_min": 1}, 3),      # 2 x 3 tiles, interior 1 x 2
+    (("enc", 20, 128, 64, True, 4, 1), {"split_min": 1}, 1),       # no interior tile: the bottom-row launch only
+    (("enc", 20, 160, 80, True, 4, 1), {"split_min": 1}, 1),       # an interior column but no interior row
+    (("enc", 20, 96, 160, True, 4, 1), {"split_min": 1}, 1),       # an interior row but no interior column
+    (("enc", 20, 160, 96, True, 5, 1), {"split_min": 1}, 5),       # decimate + coarse (1 level, one launch) + split fine pass
+    (("enc", 20, 160, 96, True, 8, 1), {"split_min": 1, "hist": True}, 6),   # decimate + coarse split (bottom row only) + 3 + hist
+    (("enc", 20, 2320, 1296, True, 8, 1), {"split_min": 1}, 7),    # the 145 x 81 coarse plane has an interior tile: 1 + 3 + 3
+    (("dec", 0, 160, 96, True, 8, 1), {}, 3),
+    (("enc", 20, 160, 96, True, 4, 66000), {"hist": True}, 5),     # 65535 images split, the remaining 465 (1860 tiles) do not
+    (("enc", 20, 160, 96, True, 8, 66000), {}, 2 + 2 + 3 + 1),     # two decimate launches, two coarse chunks, split + plain fine
+    (("enc", 20, 160, 96, True, 0, 3), {}, 0),                     # L = 0 is a copy
+    (("enc", 20, 160, 96, True, 0, 3), {"hist": True}, 1),
+    (("enc", 20, 0, 96, True, 4, 3), {"hist": True}, 0),
+])
+def test_expected_launches(args, kw, want):
+    """The plain statement of the launch dispatch (tile_model.expected_launches) on hand-worked shapes."""
+    assert tm.expected_launches(*args, **kw) == want
+
+
 def test_pass_plan():
     assert tm.plan_passes(4) == [(0, 4)]
     assert tm.plan_passes(6) == [(4, 2), (0, 4)]

@@ -31,6 +31,38 @@ def plan_passes(levels):
     return out[::-1]
 
 
+SPLIT_MIN_TILES = 4 * 1480      # split_min_tiles() in hgi_tile_fast.cu (HGI_B200_SPLIT_MIN overrides it)
+MAX_GRID_Z = 65535               # images per launch (gridDim.z)
+
+
+def expected_launches(mode, qerr, w, h, pitch_aligned, levels, n, split_min=SPLIT_MIN_TILES, hist=False):
+    """Kernels one device-API call of the tile path launches (hgi_ctx_kernel_launches), stated plainly: per pass of
+    plan_passes(L), one decimate launch per 65535-image chunk for a coarse pass, then per chunk either one launch or,
+    for a split quantizing encode, the interior / right-column / bottom-row launches that have tiles; plus one for the
+    histogram.  `mode` is "enc" or "dec", `qerr` the quantizer's error (0: Lossless / NoOp), `pitch_aligned` whether
+    the fine pass runs the 128-bit instantiation (16-byte rows and bases; coarse passes always do)."""
+    if n == 0 or w * h == 0:
+        return 0
+    total = 1 if hist else 0
+    chunks = [min(MAX_GRID_Z, n - first) for first in range(0, n, MAX_GRID_Z)]
+    for (d, nlev) in plan_passes(effective_levels(levels, w, h)):
+        wD, hD = -(-w >> d), -(-h >> d)
+        tx, ty = -(-wD // TW), -(-hD // TH)
+        if d > 0:
+            total += len(chunks)
+        for cnt in chunks:
+            split = mode == "enc" and qerr != 0 and (pitch_aligned or d > 0) and nlev == 4 and tx * ty * cnt >= split_min
+            if not split:
+                total += 1
+                continue
+            itx = min(tx, (wD - (FMAX + 1)) // TW) if wD >= FMAX + 1 else 0
+            ity = min(ty, (hD - (FMAX + 1)) // TH) if hD >= FMAX + 1 else 0
+            if itx == 0 or ity == 0:
+                itx = ity = 0
+            total += (itx > 0) + (tx - itx > 0 and ity > 0) + (ty - ity > 0)
+    return total
+
+
 def need_limit(extent, s):
     return extent - 1 if s == 1 else (extent if s == 2 else extent + s)
 
