@@ -75,7 +75,8 @@ typedef enum {
     HGI_PATH_TILE = 0,         /* default: fused multi-level tile kernels (register-prefetch SWAR kernel where eligible) */
     HGI_PATH_PER_LEVEL = 1,    /* one kernel per level over HBM (north_star's literal shape) */
     HGI_PATH_TILE_GENERIC = 2, /* fused tiles, always the generic (scalar, any alignment) kernel */
-    HGI_PATH_TILE_TMA = 3      /* fused tiles, persistent TMA-pipelined SWAR kernel instead of the prefetch one */
+    HGI_PATH_TILE_TMA = 3      /* accepted for compatibility: runs exactly what HGI_PATH_TILE runs (the TMA kernel it
+                                  once selected has been removed) */
 } hgi_path_t;
 
 #define HGI_MAX_LEVELS 31u

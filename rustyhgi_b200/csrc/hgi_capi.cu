@@ -373,10 +373,8 @@ int run_tile_path(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint3
             a.s_q = sc.compact[set + 1].p;
             a.dec_in = sc.dec_in.p;
         }
-        const int variant = ctx->path == HGI_PATH_TILE_GENERIC ? hgi::kTileGeneric
-                            : (ctx->path == HGI_PATH_TILE_TMA ? hgi::kTileTma : hgi::kTileAuto);
         const uint64_t before = hgi::launch_count();
-        HGI_CUDA(ctx, hgi::launch_tile_pass(mode, prm->interp, a, st, variant));
+        HGI_CUDA(ctx, hgi::launch_tile_pass(mode, prm->interp, a, st, ctx->path == HGI_PATH_TILE_GENERIC));
         ctx->launches += hgi::launch_count() - before;
         c_recon = a.s_recon;
         c_q = a.s_q;

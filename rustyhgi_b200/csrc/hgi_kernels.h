@@ -52,17 +52,14 @@ struct PassArgs {
     cudaEvent_t ev_fork, ev_join;
 };
 
-// Dispatch of one pass.  kTileAuto: D == 1 passes on 16-byte-aligned planes go to the register-prefetch SWAR
-// kernel (hgi_tile_fast.cu), everything else to the generic kernel (hgi_tile_kernels.cu).  kTileTma selects
-// the persistent TMA-pipelined kernel (hgi_tile_tma.cu) for the eligible passes instead -- measured slower
-// than the prefetch kernel in round 1 (profiles/), kept as a tested alternative.
-enum TileVariant : int { kTileAuto = 0, kTileGeneric = 1, kTileTma = 2 };
+// Dispatch of one pass.  By default every pass of a plane up to 65535 tiles tall goes to the register-prefetch SWAR
+// kernel (hgi_tile_fast.cu), taller planes to the generic kernel (hgi_tile_kernels.cu); `generic` forces the generic
+// kernel, the independent formulation the tests cross-check against.
 // Kernels launched so far by the calling thread's launch_* calls (for hgi_ctx_kernel_launches).
 uint64_t& launch_count();
 
-cudaError_t launch_tile_pass(int mode, int interp, const PassArgs& args, cudaStream_t stream, int variant = kTileAuto);
+cudaError_t launch_tile_pass(int mode, int interp, const PassArgs& args, cudaStream_t stream, bool generic);
 cudaError_t launch_tile_pass_fast(int mode, int interp, const PassArgs& args, cudaStream_t stream);
-cudaError_t launch_tile_pass_tma(int mode, int interp, const PassArgs& args, cudaStream_t stream, bool* used);
 bool quant_swar_self_check();
 
 // ---- per-level path -----------------------------------------------------------------------

@@ -34,9 +34,7 @@ constexpr int kHistBinStride = 256;                         // bytes between bin
 constexpr int kHistSmem = 256 * kHistBinStride;             // 64 KB
 __device__ __forceinline__ void hist_count_word(uint8_t* bins, uint32_t w, uint32_t lane4)
 {
-#ifndef HGI_VAR_HIST_NOSWZ
     w ^= lane4 * 0x02020202u;   // row = bin ^ (8 * lane): equal symbols of different lanes go to different rows (see below)
-#endif
     atomicAdd(reinterpret_cast<uint32_t*>(bins + __byte_perm(w, lane4, 0x6504u)), 1u);
     atomicAdd(reinterpret_cast<uint32_t*>(bins + __byte_perm(w, lane4, 0x6514u)), 1u);
     atomicAdd(reinterpret_cast<uint32_t*>(bins + __byte_perm(w, lane4, 0x6524u)), 1u);
@@ -44,9 +42,7 @@ __device__ __forceinline__ void hist_count_word(uint8_t* bins, uint32_t w, uint3
 }
 __device__ __forceinline__ void hist_count_byte(uint8_t* bins, uint32_t b, uint32_t lane4)
 {
-#ifndef HGI_VAR_HIST_NOSWZ
     b ^= 2u * lane4;
-#endif
     atomicAdd(reinterpret_cast<uint32_t*>(bins + b * kHistBinStride + lane4), 1u);
 }
 
@@ -98,11 +94,7 @@ hgi_hist_kernel(const uint8_t* __restrict__ data, uint32_t w, uint32_t h, uint32
     // warp k reduces its share of the bins: lane-parallel reads of one bin row, shuffle tree
     constexpr int kBinsPerWarp = 256 / (HT / 32);
     for (int bin = (tid >> 5) * kBinsPerWarp; bin < (tid >> 5) * kBinsPerWarp + kBinsPerWarp; ++bin) {
-#ifndef HGI_VAR_HIST_NOSWZ
         uint32_t v = *reinterpret_cast<const uint32_t*>(bins + (bin ^ (int)(2u * lane4)) * kHistBinStride + lane4);
-#else
-        uint32_t v = *reinterpret_cast<const uint32_t*>(bins + bin * kHistBinStride + lane4);
-#endif
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xFFFFFFFFu, v, o);
         if (lane == 0 && v) atomicAdd(&hist[(size_t)img * 256 + bin], v);

@@ -35,16 +35,6 @@
 // Tile shape / CTA size / residency of the register-prefetch kernel.  Measured on B200 (bench.py, 4096 frames,
 // ms per step, at the time of the sweep): 128x64 tiles with 128 threads (2 units per thread) at 10 CTAs/SM 14.5;
 // 128x128 / 256 / 6: 15.1; 128x64 / 256 / 8: 16.0.  Small CTAs keep every barrier inside four warps.
-#ifndef HGI_FAST_TILE_H
-#define HGI_FAST_TILE_H 64
-#endif
-#ifndef HGI_FAST_NT
-#define HGI_FAST_NT 128
-#endif
-#define HGI_TILE_H HGI_FAST_TILE_H
-#ifdef HGI_FAST_NT
-#define HGI_TILE_NT HGI_FAST_NT
-#endif
 #include <cstdlib>
 #include "hgi_tile_swar.cuh"
 
@@ -111,13 +101,7 @@ __device__ __forceinline__ void store_chunk(uint8_t* __restrict__ ptr, const uin
 {
     if (nvalid <= 0) return;
     if (ALIGNED) {
-#if defined(HGI_VAR_STCS)
-        __stcs(reinterpret_cast<uint4*>(ptr), make_uint4(w[0], w[1], w[2], w[3]));   // streaming (evict-first) store, A/B hook
-#elif defined(HGI_VAR_STCG)
-        __stcg(reinterpret_cast<uint4*>(ptr), make_uint4(w[0], w[1], w[2], w[3]));
-#else
         *reinterpret_cast<uint4*>(ptr) = make_uint4(w[0], w[1], w[2], w[3]);
-#endif
         return;
     }
     const uint32_t sh = (uint32_t)((uintptr_t)ptr & 3u);
@@ -146,19 +130,14 @@ __device__ __forceinline__ void store_chunk(uint8_t* __restrict__ ptr, const uin
 // compile to LDS/STS because the pointer is rebuilt with the shared->generic intrinsic.
 __device__ __forceinline__ FastSmem& opaque_smem(FastSmem& s)
 {
-#ifdef HGI_VAR_NO_OPAQUE_SMEM
-    return s;
-#else
     uint32_t a = (uint32_t)__cvta_generic_to_shared(&s);
     asm volatile("" : "+r"(a));
     return *reinterpret_cast<FastSmem*>(__cvta_shared_to_generic(a));
-#endif
 }
 
 // EDGE = 0: the tile and its whole halo lie inside the image, so every extent is a compile-time constant
 // EDGE = 2: a tile of the right tile column of a plane whose width is a multiple of the tile width, in a tile row whose
 //           halo rows are inside the image: exactly TW columns (no right halo), all rows -- constants again
-// EDGE = 3: a tile of a bottom tile row whose column (with its right halo) is inside the image: all columns, run-time rows
 // EDGE = 1: anything else
 // and all the in-image predicates (loads, stores, fringe cells, masks) fold away.
 template <int MODE, int INTERP, bool IDENTITY, bool EXTRA, int NLEV, bool ALIGNED, int EDGE>
@@ -166,13 +145,11 @@ __device__ __forceinline__ void tile_body(const PassArgs& p, FastSmem& sm, uint3
 {
     constexpr int F = 1 << NLEV;
     const int tid = threadIdx.x;
-#ifndef HGI_VAR_NO_ASSUME
     __builtin_assume(tid >= 0 && tid < NT);     // lets the row/column range tests of interior tiles fold
-#endif
     const uint32_t img = blockIdx.z;
     const uint32_t X0 = tx * TW, Y0 = ty * TH;
     const int xin = EDGE == 1 ? (int)min((uint32_t)(TW + FMAX + 1), p.w - X0) : (EDGE == 2 ? TW : TW + FMAX + 1);   // in-image extent of tile + halo
-    const int yin = (EDGE == 1 || EDGE == 3) ? (int)min((uint32_t)(TH + FMAX + 1), p.h - Y0) : TH + FMAX + 1;
+    const int yin = EDGE == 1 ? (int)min((uint32_t)(TH + FMAX + 1), p.h - Y0) : TH + FMAX + 1;
     const bool edge = EDGE != 0;
     const size_t tile_off = ((size_t)img * p.h + Y0) * p.pitch + X0;   // CTA-uniform; the same in the source and output planes
     const size_t pitch = (size_t)p.pitch;
@@ -223,23 +200,10 @@ __device__ __forceinline__ void tile_body(const PassArgs& p, FastSmem& sm, uint3
     // (2048 frames, same box): spread over the upper half of the CTA, one chunk per thread (decode 1.258 ms, encode
     // Medium 1.681, encode Lossless 1.274), or all on the LAST WARP, NRIGHT/32 + 1 chunks per lane, so that the other
     // warps skip the block with one uniform branch (1.266 / 1.722 / 1.242): the identity encode takes the second.
-#ifdef HGI_VAR_HALO_WARP_DECODE
-    constexpr bool HALO_WARP = ((MODE == kModeEncode) && IDENTITY) || MODE == kModeDecode;
-#else
     constexpr bool HALO_WARP = (MODE == kModeEncode) && IDENTITY;
-#endif
     constexpr int NRIGHT = TH / 2, NHALO = NRIGHT + 27, NRL = NRIGHT / 32;
-    // HGI_VAR_HALO_TWO_WARPS / _DECODE: whole warps fetch the halo (warp 1 the right column, warp 2 the bottom rows), A/B
-    // hook: encode Medium +1 % slower, decode -0.8 % (inside the noise) -- not the default
-#if defined(HGI_VAR_HALO_TWO_WARPS_DECODE)
-    constexpr bool HALO_TWO_WARPS = (TH == 64 && NT == 128);
-#elif defined(HGI_VAR_HALO_TWO_WARPS)
-    constexpr bool HALO_TWO_WARPS = (TH == 64 && NT == 128) && !(MODE == kModeDecode);
-#else
-    constexpr bool HALO_TWO_WARPS = false;
-#endif
     // -- spread form
-    const int hj = tid - (NT - (TH == 64 ? 64 : 128));
+    const int hj = tid - (NT - 64);
     int hy = 2 * hj, hc = 8;
     bool halo = false;
     uint4 hv = make_uint4(0u, 0u, 0u, 0u);
@@ -251,23 +215,7 @@ __device__ __forceinline__ void tile_body(const PassArgs& p, FastSmem& sm, uint3
     for (int k = 0; k < NRL; ++k) hvr[k] = make_uint4(0u, 0u, 0u, 0u);
     int hyb = TH, hcb = 0;
     bool has_b = false;
-    if (!HALO_WARP && HALO_TWO_WARPS) {
-        // warp 1: the 32 right-halo chunks, one per lane; warp 2: the 27 bottom chunks.  Whole warps, so the others skip
-        // the address arithmetic with a uniform branch (the spread form below is if-converted: every warp issues it),
-        // and warps 1 and 2 are the ones with the least other work (warp 0 runs the s = 8 level, warp 3 the s = 2 fringe).
-        const int wid = tid >> 5, lane = tid & 31;
-        if (NLEV > 1 && wid == 1) {
-            hy = 2 * lane;
-            halo = true;
-            if (hy < yin) hv = load_chunk<ALIGNED>(tile + (uint32_t)hy * p.pitch + (uint32_t)TW, min(16, xin - TW), false, ragged);
-        } else if (NLEV > 1 && wid == 2 && lane < 27) {
-            const int r = (lane >= 9) + (lane >= 18);
-            hc = lane - 9 * r;
-            hy = TH + 4 * r;
-            halo = true;
-            if (hy < yin) hv = load_chunk<ALIGNED>(tile + (uint32_t)hy * p.pitch + (uint32_t)(16 * hc), min(16, xin - 16 * hc), false, ragged);
-        }
-    } else if (!HALO_WARP) {
+    if (!HALO_WARP) {
         if (hj >= NRIGHT) {
             const int r = (hj - NRIGHT) / 9;
             hc = (hj - NRIGHT) - 9 * r;
@@ -292,11 +240,7 @@ __device__ __forceinline__ void tile_body(const PassArgs& p, FastSmem& sm, uint3
     }
 
     // ---- 2. stage the dense coarse planes + the coarse lattice of this pass ---------------------
-#ifdef HGI_VAR_NO_OWN2
-    constexpr bool OWN2 = false;
-#else
-    constexpr bool OWN2 = (F >= 4) && (NU == 2);   // the s = 2 level runs from this thread's registers (level2_owner)
-#endif
+    constexpr bool OWN2 = F >= 4;   // the s = 2 level runs from this thread's registers (level2_owner)
 #pragma unroll
     for (int u = 0; u < NU; ++u) stage_chunk<F, OWN2>(sm.P, ev[u], 2 * (NU * ry + u), sx);
     if (halo) stage_chunk<F>(sm.P, hv, hy, hc);
@@ -371,39 +315,16 @@ __device__ __forceinline__ void tile_body(const PassArgs& p, FastSmem& sm, uint3
         }
     }
     __syncthreads();
-#ifdef HGI_VAR_STOP_AFTER   // timing experiment (tools/time_encode.py): cut the kernel after a phase, keep the HBM traffic
-#define HGI_EARLY_STORE(extra)                                                                                        \
-    {                                                                                                                 \
-        uint8_t* o_ = (MODE == kModeEncode ? p.grid_out : p.recon_out) + tile_off;                                    \
-        for (int u = 0; u < NU; ++u) {                                                                                \
-            uint4 e_ = ev[u], d_ = od[u];                                                                             \
-            e_.x ^= (extra);                                                                                          \
-            const int y_ = 2 * (NU * ry + u);                                                                         \
-            if (nvalid > 0 && y_ < yin) *reinterpret_cast<uint4*>(o_ + toff + (uint32_t)(2 * u) * p.pitch) = e_;          \
-            if (nvalid > 0 && y_ + 1 < yin) *reinterpret_cast<uint4*>(o_ + toff + (uint32_t)(2 * u + 1) * p.pitch) = d_;  \
-        }                                                                                                             \
-        return;                                                                                                       \
-    }
-    if (HGI_VAR_STOP_AFTER == 1) HGI_EARLY_STORE(sm.P[tid])
-#endif
 
     // ---- 3. coarse levels of the pass, s = F/2 .. 2 ---------------------------------------------
     if (F >= 16) coarse_level<MODE, INTERP, IDENTITY, 8>(sm, tid, qc, edge, xin, yin);
     if (F >= 8) coarse_level<MODE, INTERP, IDENTITY, 4>(sm, tid, qc, edge, xin, yin);
-#ifdef HGI_VAR_STOP_AFTER
-    if (HGI_VAR_STOP_AFTER == 2) HGI_EARLY_STORE(sm.P[plane_off(4) + tid] ^ sm.Q[plane_off(4) + tid])
-#endif
     uint32_t p2e[2] = {0u, 0u}, p2o[2] = {0u, 0u}, q2e[2] = {0u, 0u}, q2o[2] = {0u, 0u};
     if (OWN2) {
         level2_owner<MODE, INTERP, IDENTITY>(sm, ev[0], ev[1], sx, ry, qc, edge, xin, yin, p2e, p2o, q2e, q2o);
-        coarse_level<MODE, INTERP, IDENTITY, 2, NT, 0, false>(sm, tid, qc, edge, xin, yin);   // fringe cells + barrier
-    } else if (F >= 4) {
-        coarse_level<MODE, INTERP, IDENTITY, 2>(sm, tid, qc, edge, xin, yin);
+        coarse_level<MODE, INTERP, IDENTITY, 2, false>(sm, tid, qc, edge, xin, yin);   // fringe cells + barrier
     }
 
-#ifdef HGI_VAR_STOP_AFTER
-    if (HGI_VAR_STOP_AFTER == 3) HGI_EARLY_STORE(p2e[0] ^ p2o[1] ^ q2e[1] ^ q2o[0] ^ sm.P[plane_off(2) + tid])
-#endif
     // ---- 4. finest level: registers + P_2 / Q_2 -> HBM -------------------------------------------
     uint8_t* __restrict__ out = (MODE == kModeEncode ? p.grid_out : p.recon_out) + tile_off;
     uint32_t A[4], B[4], C[4], D[4];
@@ -451,7 +372,7 @@ __device__ __forceinline__ void tile_body(const PassArgs& p, FastSmem& sm, uint3
                     rec_od[k] = interleave(r[1], r[2]);
                 }
             } else {
-                const uint32_t pr = pred2<INTERP, true>(A[k], B[k], C[k], D[k], qc.one);
+                const uint32_t pr = pred2<INTERP>(A[k], B[k], C[k], D[k], qc.one);
                 out_ev[k] = pack_lo(A[k], decode2(a1, pr, qc.one));
                 out_od[k] = pack_lo(decode2(a2, pr, qc.one), decode2(a3, pr, qc.one));
             }
@@ -479,16 +400,11 @@ hgi_tile_fast_kernel(const PassArgs p)
     // bodies in one kernel its code is 43 KB and it runs 12 % slower, an instruction-cache effect
     constexpr bool kSplit = ((MODE == kModeDecode) || IDENTITY) && ALIGNED && NLEV == 4;
     if (kSplit) {
-#ifdef HGI_VAR_INTERIOR_BY_SIZE
-        const bool interior = (blockIdx.x + 1) * TW + FMAX + 1 <= p.w && (blockIdx.y + 1) * TH + FMAX + 1 <= p.h;
-#else
         const bool interior = blockIdx.x < p.fast_itx && blockIdx.y < p.fast_ity;   // the launcher's counts of interior tile columns / rows
-#endif
         if (interior) {
             tile_body<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 0>(p, sm, blockIdx.x, blockIdx.y);
             return;
         }
-#ifndef HGI_VAR_NO_LIGHT_RIGHT_BODY
         // the right tile column of a plane whose width is a multiple of the tile width: constant extents again (EDGE = 2;
         // 6 % of the tiles of a 1080p frame at the interior body's ~400 instructions per warp instead of the general
         // edge body's ~810: -0.7 % per light kernel in power-capped runs, nothing at full clock where they are DRAM-bound)
@@ -496,13 +412,6 @@ hgi_tile_fast_kernel(const PassArgs p)
             tile_body<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 2>(p, sm, blockIdx.x, blockIdx.y);
             return;
         }
-#endif
-#ifdef HGI_VAR_LIGHT_BOTTOM_BODY
-        if (blockIdx.x < p.fast_itx) {   // a bottom tile row under interior tile columns: constant column extents (EDGE = 3)
-            tile_body<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 3>(p, sm, blockIdx.x, blockIdx.y);
-            return;
-        }
-#endif
     }
     tile_body<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 1>(p, sm, blockIdx.x, blockIdx.y);
 }
@@ -511,9 +420,7 @@ hgi_tile_fast_kernel(const PassArgs p)
 // PART 1 = the interior tiles [0, fast_itx) x [0, fast_ity) with the predicate-free body;
 // PART 2 = the right tile columns [fast_itx, tiles_x) of the interior tile rows, general edge body;
 // PART 4 = the same when there is ONE right column and it is exactly TW wide (width % TW == 0): constants again;
-// PART 3 = the bottom tile rows [fast_ity, tiles_y), all columns, general edge body;
-// PART 5 + 6 (-DHGI_VAR_SPLIT_BOTTOM) = the bottom tile rows as interior columns (constant column extents, EDGE = 3) +
-//          right columns (general edge body).
+// PART 3 = the bottom tile rows [fast_ity, tiles_y), all columns, general edge body.
 template <int MODE, int INTERP, bool IDENTITY, bool EXTRA, int NLEV, bool ALIGNED, int PART>
 __global__ void __launch_bounds__(NT, (IDENTITY && !EXTRA && ALIGNED && NLEV == 4) ? HGI_FAST_MIN_BLOCKS_LIGHT : HGI_FAST_MIN_BLOCKS)
 hgi_tile_fast_part_kernel(const PassArgs p)
@@ -523,8 +430,6 @@ hgi_tile_fast_part_kernel(const PassArgs p)
     if (PART == 1) tile_body<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 0>(p, sm, blockIdx.x, blockIdx.y);
     else if (PART == 2) tile_body<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 1>(p, sm, p.fast_itx + blockIdx.x, blockIdx.y);
     else if (PART == 4) tile_body<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 2>(p, sm, p.fast_itx + blockIdx.x, blockIdx.y);
-    else if (PART == 5) tile_body<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 3>(p, sm, blockIdx.x, p.fast_ity + blockIdx.y);
-    else if (PART == 6) tile_body<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 1>(p, sm, p.fast_itx + blockIdx.x, p.fast_ity + blockIdx.y);
     else tile_body<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 1>(p, sm, blockIdx.x, p.fast_ity + blockIdx.y);
 }
 
@@ -565,13 +470,6 @@ cudaError_t launch_fast_split(PassArgs& a, uint32_t tiles_x, uint32_t tiles_y, c
             hgi_tile_fast_part_kernel<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 2><<<nb, NT, 0, es>>>(a); ++launch_count();
         }
     }
-#ifdef HGI_VAR_SPLIT_BOTTOM
-    if (nbr && a.fast_itx && ncr) {   // bottom tile rows: interior columns with constant column extents + the right columns
-        const dim3 nb5(a.fast_itx, nbr, a.n_images), nb6(ncr, nbr, a.n_images);
-        hgi_tile_fast_part_kernel<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 5><<<nb5, NT, 0, es>>>(a); ++launch_count();
-        hgi_tile_fast_part_kernel<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 6><<<nb6, NT, 0, es>>>(a); ++launch_count();
-    } else
-#endif
     if (nbr) {                 // bottom tile rows
         const dim3 nb(tiles_x, nbr, a.n_images);
         hgi_tile_fast_part_kernel<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 3><<<nb, NT, 0, es>>>(a); ++launch_count();
@@ -624,32 +522,11 @@ cudaError_t launch_fast_n(const PassArgs& args, cudaStream_t stream)
         a.fast_itx = a.w >= (uint32_t)(FMAX + 1) ? min(tiles_x, (a.w - (FMAX + 1)) / TW) : 0u;
         a.fast_ity = a.h >= (uint32_t)(FMAX + 1) ? min(tiles_y, (a.h - (FMAX + 1)) / TH) : 0u;
         a.fast_rcol = (a.fast_itx + 1 == tiles_x && a.w == tiles_x * (uint32_t)TW) ? 1u : 0u;   // ONE right column, exactly TW wide
-#ifdef HGI_VAR_SPLIT_LIGHT
-        // the light kernels as interior + right-column + bottom-row launches too (headline instantiations only)
-        constexpr bool kSplitLight = ALIGNED && NLEV == 4;
-#else
-        constexpr bool kSplitLight = false;
-#endif
-        const bool big = (uint64_t)tiles_x * tiles_y * a.n_images >= kSplitMinTiles;
         if (MODE == kModeDecode) {
-            if constexpr (kSplitLight && MODE == kModeDecode) {
-                if (big) {
-                    const cudaError_t es = launch_fast_split<kModeDecode, INTERP, true, false, NLEV, ALIGNED>(a, tiles_x, tiles_y, stream);
-                    if (es != cudaSuccess) return es;
-                    continue;
-                }
-            }
             hgi_tile_fast_kernel<kModeDecode, INTERP, true, false, NLEV, ALIGNED><<<nb, NT, 0, stream>>>(a); ++launch_count();
         } else {
             const bool extra = (a.recon_out != nullptr);
             const bool ident = (a.quant_error == 0);
-            if constexpr (kSplitLight && MODE == kModeEncode) {
-                if (ident && !extra && big) {
-                    const cudaError_t es = launch_fast_split<kModeEncode, INTERP, true, false, NLEV, ALIGNED>(a, tiles_x, tiles_y, stream);
-                    if (es != cudaSuccess) return es;
-                    continue;
-                }
-            }
             if (ident && !extra) { hgi_tile_fast_kernel<kModeEncode, INTERP, true, false, NLEV, ALIGNED><<<nb, NT, 0, stream>>>(a); ++launch_count(); }
             else if (ident) { hgi_tile_fast_kernel<kModeEncode, INTERP, true, true, NLEV, ALIGNED><<<nb, NT, 0, stream>>>(a); ++launch_count(); }
             else if constexpr (ALIGNED && NLEV == 4 && MODE == kModeEncode) {

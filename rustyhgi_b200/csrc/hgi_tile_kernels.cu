@@ -1,5 +1,5 @@
 // hgi_tile_kernels.cu -- generic (scalar, byte-wise) fused multi-level HGI tile kernel (sm_100a) + pass dispatch.
-// The SWAR kernels (hgi_tile_fast.cu, hgi_tile_tma.cu) share this decomposition; this file keeps the plain
+// The SWAR kernel (hgi_tile_fast.cu) shares this decomposition; this file keeps the plain
 // formulation that the CPU model tests/tile_model.py mirrors line by line.
 //
 // One launch ("pass") runs up to four consecutive levels of the closed loop for every 128x64
@@ -220,18 +220,11 @@ uint64_t& launch_count()
     return n;
 }
 
-cudaError_t launch_tile_pass(int mode, int interp, const PassArgs& a, cudaStream_t stream, int variant)
+cudaError_t launch_tile_pass(int mode, int interp, const PassArgs& a, cudaStream_t stream, bool generic)
 {
-    // SWAR kernels: the prefetch kernel takes any width / alignment and, as a strided lattice view, the D > 1 passes;
-    // the TMA kernel needs D == 1 and 16-byte rows.  Only planes taller than 65535 tiles stay on the generic kernel
-    if (variant != kTileGeneric && (a.hD + 63) / 64 <= 65535u) {
-        if (variant == kTileTma && a.vec_ok && a.d_log2 == 0 && a.pitch == a.w) {
-            bool used = false;
-            const cudaError_t e = launch_tile_pass_tma(mode, interp, a, stream, &used);
-            if (e != cudaSuccess || used) return e;
-        }
-        return launch_tile_pass_fast(mode, interp, a, stream);
-    }
+    // the SWAR kernel takes any width / alignment and, through a decimated copy of the lattice, the D > 1 passes.
+    // Only planes taller than 65535 tiles stay on the generic kernel
+    if (!generic && (a.hD + 63) / 64 <= 65535u) return launch_tile_pass_fast(mode, interp, a, stream);
     if (mode == kModeEncode)
         return interp == kInterpLeftTop ? launch_t<kModeEncode, kInterpLeftTop>(a, stream)
                                         : launch_t<kModeEncode, kInterpCrossed>(a, stream);

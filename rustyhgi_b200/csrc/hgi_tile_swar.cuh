@@ -1,15 +1,10 @@
 // hgi_tile_swar.cuh -- shared device code of the fast HGI tile kernels (sm_100a): dense per-level plane
 // geometry, 16-bit-lane SWAR arithmetic (predictor, quantizer, fix-up), plane staging and the coarse-level
-// routines.  Included by hgi_tile_fast.cu (register-prefetch kernel, 128x64 tiles, 128 threads) and
-// hgi_tile_tma.cu (persistent TMA-pipelined kernel, 128x128 tiles, 512 threads); each defines HGI_TILE_H /
-// HGI_TILE_NT before including this file.
+// routines of hgi_tile_fast.cu (register-prefetch kernel, 128x64 tiles, 128 threads).
 //
 // Reference semantics: src/encoder.rs:39-71, src/decoder.rs:18-46, src/utils.rs:11-41,
 // src/interpolator.rs:15-28,41-91, src/quantizator.rs:41-74.
 #pragma once
-#ifndef HGI_TILE_H
-#error "define HGI_TILE_H (64 or 128) before including hgi_tile_swar.cuh"
-#endif
 #include "hgi_device.cuh"
 #include "hgi_kernels.h"
 
@@ -17,18 +12,15 @@ namespace hgi {
 namespace {
 
 constexpr int TW = 128;                  // tile width  (lattice points)
-constexpr int TH = HGI_TILE_H;      // tile height: 64 or 128 (NU = TH/64 16x2 units per thread)
-#ifndef HGI_TILE_NT
-#define HGI_TILE_NT 256
-#endif
-constexpr int NT = HGI_TILE_NT;          // threads per CTA (128, 256 or 512)
+constexpr int TH = 64;                   // tile height
+constexpr int NT = 128;                  // threads per CTA
 constexpr int NU = TH * 4 / NT;          // 16x2-pixel units per thread in the finest level
 constexpr int RPB = NT / 8;              // row pairs covered by one unit block (8 column strips x RPB row pairs)
 constexpr int NWARPS = NT / 32;
 constexpr int FMAX = 1 << kMaxPassLevels;
 constexpr uint32_t M16 = 0x00FF00FFu;
 
-static_assert(TW == 128 && (TH == 64 || TH == 128) && NU >= 1 && NU * NT == TH * 4 && NT >= 128, "thread mapping assumes 128-wide tiles");
+static_assert(TW == 128 && NU == 2 && NU * NT == TH * 4, "thread mapping assumes 128x64 tiles, two units per thread");
 
 // Dense level planes.  P_s holds lattice-s points of the tile + halo: columns 0..TW/s+1,
 // rows 0..TH/s+1 (the last ones are only partially needed, see fringe_cell).
@@ -40,7 +32,7 @@ __host__ __device__ constexpr int plane_off(int s)
     return s == 2 ? 0 : (s == 4 ? plane_bytes(2) : (s == 8 ? plane_bytes(2) + plane_bytes(4)
                                                                : plane_bytes(2) + plane_bytes(4) + plane_bytes(8)));
 }
-constexpr int PLANE_BYTES = plane_bytes(2) + plane_bytes(4) + plane_bytes(8) + plane_bytes(16);  // 4544 (TH=64) / 8704 (TH=128)
+constexpr int PLANE_BYTES = plane_bytes(2) + plane_bytes(4) + plane_bytes(8) + plane_bytes(16);  // 4544
 
 // Highest tile-relative coordinate at which a new point of sub-step s is still needed (see DESIGN.md 4.1):
 // TW-1, TW, TW+s for s = 1, 2, >= 4.  Used as compile-time constants in fringe_cell().
@@ -90,17 +82,6 @@ __device__ __forceinline__ uint32_t fadd(uint32_t a, uint32_t b, uint32_t one)
     asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(one), "r"(b));
     return r;
 }
-// pk for encode2: per lane 256 - p.  The predictor may keep stray bits 14/15 in lane 0 (pred2<.., DIRTY>), so the
-// subtraction must not borrow across the lanes: ~p (as p * -1 - 1 on the FMA pipe, opaque -1) plus 257 with a
-// lane-wise add (VIADD.16x2).  The strays survive in pk and dd but sit above bit 8 and below the next lane.
-constexpr bool kDirtyEncodePred = true;
-__device__ __forceinline__ uint32_t bias_sub(uint32_t p, uint32_t one)
-{
-    uint32_t np, r;
-    asm("mad.lo.u32 %0, %1, %2, %2;" : "=r"(np) : "r"(p), "r"(0u - one));
-    asm("add.u16x2 %0, %1, %2;" : "=r"(r) : "r"(np), "r"(0x01010101u));
-    return r;
-}
 // ---- fp16x2 arithmetic on integer lanes ------------------------------------------------------------------------
 // A 16-bit lane that holds an integer n < 2048 is, read as an fp16 bit pattern, the number n * 2^-24 (subnormals and
 // the first normal binade share the ulp 2^-24; sm_100 does not flush them).  HFMA2 therefore does exact integer
@@ -121,10 +102,6 @@ __device__ __forceinline__ uint32_t hmul2(uint32_t a, uint32_t b)
     asm("mul.rn.f16x2 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b));
     return r;
 }
-constexpr uint32_t kH_eighth = 0x30003000u;       // 0.125
-constexpr uint32_t kH_neg_eighth = 0xB000B000u;   // -0.125
-constexpr uint32_t kH_511ulp = 0x01FF01FFu;       // 511 * 2^-24
-constexpr uint32_t kH_257ulp = 0x01010101u;       // 257 * 2^-24
 constexpr uint32_t kH_255_256 = 0x3BF83BF8u;      // 255/256: 0x0100 -> 0x00FF per lane
 
 // Crossed predictor for the quantizing encode: returns pk = 256 - pred per lane and, if WANT_P, p = pred + 512 (the
@@ -149,24 +126,12 @@ __device__ __forceinline__ uint32_t pred_pk2(uint32_t A, uint32_t B, uint32_t C,
         asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(pk) : "r"(A), "r"(0u - one), "r"(0x01000100u));
         return pk;
     }
-#ifdef HGI_VAR_PRED_YB
-    const uint32_t x1 = (A ^ B) & 0x00010001u;
-    const uint32_t w = x1 & (C ^ D) & (A ^ C);
-    uint32_t t2, yb;
-    const uint32_t t3 = fadd(fadd(A, B, one), C, one);                         // two IMADs: one instruction more, but off the ALU pipe (-0.7 %, A/B)
-    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(t2) : "r"(D), "r"(one + one), "r"(0x00070007u));
-    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(t2) : "r"(t3), "r"(one + one), "r"(t2));
-    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(yb) : "r"(w), "r"(4u * one), "r"(t2));
-    if (WANT_P) p = hfma2(yb, kH_eighth, kH_511ulp);
-    return hfma2(yb, kH_neg_eighth, kH_257ulp);
-#else
     const uint32_t va = fadd(A, B, one), vc = fadd(C, D, one);                 // column sums, lanes <= 510
     const uint32_t w = ((A ^ C) & 0x00010001u) & va & vc;                      // two LOP3
     uint32_t m = fadd(va, vc, one);                                            // T
     asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(m) : "r"(w), "r"(one + one), "r"(m));   // T + 2w <= 1022
     if (WANT_P) p = hfma2(m, kH_quarter_lo, kH_512ulp);
     return hfma2(m, kH_neg_quarter_lo, kH_256ulp);
-#endif
 }
 
 // src/interpolator.rs:43-54 per lane.  With avg(x,y) = (x+y+1)>>1 = (x + y + ((x^y)&1)) / 2, the sum of the
@@ -175,30 +140,17 @@ __device__ __forceinline__ uint32_t pred_pk2(uint32_t A, uint32_t B, uint32_t C,
 //     pred = (((T + 1) >> 1) + w) >> 1,    w = (A^B) & (C^D) & (A^C) & 1
 // (E/2 only matters when it makes T+E/2 cross a multiple of 4: T odd -> the +1; T = 2 mod 4 with all
 // three parity tests true -> the w).  Checked against the four-average form in tests/test_swar_model.py.
-// 6 ALU-pipe operations per register (two cells) instead of 16.
-// DIRTY: the caller only consumes the low byte of each lane (decode), so the final mask is
-// skipped and the lanes keep stray bits 14/15 (they never reach a low byte: every later sum stays below 2^16).
-template <int INTERP, bool DIRTY = false>
+// pred == (T + 1 + 2w) >> 2, computed with the division of pred_pk2: RN(m (1/4 - 2^-13)) with m = T + 2w.  Clean
+// lanes; 2 ALU-pipe and 5 FMA-pipe operations per register (two cells) instead of 16 for the four averages.
+template <int INTERP>
 __device__ __forceinline__ uint32_t pred2(uint32_t A, uint32_t B, uint32_t C, uint32_t D, uint32_t one)
 {
     if (INTERP == kInterpLeftTop) return A;                                    // src/interpolator.rs:26
-#ifndef HGI_VAR_PRED2_SHIFT
-    {   // the same division as pred_pk2: RN(m (1/4 - 2^-13)) = (m + 1) >> 2, clean lanes; 2 ALU + 5 FMA instead of 5 + 4
-        const uint32_t va = fadd(A, B, one), vc = fadd(C, D, one);
-        const uint32_t w = ((A ^ C) & 0x00010001u) & va & vc;
-        uint32_t m = fadd(va, vc, one);
-        asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(m) : "r"(w), "r"(one + one), "r"(m));
-        return hfma2(m, kH_quarter_lo, 0u);
-    }
-#endif
-    const uint32_t x1 = (A ^ B) & 0x00010001u;
-    const uint32_t w = x1 & (C ^ D) & (A ^ C);
-    // (((T + 1) >> 1) + w) >> 1 == (T + 1 + 2 w) >> 2: the doubling rides on the multiply-add, one shift instead of two
-    const uint32_t t1 = fadd(fadd(A, B, one), fadd(C, D + 0x00010001u, one), one);       // lanes <= 1021
-    uint32_t r;
-    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(w), "r"(one + one), "r"(t1));       // lanes <= 1023
-    r >>= 2;                                                                   // :51 (+ stray bits 14, 15 in lane 0)
-    return DIRTY ? r : (r & M16);
+    const uint32_t va = fadd(A, B, one), vc = fadd(C, D, one);
+    const uint32_t w = ((A ^ C) & 0x00010001u) & va & vc;
+    uint32_t m = fadd(va, vc, one);
+    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(m) : "r"(w), "r"(one + one), "r"(m));
+    return hfma2(m, kH_quarter_lo, 0u);
 }
 
 // Linear quantizer as an exact per-lane multiply-shift: ((d + e) / scale) * scale for d in 0..255.
@@ -274,11 +226,8 @@ __host__ inline void fill_quant_args(PassArgs& a)
 // src/encoder.rs:52-64 for two pixels.  Returns the symbols; `recon` = what the decoder rebuilds.
 // p, pk = 256 - p: clean lanes (pred_pk2).  Quantizer (src/quantizator.rs:50-60) on the FMA pipe: two HFMA2, see
 // QuantSwar; the lanes of q come out as plain integers.
-#ifndef HGI_VAR_INTQ
-#ifndef HGI_VAR_HMUL_MASKS
-#define HGI_VAR_HMUL_MASKS 2     // of the three fix-up masks per cell pair, how many are built on the FMA pipe (HMUL2) instead of the ALU pipe (VIMNMX)
-#endif
-template <bool IDENTITY, bool FMA_MASK = false>
+// FMA_MASK: the fix-up mask is built on the FMA pipe (HMUL2) instead of the ALU pipe (VIMNMX).
+template <bool IDENTITY, bool FMA_MASK>
 __device__ __forceinline__ uint32_t encode2(uint32_t a, uint32_t p, uint32_t pk, const QuantSwar& qc, uint32_t& recon)
 {
     const uint32_t dd = fadd(a, pk, qc.one);          // per lane a + 256 - p: low byte = the residual, bit 8 = [a >= p]
@@ -308,48 +257,11 @@ __device__ __forceinline__ void encode_cells(uint32_t A, uint32_t B, uint32_t C,
 {
     uint32_t p = 0u;
     const uint32_t pk = pred_pk2<INTERP, !IDENTITY>(A, B, C, D, qc.one, p);
-    q[0] = encode2<IDENTITY, (HGI_VAR_HMUL_MASKS > 0)>(a1, p, pk, qc, r[0]);
-    q[1] = encode2<IDENTITY, (HGI_VAR_HMUL_MASKS > 1)>(a2, p, pk, qc, r[1]);
-    q[2] = encode2<IDENTITY, (HGI_VAR_HMUL_MASKS > 2)>(a3, p, pk, qc, r[2]);
+    // two of the three fix-up masks on the FMA pipe balance it best against the ALU pipe (profiles/r02_fast_tile_kernel.md)
+    q[0] = encode2<IDENTITY, true>(a1, p, pk, qc, r[0]);
+    q[1] = encode2<IDENTITY, true>(a2, p, pk, qc, r[1]);
+    q[2] = encode2<IDENTITY, false>(a3, p, pk, qc, r[2]);
 }
-#else
-// round-1 form (A/B variant): integer multiply-shift quantizer, predictor lanes with stray bits
-template <bool IDENTITY>
-__device__ __forceinline__ uint32_t encode2(uint32_t a, uint32_t p, uint32_t pk, const QuantSwar& qc, uint32_t& recon)
-{
-    const uint32_t dd = fadd(a, pk, qc.one);                  // pk = 0x01000100 - p: per lane a + 256 - p, bit 8 = [a >= p]
-    if (IDENTITY) {
-        recon = a;                                    // p + (a - p) == a
-        return dd;                                    // low byte of each lane = the symbol; packed with pack_lo()
-    }
-    const uint32_t d = dd & M16;                      // :53 wrapping_sub
-    const uint32_t t = d * qc.mul + qc.add;           // lanes: (d + e) * k + c  < 2^16
-    // r = t >> shift per lane, q = r * scale -- done as one high multiply on the masked quotient bits, which
-    // moves the shift off the ALU pipe: ((r << n) * (scale << (32 - n))) >> 32 == r * scale in both lanes
-    uint32_t q = __umulhi(t & qc.rmask, qc.qmul);     // :54 table[d]
-    const uint32_t ov = fadd(q, p, qc.one);                   // bit 8 = overflow                      (:56)
-    // overflow_is_expected = [a < p] = !bit8(dd)  =>  mismatch iff bit8(ov) == bit8(dd)       (:57-58)
-    const uint32_t x = ~(ov ^ dd) & 0x01000100u;
-    uint32_t m;                                       // 0x00FF in every mismatching lane: per-lane min(0x0100, 0x00FF),
-    asm("min.u16x2 %0, %1, %2;" : "=r"(m) : "r"(x), "r"(0x00FF00FFu));   // one VIMNMX.U16x2 instead of shift + subtract
-    q = (q & ~m) | (dd & m);                          // :59 (m only covers the low byte of a lane, so dd's flag bit drops out: one LOP3)
-    // :63 (p + q) mod 256.  p + d == a (mod 256) and, once the fix-up has run, a + (q - d) stays inside 0..255
-    // (that is exactly what the overflow test guards), so the lanes need neither a borrow nor a mask.
-    recon = a + q - d;
-    return q;
-}
-
-template <int INTERP, bool IDENTITY>
-__device__ __forceinline__ void encode_cells(uint32_t A, uint32_t B, uint32_t C, uint32_t D, uint32_t a1, uint32_t a2, uint32_t a3,
-                                             const QuantSwar& qc, uint32_t (&q)[3], uint32_t (&r)[3])
-{
-    const uint32_t p = pred2<INTERP, kDirtyEncodePred>(A, B, C, D, qc.one);
-    const uint32_t pk = bias_sub(p, qc.one);
-    q[0] = encode2<IDENTITY>(a1, p, pk, qc, r[0]);
-    q[1] = encode2<IDENTITY>(a2, p, pk, qc, r[1]);
-    q[2] = encode2<IDENTITY>(a3, p, pk, qc, r[2]);
-}
-#endif
 
 // src/decoder.rs:39 for two pixels; the low byte of each lane is the pixel (pack with pack_lo())
 __device__ __forceinline__ uint32_t decode2(uint32_t g, uint32_t p, uint32_t one) { return fadd(p, g, one); }
@@ -409,7 +321,7 @@ __device__ __forceinline__ void level_word(FastSmem& sm, int g, int cy, const Qu
     uint32_t* pev = reinterpret_cast<uint32_t*>(Ps + (2 * cy) * ps + 4 * g);
     uint32_t* pod = reinterpret_cast<uint32_t*>(Ps + (2 * cy + 1) * ps + 4 * g);
     const uint32_t ev = *pev, od = *pod;
-    const uint32_t a1 = lanes_odd(ev), a2 = lanes_even(od), a3 = lanes_odd(od);   // clean: p may be dirty, the sums must stay < 2^16
+    const uint32_t a1 = lanes_odd(ev), a2 = lanes_even(od), a3 = lanes_odd(od);   // clean lanes: the sums must stay < 2^16
     uint32_t r[3];
     if (MODE == kModeEncode) {
         uint32_t q[3];
@@ -420,7 +332,7 @@ __device__ __forceinline__ void level_word(FastSmem& sm, int g, int cy, const Qu
         *reinterpret_cast<uint32_t*>(Qs + (2 * cy) * ps + 4 * g) = pack_even_row(qcw, q[0], false);
         *reinterpret_cast<uint32_t*>(Qs + (2 * cy + 1) * ps + 4 * g) = pack_sym<IDENTITY>(q[1], q[2]);
     } else {
-        const uint32_t p = pred2<INTERP, true>(A, B, C, D, qc.one);   // no consumer needs clean predictor lanes
+        const uint32_t p = pred2<INTERP>(A, B, C, D, qc.one);
         r[0] = decode2(a1, p, qc.one);
         r[1] = decode2(a2, p, qc.one);
         r[2] = decode2(a3, p, qc.one);
@@ -467,7 +379,7 @@ __device__ __forceinline__ void level2_owner(FastSmem& sm, const uint4& r0, cons
             q2e[k] = pack_even_row(qcw, q[0], k != 0);
             q2o[k] = pack_sym<IDENTITY>(q[1], q[2]);
         } else {
-            const uint32_t p = pred2<INTERP, true>(A, B, C, D, qc.one);
+            const uint32_t p = pred2<INTERP>(A, B, C, D, qc.one);
             r[0] = decode2(a1, p, qc.one);
             r[1] = decode2(a2, p, qc.one);
             r[2] = decode2(a3, p, qc.one);
@@ -515,14 +427,10 @@ __device__ __forceinline__ void fringe2_word(FastSmem& sm, int it, const QuantSw
     if (MODE == kModeEncode) {
         uint32_t p = 0u;
         const uint32_t pk = pred_pk2<INTERP, !IDENTITY>(A, B, C, D, qc.one, p);
-#ifndef HGI_VAR_INTQ
         (void)encode2<IDENTITY, false>(a, p, pk, qc, r);
-#else
-        (void)encode2<IDENTITY>(a, p, pk, qc, r);
-#endif
         wev = interleave(A, r);
     } else {
-        r = decode2(a, pred2<INTERP, true>(A, B, C, D, qc.one), qc.one);
+        r = decode2(a, pred2<INTERP>(A, B, C, D, qc.one), qc.one);
         wev = pack_lo(A, r);
     }
     if (edge) {   // out-of-image reconstruction must read as 0 (src/interpolator.rs:75-82)
@@ -574,42 +482,24 @@ __device__ __forceinline__ void fringe_cell(FastSmem& sm, int cx, int cy, const 
 }
 
 // One coarse level (sub-step S >= 2) of the tile: SWAR words over the tile's own cells on the low
-// threads, the fringe cells (cell column TW/(2S), cell row TH/(2S)) on the high threads.
-// Barrier over `GS` threads: the whole CTA (BAR == 0) or a named barrier shared by one warp group.
-template <int GS, int BAR>
-__device__ __forceinline__ void group_sync()
-{
-    if (BAR == 0) __syncthreads();
-    else asm volatile("bar.sync %0, %1;" ::"n"(BAR), "n"(GS) : "memory");
-}
-
-// `tid` in [0, GS) is the thread's index inside the group that runs the coarse levels (default: the whole CTA).
+// threads, the fringe cells (cell column TW/(2S), cell row TH/(2S)) on the high threads; ends with a CTA barrier.
 // The fringe (cell column TW/(2S) and cell row TH/(2S), needed by the finer levels of this tile) is computed as
 // ordinary SWAR words: word column `wpr` and cell row `ncy` extend the loop.  Their second cell / odd row reaches
 // two plane columns (one plane row) further than any consumer reads -- inside the plane pitch, computed from stale
 // bytes, never used.
 // WORDS = false: only the fringe words (the caller has run the tile's own cells itself, see level2_owner).
-template <int MODE, int INTERP, bool IDENTITY, int S, int GS = NT, int BAR = 0, bool WORDS = true>
+template <int MODE, int INTERP, bool IDENTITY, int S, bool WORDS = true>
 __device__ __forceinline__ void coarse_level(FastSmem& sm, int tid, const QuantSwar& qc, bool edge, int xin, int yin)
 {
     constexpr int wpr = TW / (4 * S);               // SWAR words per cell row (2 cells each)
     constexpr int ncy = TH / (2 * S), ncx = TW / (2 * S);
     const int xin_s = (int)(((uint32_t)xin + S - 1) / (uint32_t)S), yin_s = (int)(((uint32_t)yin + S - 1) / (uint32_t)S);
-#ifdef HGI_VAR_SCALAR_FRINGE
-    constexpr bool kScalarFringe = true;
-#elif defined(HGI_VAR_WORD_FRINGE_ALL)
-    constexpr bool kScalarFringe = false;
-#else
     // the identity encode's s = 2 fringe stays scalar: one point per cell without a quantizer is ~35 instructions on
     // two warps, cheaper for that latency-bound kernel than 32 full words on one warp (A/B)
     constexpr bool kScalarFringe = !WORDS && IDENTITY && MODE == kModeEncode;
-#endif
     if (kScalarFringe) {
         constexpr int nfr = (ncy + 1) + ncx;
-        if (WORDS)
-            for (int it = tid; it < wpr * ncy; it += GS)
-                level_word<MODE, INTERP, IDENTITY, S>(sm, it % wpr, it / wpr, qc, edge, xin_s, yin_s);
-        for (int it = GS - 1 - tid; it < nfr; it += GS) {
+        for (int it = NT - 1 - tid; it < nfr; it += NT) {
             const int cx = it <= ncy ? ncx : it - (ncy + 1);
             const int cy = it <= ncy ? it : ncy;
             if (2 * cx < xin_s && 2 * cy < yin_s)
@@ -619,7 +509,7 @@ __device__ __forceinline__ void coarse_level(FastSmem& sm, int tid, const QuantS
         }
     } else if (WORDS) {
         constexpr int wx = wpr + 1, nwords = wx * (ncy + 1);
-        for (int it = tid; it < nwords; it += GS) {
+        for (int it = tid; it < nwords; it += NT) {
             const int cy = (int)((uint32_t)it / (uint32_t)wx);
             level_word<MODE, INTERP, IDENTITY, S>(sm, it - cy * wx, cy, qc, edge, xin_s, yin_s);
         }
@@ -628,18 +518,14 @@ __device__ __forceinline__ void coarse_level(FastSmem& sm, int tid, const QuantS
         // (32 words = one warp at S = 2); of the corner cell only the lattice point itself is read by anyone: a copy of
         // the coarser plane's byte (0 when out of the image)
         constexpr int nfw = wpr + ncy;
-        for (int it = GS - 1 - tid; it < nfw; it += GS) {
-#ifdef HGI_VAR_FULL_FRINGE2
-            level_word<MODE, INTERP, IDENTITY, S>(sm, it < wpr ? it : wpr, it < wpr ? ncy : it - wpr, qc, edge, xin_s, yin_s);
-#else
+        for (int it = NT - 1 - tid; it < nfw; it += NT) {
             if (S == 2) fringe2_word<MODE, INTERP, IDENTITY>(sm, it, qc, edge, xin_s, yin_s);
             else level_word<MODE, INTERP, IDENTITY, S>(sm, it < wpr ? it : wpr, it < wpr ? ncy : it - wpr, qc, edge, xin_s, yin_s);
-#endif
         }
-        if (tid == GS - 1)
+        if (tid == NT - 1)
             (sm.P + plane_off(S))[(2 * ncy) * plane_pitch(S) + 4 * wpr] = (sm.P + plane_off(2 * S))[ncy * plane_pitch(2 * S) + 2 * wpr];
     }
-    group_sync<GS, BAR>();
+    __syncthreads();
 }
 
 }  // namespace

@@ -13,7 +13,7 @@ from oracle import c as oc
 from rustyhgi_b200 import cli
 
 pytestmark = pytest.mark.gpu
-PATHS = {"tile": hgi.PATH_TILE, "generic": hgi.PATH_TILE_GENERIC, "tma": hgi.PATH_TILE_TMA}
+PATHS = {"tile": hgi.PATH_TILE, "generic": hgi.PATH_TILE_GENERIC}
 INTERPS = {"crossed": (hgi.Crossed, oc.INTERP_CROSSED), "lefttop": (hgi.LeftTop, oc.INTERP_LEFTTOP)}
 
 

@@ -16,7 +16,7 @@ def ref_pred(A, B, C, D):
     return (avg(A, B) + avg(D, C) + avg(C, A) + avg(D, B)) >> 2
 
 
-def swar_pred(A, B, C, D):                                    # pred2<Crossed>, -DHGI_VAR_PRED2_SHIFT (integer shift form)
+def swar_pred(A, B, C, D):                                    # pred2<Crossed> of round 1 (integer shift form)
     x1 = (A ^ B) & 0x00010001
     w = x1 & (C ^ D) & (A ^ C)
     t1 = (A + B + C) + (D + 0x00010001)                       # T + 1 per lane
@@ -38,7 +38,7 @@ QUANT = {10: (195, 195, 12), 20: (25, 0, 10), 30: (67, 67, 12)}   # quant_swar()
 
 
 def swar_encode2(a, p, error):
-    """encode2<false>: returns (q lanes, recon lanes)."""
+    """encode2<false> of round 1 (integer multiply-shift quantizer): returns (q lanes, recon lanes)."""
     k, c, n = QUANT[error]
     scale = 2 * error + 1
     add = ((error * k + c) * 0x00010001) & U32
@@ -105,7 +105,7 @@ def test_pack_lo_drops_the_carry_bits():
 
 
 def test_dirty_predictor_lanes_are_harmless_for_decode():
-    """Decode skips the predictor's final mask (pred2<.., DIRTY>): the lanes then carry stray bits 14/15 (lane 1's low bits after the >> 2), which
+    """Round 1's decode skipped the shift-form predictor's final mask: the lanes then carry stray bits 14/15 (lane 1's low bits after the >> 2), which
     must never reach a low byte nor carry into the other lane when a clean residual lane is added."""
     rng = np.random.default_rng(7)
     for _ in range(20000):
@@ -141,7 +141,7 @@ def test_pack_even_row_selectors():
 
 
 def test_lanewise_bias_tolerates_dirty_predictor_lanes():
-    """bias_sub: pk = ~p + 257 per 16-bit lane (mad.lo with -1, then add.u16x2).  With stray bits 14/15 in lane 0 of
+    """Round 1's bias_sub: pk = ~p + 257 per 16-bit lane (mad.lo with -1, then add.u16x2).  With stray bits 14/15 in lane 0 of
     the predictor, dd = a + pk still has the residual in its low byte, [a >= p] in bit 8, and lane 1 untouched; the
     overflow sum q + p keeps its bit 8 too."""
     def add16x2(x, y):
@@ -188,12 +188,13 @@ def f16_quant_constants(error):
             _f2h(inv_ulp * scale * 2.0 ** -24), _f2h(-1024.0 * scale * 2.0 ** -24))
 
 
+# H_EIGHTH .. H_257ULP belong to round 2's first predictor form (fp16_pred_pk_yb), the others to the kernel
 H_EIGHTH, H_NEG_EIGHTH, H_511ULP, H_257ULP, H_255_256 = 0x3000, 0xB000, 0x01FF, 0x0101, 0x3BF8
 H_QUARTER_LO, H_NEG_QUARTER_LO, H_512ULP, H_256ULP = 0x33FF, 0xB3FF, 0x0200, 0x0100
 
 
 def fp16_pred_pk_yb(A, B, C, D):
-    """pred_pk2<Crossed>, -DHGI_VAR_PRED_YB (the first fp16 form): lanes 2T + 4w + 7, times 1/8."""
+    """pred_pk2<Crossed> of round 2's first fp16 form: lanes 2T + 4w + 7, times 1/8."""
     x1 = (A ^ B) & 0x00010001
     w = x1 & (C ^ D) & (A ^ C)
     yb = (2 * (A + B + C) + 2 * D + 0x00070007 + 4 * w) & U32

@@ -1,27 +1,15 @@
 #!/bin/bash
 # Build a kernel variant of libhgi_b200.so for tools/ab_bench.py:  tools/build_variant.sh NAME [-DFLAG ...]
-# Recompiles the tile kernels with the extra flags into build/NAME/ and links them with the stock objects.
-# A/B hooks in the kernels (each restores the behaviour a change replaced, or cuts the kernel for timing):
-#   -DHGI_VAR_NO_OPAQUE_SMEM     shared-memory window base rebuilt in every basic block (ptxas default)
-#   -DHGI_VAR_NO_ASSUME          no __builtin_assume on the thread index
-#   -DHGI_VAR_NO_OWN2            s = 2 level through shared memory (level_word) instead of level2_owner
-#   -DHGI_VAR_SCALAR_FRINGE      fringe cells as scalar code;  -DHGI_VAR_WORD_FRINGE_ALL  as SWAR words everywhere
+# Recompiles the fast tile kernel with the extra flags into build/NAME/ and links it with the stock objects.
+# Compile-time hooks of the kernel:
 #   -DHGI_FAST_MIN_BLOCKS=n / -DHGI_FAST_MIN_BLOCKS_LIGHT=n   CTAs per SM (quantizing encode / light kernels)
-#   -DHGI_FAST_TILE_H=128 -DHGI_FAST_NT=256                   tile shape / CTA size
-#   -DHGI_VAR_STOP_AFTER=1|2|3   cut after set-up / s=8,4 / s=2 and copy the pixels out (tools/time_encode.py)
-#   -DHGI_VAR_PRED_YB            predictor lanes 2T + 4w + 7 times 1/8 (first fp16 form);  -DHGI_VAR_PRED2_SHIFT  decode predictor as an integer shift
-#   -DHGI_VAR_FULL_FRINGE2       s = 2 fringe as full SWAR words (three points per cell) instead of fringe2_word
-#   -DHGI_VAR_HALO_TWO_WARPS[_DECODE]   halo chunks fetched by whole warps 1 and 2
-#   -DHGI_VAR_STCS / -DHGI_VAR_STCG     streaming / L2-only stores of the output chunks
-#   -DHGI_VAR_SPLIT_LIGHT        decode and the identity encode as interior + edge launches too;  -DHGI_VAR_SPLIT_BOTTOM  bottom rows of the quantizing encode as two launches
-#   -DHGI_VAR_NO_LIGHT_RIGHT_BODY / -DHGI_VAR_LIGHT_BOTTOM_BODY / -DHGI_VAR_INTERIOR_BY_SIZE / -DHGI_VAR_HALO_WARP_DECODE   bodies and roles of the light kernels
-#   -DHGI_VAR_HMUL_MASKS=n, -DHGI_VAR_INTQ, -DHGI_VAR_POISON_SMEM=0xXX   see hgi_tile_swar.cuh / hgi_tile_fast.cu
+#   -DHGI_VAR_POISON_SMEM=0xXX   the shared-memory planes start as this byte pattern (see hgi_tile_fast.cu)
 # Run-time knobs for tools/ab_bench.py (name=lib.so,ENV=VALUE): HGI_B200_PREFETCH, HGI_B200_SPLIT_MIN
 set -e
 cd "$(dirname "$0")/../rustyhgi_b200/csrc"
 name=$1; shift
 out=../../build/$name; mkdir -p $out
 NV="/usr/local/cuda/bin/nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -Xcompiler -fPIC -fmad=false"
-for f in hgi_tile_fast hgi_tile_tma; do $NV "$@" -c -o $out/$f.o $f.cu & done; wait
-$NV -shared -cudart static -o ../../build/libhgi_$name.so $out/hgi_tile_fast.o $out/hgi_tile_tma.o hgi_capi.o hgi_tile_kernels.o hgi_level_kernels.o hgi_reduce_kernels.o hgi_archive.o -lz
+$NV "$@" -c -o $out/hgi_tile_fast.o hgi_tile_fast.cu
+$NV -shared -cudart static -o ../../build/libhgi_$name.so $out/hgi_tile_fast.o hgi_capi.o hgi_tile_kernels.o hgi_level_kernels.o hgi_reduce_kernels.o hgi_region.o hgi_archive.o -lz
 echo built build/libhgi_$name.so

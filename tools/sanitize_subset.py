@@ -4,7 +4,7 @@
     compute-sanitizer --tool memcheck|racecheck|initcheck python tools/sanitize_subset.py [--light]
 
 Touches every kernel of libhgi_b200.so through the C ABI -- fast tile kernel (interior + edge launches, all level
-counts, aligned / unaligned / pitched planes), TMA kernel, generic kernel, per-level kernels, decimated coarse passes,
+counts, aligned / unaligned / pitched planes), generic kernel, per-level kernels, decimated coarse passes,
 histogram, RLE token table, RGB->luma, error metrics -- and checks each result against the oracle."""
 import argparse
 import os
@@ -41,7 +41,7 @@ def check(ctx, img, levels, q, interp=hgi.Crossed):
     n_checked += 1
 
 
-paths = {"tile": hgi.PATH_TILE, "tma": hgi.PATH_TILE_TMA, "generic": hgi.PATH_TILE_GENERIC, "level": hgi.PATH_PER_LEVEL}
+paths = {"tile": hgi.PATH_TILE, "generic": hgi.PATH_TILE_GENERIC, "level": hgi.PATH_PER_LEVEL}
 ctxs = {k: hgi.Context(0, v) for k, v in paths.items()}
 lena = get_plane("lena_tif")
 for name, ctx in ctxs.items():
@@ -53,7 +53,6 @@ for name, ctx in ctxs.items():
 big = photo_like(640, 400, 5) if a.light else get_plane("fullhd")
 check(ctxs["tile"], big, 4, 2)
 check(ctxs["tile"], big, 4, 0)
-check(ctxs["tma"], big, 4, 2)
 check(ctxs["tile"], photo_like(700, 530, 6) if a.light else photo_like(2368, 1400, 6), 6, 3)      # decimated coarse pass
 check(ctxs["tile"], photo_like(300, 1100, 9), 9, 2)                                                 # three passes
 
