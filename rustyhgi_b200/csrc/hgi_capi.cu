@@ -4,6 +4,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <new>
 #include <vector>
 
@@ -66,9 +67,7 @@ struct Scratch {
 
 struct Slot {
     cudaStream_t stream = nullptr;
-    DevBuf in, out, aux;
-    uint32_t* hist = nullptr;
-    size_t hist_cap = 0;
+    DevBuf in, out, aux, hist;
     Scratch scratch;
 };
 
@@ -140,10 +139,15 @@ struct hgi_pool {
 
 namespace {
 
+// Scope of one context's work: makes its device current (the caller's device is restored at the end) and charges the
+// kernels launched inside the scope to it (hgi_ctx_kernel_launches).  Scopes nest: an inner scope takes its kernels
+// out of hgi::launch_count(), so the outer one does not charge them again.
 struct DeviceGuard {
+    hgi_ctx* ctx;
     int prev = -1;
     bool ok = true;
-    explicit DeviceGuard(hgi_ctx* ctx)
+    const uint64_t launched = hgi::launch_count();
+    explicit DeviceGuard(hgi_ctx* c) : ctx(c)
     {
         if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
         if (prev != ctx->device) {
@@ -153,6 +157,8 @@ struct DeviceGuard {
     }
     ~DeviceGuard()
     {
+        ctx->launches += hgi::launch_count() - launched;
+        hgi::launch_count() = launched;
         if (prev >= 0) cudaSetDevice(prev);
     }
 };
@@ -187,16 +193,48 @@ int reserve(hgi_ctx* ctx, DevBuf& b, size_t bytes)
     return HGI_OK;
 }
 
+void free_bufs(std::initializer_list<DevBuf*> bufs)
+{
+    for (DevBuf* b : bufs) {
+        if (b->p) cudaFree(b->p);
+        *b = DevBuf{};
+    }
+}
+
+void destroy_side(Scratch& sc)
+{
+    if (sc.side) cudaStreamDestroy(sc.side);
+    if (sc.ev_fork) cudaEventDestroy(sc.ev_fork);
+    if (sc.ev_join) cudaEventDestroy(sc.ev_join);
+    sc.side = nullptr;
+    sc.ev_fork = sc.ev_join = nullptr;
+}
+
 void free_scratch(Scratch& sc)
 {
-    for (auto& b : sc.compact) if (b.p) { cudaFree(b.p); b = DevBuf{}; }
-    if (sc.dec_in.p) { cudaFree(sc.dec_in.p); sc.dec_in = DevBuf{}; }
-    if (sc.level_recon.p) { cudaFree(sc.level_recon.p); sc.level_recon = DevBuf{}; }
-    if (sc.region_in.p) { cudaFree(sc.region_in.p); sc.region_in = DevBuf{}; }
-    if (sc.region_out.p) { cudaFree(sc.region_out.p); sc.region_out = DevBuf{}; }
-    if (sc.side) { cudaStreamDestroy(sc.side); sc.side = nullptr; }
-    if (sc.ev_fork) { cudaEventDestroy(sc.ev_fork); sc.ev_fork = nullptr; }
-    if (sc.ev_join) { cudaEventDestroy(sc.ev_join); sc.ev_join = nullptr; }
+    free_bufs({&sc.compact[0], &sc.compact[1], &sc.compact[2], &sc.compact[3], &sc.dec_in, &sc.level_recon, &sc.region_in,
+               &sc.region_out});
+    destroy_side(sc);
+}
+
+// Stream of pipeline slot `k`, created on first use.
+int slot_stream(hgi_ctx* ctx, int k)
+{
+    if (!ctx->slots[k].stream) HGI_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->slots[k].stream, cudaStreamNonBlocking));
+    return HGI_OK;
+}
+
+// Waits for the streams of slots [0, n): nothing may still write into the caller's buffers when an entry point
+// returns, on the error path too.  The first error (`rc`, else the first failed wait) is the one reported.
+int drain(hgi_ctx* ctx, int n, int rc)
+{
+    for (int k = 0; k < n; ++k)
+        if (ctx->slots[k].stream) {
+            const cudaError_t e = cudaStreamSynchronize(ctx->slots[k].stream);
+            if (e != cudaSuccess && rc == HGI_OK) rc = fail(ctx, e);
+        }
+    if (rc != HGI_OK) (void)cudaGetLastError();
+    return rc;
 }
 
 // Scratch set of a device-API caller stream (created on first use).
@@ -235,6 +273,21 @@ int reserve(hgi_ctx* ctx, Scratch& sc, DevBuf& b, size_t bytes)
     ++sc.gen;
     return reserve(ctx, b, bytes);
 }
+
+// Prologue of a device-API call: the context's device for the call's duration, the caller's stream (NULL: the
+// context's own) and, when asked for, that stream's scratch set.  A non-zero `rc` is the status to return.
+struct DevCall {
+    DeviceGuard g;
+    cudaStream_t st;
+    Scratch* sc = nullptr;
+    int rc = HGI_OK;
+    DevCall(hgi_ctx* ctx, void* stream, bool want_scratch = false)
+        : g(ctx), st(stream ? (cudaStream_t)stream : ctx->stream)
+    {
+        if (!g.ok) rc = HGI_ERR_CUDA;
+        else if (want_scratch && !(sc = scratch_for(ctx, st))) rc = HGI_ERR_ALLOC;
+    }
+};
 
 int check_params(const hgi_params_t* p, bool encode)
 {
@@ -320,9 +373,7 @@ int run_tile_path(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint3
             cudaEventCreateWithFlags(&sc.ev_fork, cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&sc.ev_join, cudaEventDisableTiming) != cudaSuccess) {
             (void)cudaGetLastError();
-            if (sc.side) { cudaStreamDestroy(sc.side); sc.side = nullptr; }
-            if (sc.ev_fork) { cudaEventDestroy(sc.ev_fork); sc.ev_fork = nullptr; }
-            if (sc.ev_join) { cudaEventDestroy(sc.ev_join); sc.ev_join = nullptr; }
+            destroy_side(sc);
         }
     }
     (void)cudaGetLastError();
@@ -373,9 +424,7 @@ int run_tile_path(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint3
             a.s_q = sc.compact[set + 1].p;
             a.dec_in = sc.dec_in.p;
         }
-        const uint64_t before = hgi::launch_count();
         HGI_CUDA(ctx, hgi::launch_tile_pass(mode, prm->interp, a, st, ctx->path == HGI_PATH_TILE_GENERIC));
-        ctx->launches += hgi::launch_count() - before;
         c_recon = a.s_recon;
         c_q = a.s_q;
         cw = a.wD;
@@ -418,7 +467,6 @@ int run_level_path(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint
             HGI_CUDA(ctx, cudaMemsetAsync(r, 0, (size_t)cnt * plane, st));
             HGI_CUDA(ctx, hgi::launch_seed(mode, s, r, w, h, levels, cnt, st));
         }
-        ctx->launches++;
         for (uint32_t level = 0; level < levels; ++level) {
             hgi::LevelArgs a{};
             a.grid_in = s;
@@ -430,7 +478,6 @@ int run_level_path(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint
             a.n_images = cnt;
             a.quant_error = qerr;
             HGI_CUDA(ctx, hgi::launch_level(mode, prm->interp, a, st));
-            ctx->launches++;
         }
     }
     return HGI_OK;
@@ -459,7 +506,6 @@ int run_dev(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint32_t n_
     if (hist) {
         // The residual histogram is a pass of its own over the finished grid (hgi_hist_kernel, DESIGN.md 4.6)
         HGI_CUDA(ctx, hgi::launch_histogram(grid_out, w, h, pitch, n_images, hist, st));
-        ctx->launches++;
     }
     return HGI_OK;
 }
@@ -480,24 +526,19 @@ int run_dev_cached(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint
 {
     const uint32_t levels = effective_levels(prm->levels, w, h);
     const bool multi = levels > (uint32_t)hgi::kMaxPassLevels || ctx->path == HGI_PATH_PER_LEVEL;   // >= 3 launches
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    if (!multi || !graphs_enabled() || st == cudaStreamLegacy || st == cudaStreamPerThread ||
-        cudaStreamIsCapturing(st, &cap) != cudaSuccess || cap != cudaStreamCaptureStatusNone) {
+    auto plain = [&] {   // plain launches: the chain is not worth a graph, or its stream cannot be captured
         (void)cudaGetLastError();
         return run_dev(ctx, sc, mode, src, n_images, w, h, pitch, prm, grid_out, recon_out, hist, st);
-    }
+    };
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    if (!multi || !graphs_enabled() || st == cudaStreamLegacy || st == cudaStreamPerThread ||
+        cudaStreamIsCapturing(st, &cap) != cudaSuccess || cap != cudaStreamCaptureStatusNone)
+        return plain();
     ChainKey key{mode, ctx->path, prm->interp, prm->quant_kind, prm->quant_level, src, grid_out, recon_out, hist,
                  n_images, w, h, pitch, levels, &sc, sc.gen};
     ChainGraph* hit = nullptr;
     for (ChainGraph& g : ctx->chains)
         if (g.key == key) { hit = &g; break; }
-    if (hit && hit->exec) {
-        hit->last_use = ++ctx->chain_clock;
-        HGI_CUDA(ctx, cudaGraphLaunch(hit->exec, st));
-        ctx->launches += hit->launches;
-        ++ctx->graph_launches;
-        return HGI_OK;
-    }
     if (!hit) {   // first sighting: run it plainly and remember the key (the scratch generation may move: re-key after)
         const int rc = run_dev(ctx, sc, mode, src, n_images, w, h, pitch, prm, grid_out, recon_out, hist, st);
         if (rc) return rc;
@@ -520,33 +561,28 @@ int run_dev_cached(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint
         ctx->chains.push_back(g);
         return HGI_OK;
     }
-    // second sighting: capture the chain (nothing allocates now: the first run sized every buffer)
-    const uint64_t before = ctx->launches;
-    HGI_CUDA(ctx, cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-    const int rc = run_dev(ctx, sc, mode, src, n_images, w, h, pitch, prm, grid_out, recon_out, hist, st);
-    cudaGraph_t graph = nullptr;
-    const cudaError_t ce = cudaStreamEndCapture(st, &graph);
-    const uint64_t n_launch = ctx->launches - before;
-    ctx->launches = before;
-    if (rc != HGI_OK || ce != cudaSuccess || !graph || sc.gen != key.scratch_gen) {
-        if (graph) cudaGraphDestroy(graph);
-        (void)cudaGetLastError();
-        hit->last_use = ++ctx->chain_clock;
-        if (rc != HGI_OK) return rc;
-        return run_dev(ctx, sc, mode, src, n_images, w, h, pitch, prm, grid_out, recon_out, hist, st);   // capture refused: plain launches
-    }
-    cudaGraphExec_t exec = nullptr;
-    const cudaError_t ie = cudaGraphInstantiate(&exec, graph, 0);
-    cudaGraphDestroy(graph);
-    if (ie != cudaSuccess || !exec) {
-        (void)cudaGetLastError();
-        return run_dev(ctx, sc, mode, src, n_images, w, h, pitch, prm, grid_out, recon_out, hist, st);
-    }
-    hit->exec = exec;
-    hit->launches = n_launch;
     hit->last_use = ++ctx->chain_clock;
-    HGI_CUDA(ctx, cudaGraphLaunch(exec, st));
-    ctx->launches += n_launch;
+    if (!hit->exec) {   // second sighting: capture the chain (nothing allocates now: the first run sized every buffer)
+        const uint64_t before = hgi::launch_count();
+        HGI_CUDA(ctx, cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+        const int rc = run_dev(ctx, sc, mode, src, n_images, w, h, pitch, prm, grid_out, recon_out, hist, st);
+        cudaGraph_t graph = nullptr;
+        const cudaError_t ce = cudaStreamEndCapture(st, &graph);
+        hit->launches = hgi::launch_count() - before;
+        hgi::launch_count() = before;   // captured, not launched: the graph launch counts them
+        cudaGraphExec_t exec = nullptr;
+        if (rc == HGI_OK && ce == cudaSuccess && graph && sc.gen == key.scratch_gen &&
+            cudaGraphInstantiate(&exec, graph, 0) == cudaSuccess)
+            hit->exec = exec;
+        if (graph) cudaGraphDestroy(graph);
+        if (rc != HGI_OK) {
+            (void)cudaGetLastError();
+            return rc;
+        }
+        if (!hit->exec) return plain();   // capture refused
+    }
+    HGI_CUDA(ctx, cudaGraphLaunch(hit->exec, st));
+    hgi::launch_count() += hit->launches;
     ++ctx->graph_launches;
     return HGI_OK;
 }
@@ -555,39 +591,65 @@ int run_dev_cached(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint
 // bytes; the per-image residual histogram has 32-bit bins.
 constexpr uint32_t kMaxPitch = 1u << 26;
 
-// Two-slot pipeline of the reductions / colour conversion over host buffers (hgi_histogram_u8, hgi_error_metrics_u8,
-// hgi_rgb_to_luma_u8): streams and staging buffers of slots 0..ns-1; every stream is drained before the call returns,
-// on the error path too (the D2H copies target caller memory).
 int cuda_rc(hgi_ctx* ctx, cudaError_t e) { return e == cudaSuccess ? HGI_OK : fail(ctx, e); }
 
-int two_slots(hgi_ctx* ctx, int ns, size_t in_bytes, size_t out_bytes)
+// Two-slot pipeline of the reductions / colour conversion over host buffers (hgi_rgb_to_luma_u8, hgi_histogram_u8,
+// hgi_error_metrics_u8): [0, n) is cut into chunks of `chunk` elements that alternate between slots 0 and 1, so the
+// H2D copy of one chunk overlaps the kernel and the D2H copy of the other.  Each slot stages `in_per` (`out_per`) bytes
+// per element of a chunk in `in` (`out`) and `hist_bytes` in `hist`.  enqueue(k, slot, off, len) puts one chunk's
+// copies and kernel on slot k's stream; fold(k) takes in the result of slot k's last chunk once its stream has run
+// it: before the slot is reused, and after the final drain.
+template <class Enqueue, class Fold>
+int run_chunks(hgi_ctx* ctx, size_t n, size_t chunk, size_t in_per, size_t out_per, size_t hist_bytes, Enqueue enqueue,
+               Fold fold)
 {
+    const size_t cap = n < chunk ? n : chunk;
+    const int ns = n > chunk ? 2 : 1;
     for (int k = 0; k < ns; ++k) {
         Slot& sl = ctx->slots[k];
-        if (!sl.stream) HGI_CUDA(ctx, cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
-        int rc = reserve(ctx, sl.in, in_bytes);
-        if (!rc && out_bytes) rc = reserve(ctx, sl.out, out_bytes);
+        int rc = slot_stream(ctx, k);
+        if (!rc) rc = reserve(ctx, sl.in, in_per * cap);
+        if (!rc && out_per) rc = reserve(ctx, sl.out, out_per * cap);
+        if (!rc && hist_bytes) rc = reserve(ctx, sl.hist, hist_bytes);
         if (rc) return rc;
     }
-    return HGI_OK;
-}
-
-int drain_two(hgi_ctx* ctx, int ns, int rc)
-{
-    for (int k = 0; k < ns; ++k)
-        if (ctx->slots[k].stream) {
-            const cudaError_t e = cudaStreamSynchronize(ctx->slots[k].stream);
-            if (e != cudaSuccess && rc == HGI_OK) rc = fail(ctx, e);
+    bool pending[2] = {false, false};
+    int rc = HGI_OK;
+    size_t i = 0;
+    for (size_t off = 0; off < n && !rc; off += chunk, ++i) {
+        const int k = (int)(i & 1);
+        Slot& sl = ctx->slots[k];
+        if (pending[k]) {
+            rc = cuda_rc(ctx, cudaStreamSynchronize(sl.stream));
+            if (rc) break;
+            fold(k);
+            pending[k] = false;
         }
+        rc = enqueue(k, sl, off, n - off < chunk ? n - off : chunk);
+        if (!rc) pending[k] = true;
+    }
+    rc = drain(ctx, ns, rc);
+    if (!rc)
+        for (int k = 0; k < 2; ++k)
+            if (pending[k]) fold(k);
     return rc;
 }
 
-bool plane_size_ok(uint32_t w, uint32_t h, uint32_t n_images, uint32_t pitch = 0)
+constexpr int kEmptyJob = 1;   // check_job: the arguments are valid and there is nothing to do
+
+// Argument checks of the encode / decode entry points, in this order: the handle, the parameters, the plane size
+// (`size_ok`: a limit of the caller's own), an empty job (kEmptyJob, whatever its data pointers), null data pointers.
+int check_job(bool handle, const hgi_params_t* prm, bool encode, uint32_t w, uint32_t h, uint32_t n_images,
+              uint32_t pitch, std::initializer_list<const void*> ptrs, bool size_ok = true)
 {
-    if (pitch == 0) pitch = w;
-    if (pitch < w || pitch >= kMaxPitch) return false;
-    const unsigned __int128 total = (unsigned __int128)pitch * h * n_images;
-    return total < ((unsigned __int128)1 << 62);
+    if (!handle) return HGI_ERR_INVALID_ARG;
+    if (int rc = check_params(prm, encode)) return rc;
+    if (!size_ok || pitch < w || pitch >= kMaxPitch) return HGI_ERR_INVALID_ARG;
+    if ((unsigned __int128)pitch * h * n_images >= ((unsigned __int128)1 << 62)) return HGI_ERR_INVALID_ARG;
+    if ((size_t)w * h * n_images == 0) return kEmptyJob;
+    for (const void* p : ptrs)
+        if (!p) return HGI_ERR_INVALID_ARG;
+    return HGI_OK;
 }
 
 // Host-pointer batch driver: images are cut into chunks that flow through `kSlots` stream slots
@@ -604,19 +666,13 @@ int run_host_chunks(hgi_ctx* ctx, int mode, const uint8_t* in, uint32_t n_images
     const int used = n_chunks < (uint32_t)nslots ? (int)n_chunks : nslots;
     for (int s = 0; s < used; ++s) {
         Slot& sl = ctx->slots[s];
-        if (!sl.stream) HGI_CUDA(ctx, cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
+        if (int rc = slot_stream(ctx, s)) return rc;
         *used_out = s + 1;
         int rc = reserve(ctx, sl.in, (size_t)per * plane);
         if (!rc) rc = reserve(ctx, sl.out, (size_t)per * plane);
         if (!rc && recon_out) rc = reserve(ctx, sl.aux, (size_t)per * plane);
+        if (!rc && hist_out) rc = reserve(ctx, sl.hist, (size_t)per * 256 * sizeof(uint32_t));
         if (rc) return rc;
-        if (hist_out && sl.hist_cap < (size_t)per * 256) {
-            if (sl.hist) HGI_CUDA(ctx, cudaFree(sl.hist));
-            sl.hist = nullptr;
-            sl.hist_cap = 0;
-            HGI_CUDA(ctx, cudaMalloc((void**)&sl.hist, (size_t)per * 256 * sizeof(uint32_t)));
-            sl.hist_cap = (size_t)per * 256;
-        }
     }
     for (uint32_t c = 0; c < n_chunks; ++c) {
         Slot& sl = ctx->slots[c % (uint32_t)used];
@@ -627,33 +683,28 @@ int run_host_chunks(hgi_ctx* ctx, int mode, const uint8_t* in, uint32_t n_images
         HGI_CUDA(ctx, cudaMemcpyAsync(sl.in.p, in + off, bytes, cudaMemcpyHostToDevice, sl.stream));
         uint8_t* d_grid = (mode == hgi::kModeEncode) ? sl.out.p : nullptr;
         uint8_t* d_recon = (mode == hgi::kModeEncode) ? (recon_out ? sl.aux.p : nullptr) : sl.out.p;
-        int rc = run_dev(ctx, sl.scratch, mode, sl.in.p, cnt, w, h, w, prm, d_grid, d_recon, hist_out ? sl.hist : nullptr, sl.stream);
+        uint32_t* d_hist = hist_out ? (uint32_t*)sl.hist.p : nullptr;
+        int rc = run_dev(ctx, sl.scratch, mode, sl.in.p, cnt, w, h, w, prm, d_grid, d_recon, d_hist, sl.stream);
         if (rc) return rc;
         HGI_CUDA(ctx, cudaMemcpyAsync(out + off, sl.out.p, bytes, cudaMemcpyDeviceToHost, sl.stream));
         if (mode == hgi::kModeEncode && recon_out)
             HGI_CUDA(ctx, cudaMemcpyAsync(recon_out + off, sl.aux.p, bytes, cudaMemcpyDeviceToHost, sl.stream));
         if (hist_out)
-            HGI_CUDA(ctx, cudaMemcpyAsync(hist_out + (size_t)first * 256, sl.hist, (size_t)cnt * 256 * sizeof(uint32_t),
+            HGI_CUDA(ctx, cudaMemcpyAsync(hist_out + (size_t)first * 256, d_hist, (size_t)cnt * 256 * sizeof(uint32_t),
                                           cudaMemcpyDeviceToHost, sl.stream));
     }
     return HGI_OK;
 }
 
-// Host-pointer batch driver: images are cut into chunks that flow through the stream slots (H2D -> kernels -> D2H),
-// so copies in both directions overlap the kernels.  Whatever happens, no copy into the caller's buffers is still in
-// flight when this returns: the slot streams are drained on the error path too.
+// Host-pointer batch driver of one context: run_host_chunks, then every slot it used is drained.
 int run_host(hgi_ctx* ctx, int mode, const uint8_t* in, uint32_t n_images, uint32_t w, uint32_t h,
              const hgi_params_t* prm, uint8_t* out, uint8_t* recon_out, uint32_t* hist_out)
 {
-    if (n_images == 0 || (size_t)w * h == 0) return HGI_OK;
+    DeviceGuard g(ctx);
+    if (!g.ok) return HGI_ERR_CUDA;
     int used = 0;
-    int rc = run_host_chunks(ctx, mode, in, n_images, w, h, prm, out, recon_out, hist_out, &used);
-    for (int s = 0; s < used; ++s) {
-        const cudaError_t e = cudaStreamSynchronize(ctx->slots[s].stream);
-        if (e != cudaSuccess && rc == HGI_OK) rc = fail(ctx, e);   // the first error is the one reported
-    }
-    if (rc != HGI_OK) (void)cudaGetLastError();
-    return rc;
+    const int rc = run_host_chunks(ctx, mode, in, n_images, w, h, prm, out, recon_out, hist_out, &used);
+    return drain(ctx, used, rc);
 }
 
 // Window of a scalable decode (DESIGN.md "Scalable decode"): the region [u0, u1) of the scaled image is decoded from
@@ -686,10 +737,8 @@ int plan_region(uint32_t w, uint32_t h, uint32_t levels, uint32_t k, const hgi_r
 int check_region(hgi_ctx* ctx, const hgi_params_t* prm, uint32_t w, uint32_t h, uint32_t n_images, uint32_t pitch,
                  uint32_t k, const hgi_rect_t* region, hgi_region_plan_t* pl, hgi_rect_t* r)
 {
-    if (!ctx) return HGI_ERR_INVALID_ARG;
-    int rc = check_params(prm, false);
-    if (rc) return rc;
-    if (!plane_size_ok(w, h, n_images, pitch)) return HGI_ERR_INVALID_ARG;
+    int rc = check_job(ctx, prm, false, w, h, n_images, pitch, {});
+    if (rc < 0) return rc;   // an empty job is the region rules' to judge
     rc = plan_region(w, h, prm->levels, k, region, pl, r);
     if (rc) return rc;
     if (ctx->path == HGI_PATH_PER_LEVEL) return HGI_ERR_UNSUPPORTED;   // the window decode is a tile path
@@ -711,7 +760,6 @@ int run_region(hgi_ctx* ctx, Scratch& sc, const uint8_t* src, uint64_t row_step,
     if (rc) return rc;
     HGI_CUDA(ctx, hgi::launch_region_gather(src, row_step, plane_stride, k, ww, wh, wpitch, n_images, vec, row_avail,
                                             sc.region_in.p, st));
-    ctx->launches++;
     const uint8_t* win = sc.region_in.p;
     if (levels) {
         rc = run_tile_path(ctx, sc, hgi::kModeDecode, sc.region_in.p, n_images, ww, wh, wpitch, levels, prm, nullptr,
@@ -721,7 +769,6 @@ int run_region(hgi_ctx* ctx, Scratch& sc, const uint8_t* src, uint64_t row_step,
     }
     HGI_CUDA(ctx, hgi::launch_region_crop(win, wpitch, wh, pl.crop_x, pl.crop_y, r.width, r.height, n_images, d_out,
                                           out_pitch, st));
-    ctx->launches++;
     return HGI_OK;
 }
 
@@ -764,17 +811,19 @@ int hgi_ctx_create(int device, hgi_ctx_t** ctx_out)
     hgi_ctx* ctx = new (std::nothrow) hgi_ctx();
     if (!ctx) return HGI_ERR_ALLOC;
     ctx->device = device;
-    DeviceGuard g(ctx);
-    cudaError_t e = g.ok ? cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) : ctx->last_err;
-    if (e == cudaSuccess) e = cudaMalloc((void**)&ctx->d_metrics, 4 * sizeof(unsigned long long))   /* two per pipeline slot */;
-    if (e != cudaSuccess) {
+    {
+        DeviceGuard g(ctx);
+        cudaError_t e = g.ok ? cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) : ctx->last_err;
+        if (e == cudaSuccess) e = cudaMalloc((void**)&ctx->d_metrics, 4 * sizeof(unsigned long long))   /* two per pipeline slot */;
+        if (e == cudaSuccess) {
+            *ctx_out = ctx;
+            return HGI_OK;
+        }
         if (ctx->stream) cudaStreamDestroy(ctx->stream);
-        delete ctx;
         (void)cudaGetLastError();
-        return HGI_ERR_CUDA;
     }
-    *ctx_out = ctx;
-    return HGI_OK;
+    delete ctx;   // after the guard, which writes to it when it ends
+    return HGI_ERR_CUDA;
 }
 
 void hgi_ctx_destroy(hgi_ctx_t* ctx)
@@ -791,10 +840,7 @@ void hgi_ctx_destroy(hgi_ctx_t* ctx)
         for (auto& s : ctx->slots) {
             free_scratch(s.scratch);
             if (s.stream) { cudaStreamSynchronize(s.stream); cudaStreamDestroy(s.stream); }
-            if (s.in.p) cudaFree(s.in.p);
-            if (s.out.p) cudaFree(s.out.p);
-            if (s.aux.p) cudaFree(s.aux.p);
-            if (s.hist) cudaFree(s.hist);
+            free_bufs({&s.in, &s.out, &s.aux, &s.hist});
         }
         if (ctx->d_metrics) cudaFree(ctx->d_metrics);
         if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -886,38 +932,24 @@ int hgi_encode_dev_pitched(hgi_ctx_t* ctx, const uint8_t* d_images, uint32_t n_i
                            uint32_t pitch, const hgi_params_t* params, uint8_t* d_grids_out, uint8_t* d_recon_out,
                            uint32_t* d_hist_out, void* stream)
 {
-    if (!ctx) return HGI_ERR_INVALID_ARG;
-    int rc = check_params(params, true);
-    if (rc) return rc;
-    if (!plane_size_ok(width, height, n_images, pitch)) return HGI_ERR_INVALID_ARG;
-    if (d_hist_out && (uint64_t)width * height >= (1ull << 32)) return HGI_ERR_INVALID_ARG;   // u32 bins
-    if ((size_t)width * height * n_images == 0) return HGI_OK;
-    if (!d_images || !d_grids_out) return HGI_ERR_INVALID_ARG;
-    DeviceGuard g(ctx);
-    if (!g.ok) return HGI_ERR_CUDA;
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-    Scratch* sc = scratch_for(ctx, st);
-    if (!sc) return HGI_ERR_ALLOC;
-    return run_dev_cached(ctx, *sc, hgi::kModeEncode, d_images, n_images, width, height, pitch, params, d_grids_out,
-                          d_recon_out, d_hist_out, st);
+    const bool bins_ok = !d_hist_out || (uint64_t)width * height < (1ull << 32);   // u32 bins
+    if (int rc = check_job(ctx, params, true, width, height, n_images, pitch, {d_images, d_grids_out}, bins_ok))
+        return rc == kEmptyJob ? HGI_OK : rc;
+    DevCall dc(ctx, stream, true);
+    if (dc.rc) return dc.rc;
+    return run_dev_cached(ctx, *dc.sc, hgi::kModeEncode, d_images, n_images, width, height, pitch, params, d_grids_out,
+                          d_recon_out, d_hist_out, dc.st);
 }
 
 int hgi_decode_dev_pitched(hgi_ctx_t* ctx, const uint8_t* d_grids, uint32_t n_images, uint32_t width, uint32_t height,
                            uint32_t pitch, const hgi_params_t* params, uint8_t* d_images_out, void* stream)
 {
-    if (!ctx) return HGI_ERR_INVALID_ARG;
-    int rc = check_params(params, false);
-    if (rc) return rc;
-    if (!plane_size_ok(width, height, n_images, pitch)) return HGI_ERR_INVALID_ARG;
-    if ((size_t)width * height * n_images == 0) return HGI_OK;
-    if (!d_grids || !d_images_out) return HGI_ERR_INVALID_ARG;
-    DeviceGuard g(ctx);
-    if (!g.ok) return HGI_ERR_CUDA;
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-    Scratch* sc = scratch_for(ctx, st);
-    if (!sc) return HGI_ERR_ALLOC;
-    return run_dev_cached(ctx, *sc, hgi::kModeDecode, d_grids, n_images, width, height, pitch, params, nullptr, d_images_out,
-                          nullptr, st);
+    if (int rc = check_job(ctx, params, false, width, height, n_images, pitch, {d_grids, d_images_out}))
+        return rc == kEmptyJob ? HGI_OK : rc;
+    DevCall dc(ctx, stream, true);
+    if (dc.rc) return dc.rc;
+    return run_dev_cached(ctx, *dc.sc, hgi::kModeDecode, d_grids, n_images, width, height, pitch, params, nullptr, d_images_out,
+                          nullptr, dc.st);
 }
 
 int hgi_encode_dev(hgi_ctx_t* ctx, const uint8_t* d_images, uint32_t n_images, uint32_t width, uint32_t height,
@@ -940,11 +972,9 @@ int hgi_histogram_dev(hgi_ctx_t* ctx, const uint8_t* d_grid, size_t n_per_image,
     if (n_per_image >= ((size_t)1 << 32)) return HGI_ERR_INVALID_ARG;  // u32 bins
     if (n_images == 0) return HGI_OK;
     if (!d_grid && n_per_image) return HGI_ERR_INVALID_ARG;
-    DeviceGuard g(ctx);
-    if (!g.ok) return HGI_ERR_CUDA;
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-    HGI_CUDA(ctx, hgi::launch_histogram(d_grid, (uint32_t)n_per_image, 1u, (uint32_t)n_per_image, n_images, d_hist_out, st));
-    ctx->launches++;
+    DevCall dc(ctx, stream);
+    if (dc.rc) return dc.rc;
+    HGI_CUDA(ctx, hgi::launch_histogram(d_grid, (uint32_t)n_per_image, 1u, (uint32_t)n_per_image, n_images, d_hist_out, dc.st));
     return HGI_OK;
 }
 
@@ -957,11 +987,9 @@ int hgi_rle_histogram_dev(hgi_ctx_t* ctx, const uint8_t* d_grid, size_t n, size_
     if (block_bytes == 0 || block_bytes >= ((size_t)1 << 32) || (n_blocks > 1 && block_bytes % HGI_RLE_SEGMENT_BYTES != 0) ||
         (n_blocks - 1) * block_bytes > n || n_blocks * block_bytes < n)
         return HGI_ERR_INVALID_ARG;
-    DeviceGuard g(ctx);
-    if (!g.ok) return HGI_ERR_CUDA;
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-    HGI_CUDA(ctx, hgi::launch_rle_histogram(d_grid, n, block_bytes, (uint32_t)n_blocks, d_hist_out, st));
-    ctx->launches++;
+    DevCall dc(ctx, stream);
+    if (dc.rc) return dc.rc;
+    HGI_CUDA(ctx, hgi::launch_rle_histogram(d_grid, n, block_bytes, (uint32_t)n_blocks, d_hist_out, dc.st));
     return HGI_OK;
 }
 
@@ -972,26 +1000,15 @@ int hgi_rle_histogram_u8(hgi_ctx_t* ctx, const uint8_t* grid, size_t n, size_t b
     DeviceGuard g(ctx);
     if (!g.ok) return HGI_ERR_CUDA;
     Slot& sl = ctx->slots[0];
-    if (!sl.stream) HGI_CUDA(ctx, cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
-    int rc = reserve(ctx, sl.in, n ? n : 1);
+    const size_t hbytes = n_blocks * HGI_RLE_TABLE_SYMBOLS * sizeof(uint32_t);
+    int rc = slot_stream(ctx, 0);
+    if (!rc) rc = reserve(ctx, sl.in, n ? n : 1);
+    if (!rc) rc = reserve(ctx, sl.hist, hbytes);
     if (rc) return rc;
-    const size_t hwords = n_blocks * HGI_RLE_TABLE_SYMBOLS;
-    if (sl.hist_cap < hwords) {
-        if (sl.hist) HGI_CUDA(ctx, cudaFree(sl.hist));
-        sl.hist = nullptr;
-        sl.hist_cap = 0;
-        HGI_CUDA(ctx, cudaMalloc((void**)&sl.hist, hwords * sizeof(uint32_t)));
-        sl.hist_cap = hwords;
-    }
     if (n) HGI_CUDA(ctx, cudaMemcpyAsync(sl.in.p, grid, n, cudaMemcpyHostToDevice, sl.stream));
-    rc = hgi_rle_histogram_dev(ctx, sl.in.p, n, block_bytes, n_blocks, sl.hist, sl.stream);
-    if (rc == HGI_OK) {
-        const cudaError_t e = cudaMemcpyAsync(hist_out, sl.hist, hwords * sizeof(uint32_t), cudaMemcpyDeviceToHost, sl.stream);
-        if (e != cudaSuccess) rc = fail(ctx, e);
-    }
-    const cudaError_t es = cudaStreamSynchronize(sl.stream);
-    if (es != cudaSuccess && rc == HGI_OK) rc = fail(ctx, es);
-    return rc;
+    rc = hgi_rle_histogram_dev(ctx, sl.in.p, n, block_bytes, n_blocks, (uint32_t*)sl.hist.p, sl.stream);
+    if (rc == HGI_OK) rc = cuda_rc(ctx, cudaMemcpyAsync(hist_out, sl.hist.p, hbytes, cudaMemcpyDeviceToHost, sl.stream));
+    return drain(ctx, 1, rc);
 }
 
 int hgi_error_metrics_dev(hgi_ctx_t* ctx, const uint8_t* d_before, const uint8_t* d_after, size_t n,
@@ -999,11 +1016,9 @@ int hgi_error_metrics_dev(hgi_ctx_t* ctx, const uint8_t* d_before, const uint8_t
 {
     if (!ctx || !d_out) return HGI_ERR_INVALID_ARG;
     if (n && (!d_before || !d_after)) return HGI_ERR_INVALID_ARG;
-    DeviceGuard g(ctx);
-    if (!g.ok) return HGI_ERR_CUDA;
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-    HGI_CUDA(ctx, hgi::launch_error_metrics(d_before, d_after, n, (unsigned long long*)d_out, st));
-    if (n) ctx->launches++;
+    DevCall dc(ctx, stream);
+    if (dc.rc) return dc.rc;
+    HGI_CUDA(ctx, hgi::launch_error_metrics(d_before, d_after, n, (unsigned long long*)d_out, dc.st));
     return HGI_OK;
 }
 
@@ -1012,11 +1027,9 @@ int hgi_rgb_to_luma_dev(hgi_ctx_t* ctx, const uint8_t* d_rgb, size_t n_pixels, u
     if (!ctx) return HGI_ERR_INVALID_ARG;
     if (n_pixels == 0) return HGI_OK;
     if (!d_rgb || !d_luma_out || n_pixels > ((size_t)1 << 60)) return HGI_ERR_INVALID_ARG;
-    DeviceGuard g(ctx);
-    if (!g.ok) return HGI_ERR_CUDA;
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-    HGI_CUDA(ctx, hgi::launch_rgb_to_luma(d_rgb, n_pixels, d_luma_out, st));
-    ctx->launches++;
+    DevCall dc(ctx, stream);
+    if (dc.rc) return dc.rc;
+    HGI_CUDA(ctx, hgi::launch_rgb_to_luma(d_rgb, n_pixels, d_luma_out, dc.st));
     return HGI_OK;
 }
 
@@ -1027,64 +1040,36 @@ int hgi_rgb_to_luma_u8(hgi_ctx_t* ctx, const uint8_t* rgb, size_t n_pixels, uint
     if (!rgb || !luma_out || n_pixels > ((size_t)1 << 60)) return HGI_ERR_INVALID_ARG;
     DeviceGuard g(ctx);
     if (!g.ok) return HGI_ERR_CUDA;
-    // chunks alternate between two slots: the H2D copy of chunk i+1 overlaps the kernel and the D2H copy of chunk i
     const size_t chunk = ctx->chunk_bytes ? ctx->chunk_bytes : ((size_t)64 << 20);   // pixels per chunk
-    const size_t cap = n_pixels < chunk ? n_pixels : chunk;
-    const int ns = n_pixels > chunk ? 2 : 1;
-    int rc = two_slots(ctx, ns, 3 * cap, cap);
-    if (rc) return rc;
-    size_t i = 0;
-    for (size_t off = 0; off < n_pixels && !rc; off += chunk, ++i) {
-        Slot& sl = ctx->slots[i & 1];
-        const size_t len = (n_pixels - off < chunk) ? n_pixels - off : chunk;
-        if (i >= 2) rc = cuda_rc(ctx, cudaStreamSynchronize(sl.stream));
-        if (!rc) rc = cuda_rc(ctx, cudaMemcpyAsync(sl.in.p, rgb + 3 * off, 3 * len, cudaMemcpyHostToDevice, sl.stream));
-        if (!rc) rc = cuda_rc(ctx, hgi::launch_rgb_to_luma(sl.in.p, len, sl.out.p, sl.stream));
-        if (!rc) ctx->launches++;
-        if (!rc) rc = cuda_rc(ctx, cudaMemcpyAsync(luma_out + off, sl.out.p, len, cudaMemcpyDeviceToHost, sl.stream));
-    }
-    return drain_two(ctx, ns, rc);
+    return run_chunks(ctx, n_pixels, chunk, 3, 1, 0, [&](int, Slot& sl, size_t off, size_t len) -> int {
+        HGI_CUDA(ctx, cudaMemcpyAsync(sl.in.p, rgb + 3 * off, 3 * len, cudaMemcpyHostToDevice, sl.stream));
+        HGI_CUDA(ctx, hgi::launch_rgb_to_luma(sl.in.p, len, sl.out.p, sl.stream));
+        HGI_CUDA(ctx, cudaMemcpyAsync(luma_out + off, sl.out.p, len, cudaMemcpyDeviceToHost, sl.stream));
+        return HGI_OK;
+    }, [](int) {});
 }
 
 int hgi_encode_batch_u8(hgi_ctx_t* ctx, const uint8_t* images, uint32_t n_images, uint32_t width, uint32_t height,
                         const hgi_params_t* params, uint8_t* grids_out, uint32_t* hist_out)
 {
-    if (!ctx) return HGI_ERR_INVALID_ARG;
-    int rc = check_params(params, true);
-    if (rc) return rc;
-    if (!plane_size_ok(width, height, n_images)) return HGI_ERR_INVALID_ARG;
-    if ((size_t)width * height * n_images == 0) return HGI_OK;
-    if (!images || !grids_out) return HGI_ERR_INVALID_ARG;
-    DeviceGuard g(ctx);
-    if (!g.ok) return HGI_ERR_CUDA;
+    if (int rc = check_job(ctx, params, true, width, height, n_images, width, {images, grids_out}))
+        return rc == kEmptyJob ? HGI_OK : rc;
     return run_host(ctx, hgi::kModeEncode, images, n_images, width, height, params, grids_out, nullptr, hist_out);
 }
 
 int hgi_decode_batch_u8(hgi_ctx_t* ctx, const uint8_t* grids, uint32_t n_images, uint32_t width, uint32_t height,
                         const hgi_params_t* params, uint8_t* images_out)
 {
-    if (!ctx) return HGI_ERR_INVALID_ARG;
-    int rc = check_params(params, false);
-    if (rc) return rc;
-    if (!plane_size_ok(width, height, n_images)) return HGI_ERR_INVALID_ARG;
-    if ((size_t)width * height * n_images == 0) return HGI_OK;
-    if (!grids || !images_out) return HGI_ERR_INVALID_ARG;
-    DeviceGuard g(ctx);
-    if (!g.ok) return HGI_ERR_CUDA;
+    if (int rc = check_job(ctx, params, false, width, height, n_images, width, {grids, images_out}))
+        return rc == kEmptyJob ? HGI_OK : rc;
     return run_host(ctx, hgi::kModeDecode, grids, n_images, width, height, params, images_out, nullptr, nullptr);
 }
 
 int hgi_encode_u8(hgi_ctx_t* ctx, const uint8_t* image, uint32_t width, uint32_t height, const hgi_params_t* params,
                   uint8_t* grid_out, uint8_t* recon_out)
 {
-    if (!ctx) return HGI_ERR_INVALID_ARG;
-    int rc = check_params(params, true);
-    if (rc) return rc;
-    if (!plane_size_ok(width, height, 1)) return HGI_ERR_INVALID_ARG;
-    if ((size_t)width * height == 0) return HGI_OK;
-    if (!image || !grid_out) return HGI_ERR_INVALID_ARG;
-    DeviceGuard g(ctx);
-    if (!g.ok) return HGI_ERR_CUDA;
+    if (int rc = check_job(ctx, params, true, width, height, 1, width, {image, grid_out}))
+        return rc == kEmptyJob ? HGI_OK : rc;
     return run_host(ctx, hgi::kModeEncode, image, 1, width, height, params, grid_out, recon_out, nullptr);
 }
 
@@ -1102,46 +1087,17 @@ int hgi_histogram_u8(hgi_ctx_t* ctx, const uint8_t* grid, size_t n, uint64_t his
     if (!grid) return HGI_ERR_INVALID_ARG;
     DeviceGuard g(ctx);
     if (!g.ok) return HGI_ERR_CUDA;
-    // keeps the u32 device bins far from overflow (and the length a uint32_t); two slots as in hgi_rgb_to_luma_u8
+    // keeps the u32 device bins far from overflow (and the length a uint32_t)
     const size_t chunk = ctx->chunk_bytes ? ctx->chunk_bytes : ((size_t)1 << 30);
-    const int ns = n > chunk ? 2 : 1;
-    int rc = two_slots(ctx, ns, n < chunk ? n : chunk, 0);
-    for (int k = 0; k < ns && !rc; ++k) {
-        Slot& sl = ctx->slots[k];
-        if (sl.hist_cap < 256) {
-            if (sl.hist) rc = cuda_rc(ctx, cudaFree(sl.hist));
-            sl.hist = nullptr;
-            sl.hist_cap = 0;
-            if (!rc) rc = cuda_rc(ctx, cudaMalloc((void**)&sl.hist, 256 * sizeof(uint32_t)));
-            if (!rc) sl.hist_cap = 256;
-        }
-    }
-    if (rc) return rc;
     uint32_t part[2][256];
-    bool pending[2] = {false, false};
-    size_t i = 0;
-    for (size_t off = 0; off < n && !rc; off += chunk, ++i) {
-        const int k = (int)(i & 1);
-        Slot& sl = ctx->slots[k];
-        const size_t len = (n - off < chunk) ? n - off : chunk;
-        if (pending[k]) {
-            rc = cuda_rc(ctx, cudaStreamSynchronize(sl.stream));
-            if (rc) break;
-            for (int b = 0; b < 256; ++b) hist_out[b] += part[k][b];
-            pending[k] = false;
-        }
-        rc = cuda_rc(ctx, cudaMemcpyAsync(sl.in.p, grid + off, len, cudaMemcpyHostToDevice, sl.stream));
-        if (!rc) rc = cuda_rc(ctx, hgi::launch_histogram(sl.in.p, (uint32_t)len, 1u, (uint32_t)len, 1, sl.hist, sl.stream));
-        if (!rc) ctx->launches++;
-        if (!rc) rc = cuda_rc(ctx, cudaMemcpyAsync(part[k], sl.hist, sizeof(part[k]), cudaMemcpyDeviceToHost, sl.stream));
-        if (!rc) pending[k] = true;
-    }
-    rc = drain_two(ctx, ns, rc);
-    if (!rc)
-        for (int k = 0; k < 2; ++k)
-            if (pending[k])
-                for (int b = 0; b < 256; ++b) hist_out[b] += part[k][b];
-    return rc;
+    return run_chunks(ctx, n, chunk, 1, 0, sizeof(part[0]), [&](int k, Slot& sl, size_t off, size_t len) -> int {
+        HGI_CUDA(ctx, cudaMemcpyAsync(sl.in.p, grid + off, len, cudaMemcpyHostToDevice, sl.stream));
+        HGI_CUDA(ctx, hgi::launch_histogram(sl.in.p, (uint32_t)len, 1u, (uint32_t)len, 1, (uint32_t*)sl.hist.p, sl.stream));
+        HGI_CUDA(ctx, cudaMemcpyAsync(part[k], sl.hist.p, sizeof(part[k]), cudaMemcpyDeviceToHost, sl.stream));
+        return HGI_OK;
+    }, [&](int k) {
+        for (int b = 0; b < 256; ++b) hist_out[b] += part[k][b];
+    });
 }
 
 int hgi_error_metrics_u8(hgi_ctx_t* ctx, const uint8_t* before, const uint8_t* after, size_t n,
@@ -1153,39 +1109,19 @@ int hgi_error_metrics_u8(hgi_ctx_t* ctx, const uint8_t* before, const uint8_t* a
     if (n) {
         DeviceGuard g(ctx);
         if (!g.ok) return HGI_ERR_CUDA;
-        const size_t chunk = ctx->chunk_bytes ? ctx->chunk_bytes : ((size_t)256 << 20);   // two slots as in hgi_rgb_to_luma_u8
-        const size_t cap = n < chunk ? n : chunk;
-        const int ns = n > chunk ? 2 : 1;
-        int rc = two_slots(ctx, ns, cap, cap);
-        if (rc) return rc;
+        const size_t chunk = ctx->chunk_bytes ? ctx->chunk_bytes : ((size_t)256 << 20);
         unsigned long long part[2][2];
-        bool pending[2] = {false, false};
-        size_t i = 0;
-        for (size_t off = 0; off < n && !rc; off += chunk, ++i) {
-            const int k = (int)(i & 1);
-            Slot& sl = ctx->slots[k];
-            const size_t len = (n - off < chunk) ? n - off : chunk;
-            if (pending[k]) {
-                rc = cuda_rc(ctx, cudaStreamSynchronize(sl.stream));
-                if (rc) break;
-                total += part[k][0];
-                if (part[k][1] > mx) mx = part[k][1];
-                pending[k] = false;
-            }
-            rc = cuda_rc(ctx, cudaMemcpyAsync(sl.in.p, before + off, len, cudaMemcpyHostToDevice, sl.stream));
-            if (!rc) rc = cuda_rc(ctx, cudaMemcpyAsync(sl.out.p, after + off, len, cudaMemcpyHostToDevice, sl.stream));
-            if (!rc) rc = cuda_rc(ctx, hgi::launch_error_metrics(sl.in.p, sl.out.p, len, ctx->d_metrics + 2 * k, sl.stream));
-            if (!rc) ctx->launches++;
-            if (!rc) rc = cuda_rc(ctx, cudaMemcpyAsync(part[k], ctx->d_metrics + 2 * k, sizeof(part[k]), cudaMemcpyDeviceToHost, sl.stream));
-            if (!rc) pending[k] = true;
-        }
-        rc = drain_two(ctx, ns, rc);
+        const int rc = run_chunks(ctx, n, chunk, 1, 1, 0, [&](int k, Slot& sl, size_t off, size_t len) -> int {
+            HGI_CUDA(ctx, cudaMemcpyAsync(sl.in.p, before + off, len, cudaMemcpyHostToDevice, sl.stream));
+            HGI_CUDA(ctx, cudaMemcpyAsync(sl.out.p, after + off, len, cudaMemcpyHostToDevice, sl.stream));
+            HGI_CUDA(ctx, hgi::launch_error_metrics(sl.in.p, sl.out.p, len, ctx->d_metrics + 2 * k, sl.stream));
+            HGI_CUDA(ctx, cudaMemcpyAsync(part[k], ctx->d_metrics + 2 * k, sizeof(part[k]), cudaMemcpyDeviceToHost, sl.stream));
+            return HGI_OK;
+        }, [&](int k) {
+            total += part[k][0];
+            if (part[k][1] > mx) mx = part[k][1];
+        });
         if (rc) return rc;
-        for (int k = 0; k < 2; ++k)
-            if (pending[k]) {
-                total += part[k][0];
-                if (part[k][1] > mx) mx = part[k][1];
-            }
     }
     if (sum_sq_out) *sum_sq_out = total;
     if (sd_int_out) *sd_int_out = n ? total / n : 0;  // src/main.rs:106 integer division
@@ -1216,18 +1152,16 @@ int hgi_decode_region_dev(hgi_ctx_t* ctx, const uint8_t* d_grids, uint32_t n_ima
     // the whole image into packed rows is a plain decode (with padded rows that one may write the padding)
     if (scale_log2 == 0 && r.width == width && r.height == height && out_pitch == pitch && pitch == width)
         return hgi_decode_dev_pitched(ctx, d_grids, n_images, width, height, pitch, params, d_out, stream);
-    DeviceGuard g(ctx);
-    if (!g.ok) return HGI_ERR_CUDA;
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-    Scratch* sc = scratch_for(ctx, st);
-    if (!sc) return HGI_ERR_ALLOC;
+    DevCall dc(ctx, stream, true);
+    if (dc.rc) return dc.rc;
     const uint32_t k = scale_log2;
     const uint8_t* src = d_grids + ((size_t)pl.window.y << k) * pitch + ((size_t)pl.window.x << k);
     const uint64_t row_step = (uint64_t)pitch << k, plane_stride = (uint64_t)pitch * height;
     const bool vec = aligned16(src) && row_step % 16 == 0 && (n_images == 1 || plane_stride % 16 == 0);
     // the last row of the last plane ends at its pitch: no 128-bit load may reach past that
     const uint64_t row_avail = pitch - ((uint64_t)pl.window.x << k);
-    return run_region(ctx, *sc, src, row_step, plane_stride, vec, row_avail, k, n_images, pl, r, params, d_out, out_pitch, st);
+    return run_region(ctx, *dc.sc, src, row_step, plane_stride, vec, row_avail, k, n_images, pl, r, params, d_out, out_pitch,
+                      dc.st);
 }
 
 int hgi_decode_region_u8(hgi_ctx_t* ctx, const uint8_t* grid, uint32_t width, uint32_t height, const hgi_params_t* params,
@@ -1247,8 +1181,8 @@ int hgi_decode_region_u8(hgi_ctx_t* ctx, const uint8_t* grid, uint32_t width, ui
     const uint64_t spitch = ((k <= 3 ? (uint64_t)ww << k : span) + 15) & ~(uint64_t)15;
     const size_t out_bytes = (size_t)r.width * r.height;
     Slot& sl = ctx->slots[0];
-    if (!sl.stream) HGI_CUDA(ctx, cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
-    rc = reserve(ctx, sl.in, (size_t)spitch * wh);
+    rc = slot_stream(ctx, 0);
+    if (!rc) rc = reserve(ctx, sl.in, (size_t)spitch * wh);
     if (!rc) rc = reserve(ctx, sl.out, out_bytes);
     if (rc) return rc;
     const uint8_t* src = grid + ((size_t)pl.window.y << k) * width + ((size_t)pl.window.x << k);
@@ -1256,9 +1190,7 @@ int hgi_decode_region_u8(hgi_ctx_t* ctx, const uint8_t* grid, uint32_t width, ui
     rc = cuda_rc(ctx, cudaMemcpy2DAsync(sl.in.p, spitch, src, src_pitch, span, wh, cudaMemcpyHostToDevice, sl.stream));
     if (!rc) rc = run_region(ctx, sl.scratch, sl.in.p, spitch, 0, true, spitch, k, 1, pl, r, params, sl.out.p, r.width, sl.stream);
     if (!rc) rc = cuda_rc(ctx, cudaMemcpyAsync(image_out, sl.out.p, out_bytes, cudaMemcpyDeviceToHost, sl.stream));
-    const cudaError_t e = cudaStreamSynchronize(sl.stream);   // nothing may still write into image_out on return
-    if (e != cudaSuccess && rc == HGI_OK) rc = fail(ctx, e);
-    return rc;
+    return drain(ctx, 1, rc);
 }
 
 /* ---- pool: several GPUs behind one handle -------------------------------------------------------------------- */
@@ -1297,15 +1229,10 @@ int plan_bands(uint32_t height, uint32_t levels, uint32_t n_bands, hgi_band_t* o
 int pool_wait(hgi_pool* pool, int rc)
 {
     for (size_t d = 0; d < pool->ctxs.size(); ++d) {
-        hgi_ctx* ctx = pool->ctxs[d];
-        DeviceGuard g(ctx);
-        for (int s = 0; s < pool->used[d]; ++s) {
-            const cudaError_t e = cudaStreamSynchronize(ctx->slots[s].stream);
-            if (e != cudaSuccess && rc == HGI_OK) rc = fail(ctx, e);
-        }
+        DeviceGuard g(pool->ctxs[d]);
+        rc = drain(pool->ctxs[d], pool->used[d], rc);
         pool->used[d] = 0;
     }
-    if (rc != HGI_OK) (void)cudaGetLastError();
     return rc;
 }
 
@@ -1333,10 +1260,11 @@ int band_async(hgi_ctx* ctx, int mode, const uint8_t* in, uint32_t w, const hgi_
                uint8_t* out, int* used)
 {
     Slot& sl = ctx->slots[0];
-    if (!sl.stream) HGI_CUDA(ctx, cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
+    int rc = slot_stream(ctx, 0);
+    if (rc) return rc;
     *used = 1;
     const size_t rows_in = b.in_y1 - b.y0, rows_out = b.y1 - b.y0;
-    int rc = reserve(ctx, sl.in, rows_in * w);
+    rc = reserve(ctx, sl.in, rows_in * w);
     if (!rc) rc = reserve(ctx, sl.out, rows_in * w);
     if (rc) return rc;
     HGI_CUDA(ctx, cudaMemcpyAsync(sl.in.p, in + (size_t)b.y0 * w, rows_in * w, cudaMemcpyHostToDevice, sl.stream));
@@ -1369,13 +1297,11 @@ int pool_bands_dev(hgi_pool* pool, int mode, const uint8_t* const* d_in, uint32_
     for (int k = 0; k < nb; ++k) {
         if (!d_in[k] || !d_out[k]) return HGI_ERR_INVALID_ARG;
         hgi_ctx* ctx = pool->ctxs[(size_t)k];
-        DeviceGuard g(ctx);
-        if (!g.ok) return HGI_ERR_CUDA;
-        Scratch* sc = scratch_for(ctx, ctx->stream);
-        if (!sc) return HGI_ERR_ALLOC;
+        DevCall dc(ctx, nullptr, true);
+        if (dc.rc) return dc.rc;
         const uint32_t rows_in = bands[(size_t)k].in_y1 - bands[(size_t)k].y0;
-        const int rc = run_dev_cached(ctx, *sc, mode, d_in[k], 1, w, rows_in, w, prm, mode == hgi::kModeEncode ? d_out[k] : nullptr,
-                                      mode == hgi::kModeEncode ? nullptr : d_out[k], nullptr, ctx->stream);
+        const int rc = run_dev_cached(ctx, *dc.sc, mode, d_in[k], 1, w, rows_in, w, prm, mode == hgi::kModeEncode ? d_out[k] : nullptr,
+                                      mode == hgi::kModeEncode ? nullptr : d_out[k], nullptr, dc.st);
         if (rc) return rc;
     }
     return HGI_OK;
@@ -1454,24 +1380,16 @@ int hgi_pool_synchronize(hgi_pool_t* pool)
 int hgi_pool_encode_batch_u8(hgi_pool_t* pool, const uint8_t* images, uint32_t n_images, uint32_t width, uint32_t height,
                              const hgi_params_t* params, uint8_t* grids_out, uint32_t* hist_out)
 {
-    if (!pool) return HGI_ERR_INVALID_ARG;
-    int rc = check_params(params, true);
-    if (rc) return rc;
-    if (!plane_size_ok(width, height, n_images)) return HGI_ERR_INVALID_ARG;
-    if ((size_t)width * height * n_images == 0) return HGI_OK;
-    if (!images || !grids_out) return HGI_ERR_INVALID_ARG;
+    if (int rc = check_job(pool, params, true, width, height, n_images, width, {images, grids_out}))
+        return rc == kEmptyJob ? HGI_OK : rc;
     return pool_batch(pool, hgi::kModeEncode, images, n_images, width, height, params, grids_out, hist_out);
 }
 
 int hgi_pool_decode_batch_u8(hgi_pool_t* pool, const uint8_t* grids, uint32_t n_images, uint32_t width, uint32_t height,
                              const hgi_params_t* params, uint8_t* images_out)
 {
-    if (!pool) return HGI_ERR_INVALID_ARG;
-    int rc = check_params(params, false);
-    if (rc) return rc;
-    if (!plane_size_ok(width, height, n_images)) return HGI_ERR_INVALID_ARG;
-    if ((size_t)width * height * n_images == 0) return HGI_OK;
-    if (!grids || !images_out) return HGI_ERR_INVALID_ARG;
+    if (int rc = check_job(pool, params, false, width, height, n_images, width, {grids, images_out}))
+        return rc == kEmptyJob ? HGI_OK : rc;
     return pool_batch(pool, hgi::kModeDecode, grids, n_images, width, height, params, images_out, nullptr);
 }
 
@@ -1492,46 +1410,34 @@ int hgi_pool_plan_bands(const hgi_pool_t* pool, uint32_t height, uint32_t levels
 int hgi_pool_encode_plane_u8(hgi_pool_t* pool, const uint8_t* image, uint32_t width, uint32_t height,
                              const hgi_params_t* params, uint8_t* grid_out)
 {
-    if (!pool) return HGI_ERR_INVALID_ARG;
-    int rc = check_params(params, true);
-    if (rc) return rc;
-    if (!plane_size_ok(width, height, 1)) return HGI_ERR_INVALID_ARG;
-    if ((size_t)width * height == 0) return HGI_OK;
-    if (!image || !grid_out) return HGI_ERR_INVALID_ARG;
+    if (int rc = check_job(pool, params, true, width, height, 1, width, {image, grid_out}))
+        return rc == kEmptyJob ? HGI_OK : rc;
     return pool_plane(pool, hgi::kModeEncode, image, width, height, params, grid_out);
 }
 
 int hgi_pool_decode_plane_u8(hgi_pool_t* pool, const uint8_t* grid, uint32_t width, uint32_t height,
                              const hgi_params_t* params, uint8_t* image_out)
 {
-    if (!pool) return HGI_ERR_INVALID_ARG;
-    int rc = check_params(params, false);
-    if (rc) return rc;
-    if (!plane_size_ok(width, height, 1)) return HGI_ERR_INVALID_ARG;
-    if ((size_t)width * height == 0) return HGI_OK;
-    if (!grid || !image_out) return HGI_ERR_INVALID_ARG;
+    if (int rc = check_job(pool, params, false, width, height, 1, width, {grid, image_out}))
+        return rc == kEmptyJob ? HGI_OK : rc;
     return pool_plane(pool, hgi::kModeDecode, grid, width, height, params, image_out);
 }
 
 int hgi_pool_encode_bands_dev(hgi_pool_t* pool, const uint8_t* const* d_bands_in, uint32_t width, uint32_t height,
                               const hgi_params_t* params, uint8_t* const* d_bands_out)
 {
-    if (!pool || !d_bands_in || !d_bands_out) return HGI_ERR_INVALID_ARG;
-    int rc = check_params(params, true);
-    if (rc) return rc;
-    if (!plane_size_ok(width, height, 1)) return HGI_ERR_INVALID_ARG;
-    if ((size_t)width * height == 0) return HGI_OK;
+    // the band arrays are checked with the handle, before the parameters
+    if (int rc = check_job(pool && d_bands_in && d_bands_out, params, true, width, height, 1, width, {}))
+        return rc == kEmptyJob ? HGI_OK : rc;
     return pool_bands_dev(pool, hgi::kModeEncode, d_bands_in, width, height, params, d_bands_out);
 }
 
 int hgi_pool_decode_bands_dev(hgi_pool_t* pool, const uint8_t* const* d_bands_in, uint32_t width, uint32_t height,
                               const hgi_params_t* params, uint8_t* const* d_bands_out)
 {
-    if (!pool || !d_bands_in || !d_bands_out) return HGI_ERR_INVALID_ARG;
-    int rc = check_params(params, false);
-    if (rc) return rc;
-    if (!plane_size_ok(width, height, 1)) return HGI_ERR_INVALID_ARG;
-    if ((size_t)width * height == 0) return HGI_OK;
+    // the band arrays are checked with the handle, before the parameters
+    if (int rc = check_job(pool && d_bands_in && d_bands_out, params, false, width, height, 1, width, {}))
+        return rc == kEmptyJob ? HGI_OK : rc;
     return pool_bands_dev(pool, hgi::kModeDecode, d_bands_in, width, height, params, d_bands_out);
 }
 

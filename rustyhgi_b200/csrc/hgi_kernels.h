@@ -55,7 +55,8 @@ struct PassArgs {
 // Dispatch of one pass.  By default every pass of a plane up to 65535 tiles tall goes to the register-prefetch SWAR
 // kernel (hgi_tile_fast.cu), taller planes to the generic kernel (hgi_tile_kernels.cu); `generic` forces the generic
 // kernel, the independent formulation the tests cross-check against.
-// Kernels launched so far by the calling thread's launch_* calls (for hgi_ctx_kernel_launches).
+// Kernels the calling thread's launch_* calls have launched and no context has been charged for yet: every launcher
+// adds one per kernel it launches, and the context whose work it was takes them (hgi_ctx_kernel_launches).
 uint64_t& launch_count();
 
 cudaError_t launch_tile_pass(int mode, int interp, const PassArgs& args, cudaStream_t stream, bool generic);

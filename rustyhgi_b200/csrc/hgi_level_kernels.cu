@@ -85,6 +85,7 @@ cudaError_t launch_seed(int /*mode*/, const uint8_t* src, uint8_t* dst, uint32_t
     if (sw == 0 || sh == 0 || n_images == 0) return cudaSuccess;
     dim3 grid((uint32_t)(((uint64_t)sw * sh + 255) / 256), 1, n_images < 65535u ? n_images : 65535u);
     hgi_seed_kernel<<<grid, 256, 0, stream>>>(src, dst, w, h, levels, sw, sh, n_images);
+    ++launch_count();
     return cudaGetLastError();
 }
 
@@ -103,6 +104,7 @@ static cudaError_t launch_level_t(const LevelArgs& a, cudaStream_t stream)
         hgi_level_kernel<MODE, INTERP, true><<<grid, block, 0, stream>>>(a);
     else
         hgi_level_kernel<kModeEncode, INTERP, false><<<grid, block, 0, stream>>>(a);
+    ++launch_count();
     return cudaGetLastError();
 }
 

@@ -264,6 +264,7 @@ cudaError_t launch_rgb_to_luma(const uint8_t* rgb, size_t n_pixels, uint8_t* lum
     if (blocks < 1) blocks = 1;
     if (blocks > 148 * 32) blocks = 148 * 32;
     hgi_luma_kernel<<<(uint32_t)blocks, 256, 0, stream>>>(rgb, n_pixels, luma, vec_ok);
+    ++launch_count();
     return cudaGetLastError();
 }
 
@@ -296,6 +297,7 @@ cudaError_t launch_histogram(const uint8_t* data, uint32_t w, uint32_t h, uint32
     if (bpi * n_images > 0x7FFFFFFFull) bpi = 0x7FFFFFFFull / n_images;
     if (bpi < 1) return cudaErrorInvalidConfiguration;
     hgi_hist_kernel<<<(uint32_t)(bpi * n_images), HT, kHistSmem, stream>>>(data, w, h, pitch, (uint32_t)bpi, hist_out);
+    ++launch_count();
     return cudaGetLastError();
 }
 
@@ -309,6 +311,7 @@ cudaError_t launch_rle_histogram(const uint8_t* data, size_t n, size_t block_byt
     const size_t gx = (segs + 127) / 128;
     if (gx > 0x7FFFFFFFull || n_blocks > 65535u) return cudaErrorInvalidConfiguration;
     hgi_rle_hist_kernel<<<dim3((uint32_t)gx, n_blocks), 128, 0, stream>>>(data, n, block_bytes, hist_out);
+    ++launch_count();
     return cudaGetLastError();
 }
 
@@ -321,6 +324,7 @@ cudaError_t launch_error_metrics(const uint8_t* before, const uint8_t* after, si
     uint64_t blocks = (n + 256 * 64 - 1) / (256 * 64);
     if (blocks > 148 * 16) blocks = 148 * 16;
     hgi_error_kernel<<<(uint32_t)blocks, 256, 0, stream>>>(before, after, n, out2, vec_ok);
+    ++launch_count();
     return cudaGetLastError();
 }
 

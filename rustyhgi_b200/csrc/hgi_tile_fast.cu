@@ -440,14 +440,18 @@ inline uint64_t split_min_tiles()
     static const uint64_t v = [] { const char* e = getenv("HGI_B200_SPLIT_MIN"); return e ? (uint64_t)atoll(e) : (uint64_t)(4 * 1480); }();
     return v;
 }
-#define kSplitMinTiles split_min_tiles()
+
+// One counted launch (hgi_ctx_kernel_launches) of a fast tile kernel.
+inline void launch_one(void (*kernel)(PassArgs), dim3 nb, cudaStream_t stream, const PassArgs& a)
+{
+    kernel<<<nb, NT, 0, stream>>>(a);
+    ++launch_count();
+}
 
 template <int MODE, int INTERP, bool IDENTITY, bool EXTRA, int NLEV, bool ALIGNED>
 cudaError_t launch_fast_split(PassArgs& a, uint32_t tiles_x, uint32_t tiles_y, cudaStream_t stream)
 {
     a.fast_tx = tiles_x;
-    a.fast_itx = a.w >= (uint32_t)(FMAX + 1) ? min(tiles_x, (a.w - (FMAX + 1)) / TW) : 0u;
-    a.fast_ity = a.h >= (uint32_t)(FMAX + 1) ? min(tiles_y, (a.h - (FMAX + 1)) / TH) : 0u;
     if (a.fast_itx == 0 || a.fast_ity == 0) a.fast_itx = a.fast_ity = 0;
     // the edge launches depend on nothing the interior launch writes: fork them onto the side stream when there is one
     const bool fork = a.fast_itx && a.side_stream && a.ev_fork && a.ev_join;
@@ -457,23 +461,16 @@ cudaError_t launch_fast_split(PassArgs& a, uint32_t tiles_x, uint32_t tiles_y, c
         if (e == cudaSuccess) e = cudaStreamWaitEvent(a.side_stream, a.ev_fork, 0);
         if (e != cudaSuccess) return e;
     }
-    if (a.fast_itx) {
-        const dim3 nb(a.fast_itx, a.fast_ity, a.n_images);
-        hgi_tile_fast_part_kernel<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 1><<<nb, NT, 0, stream>>>(a); ++launch_count();
-    }
+    if (a.fast_itx)
+        launch_one(hgi_tile_fast_part_kernel<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 1>, dim3(a.fast_itx, a.fast_ity, a.n_images),
+                   stream, a);
     const uint32_t ncr = tiles_x - a.fast_itx, nbr = tiles_y - a.fast_ity;
-    if (ncr && a.fast_ity) {   // right tile columns of the interior tile rows
-        const dim3 nb(ncr, a.fast_ity, a.n_images);
-        if (ncr == 1 && a.w == tiles_x * (uint32_t)TW) {
-            hgi_tile_fast_part_kernel<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 4><<<nb, NT, 0, es>>>(a); ++launch_count();
-        } else {
-            hgi_tile_fast_part_kernel<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 2><<<nb, NT, 0, es>>>(a); ++launch_count();
-        }
-    }
-    if (nbr) {                 // bottom tile rows
-        const dim3 nb(tiles_x, nbr, a.n_images);
-        hgi_tile_fast_part_kernel<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 3><<<nb, NT, 0, es>>>(a); ++launch_count();
-    }
+    if (ncr && a.fast_ity)     // right tile columns of the interior tile rows
+        launch_one(ncr == 1 && a.w == tiles_x * (uint32_t)TW ? hgi_tile_fast_part_kernel<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 4>
+                                                            : hgi_tile_fast_part_kernel<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 2>,
+                   dim3(ncr, a.fast_ity, a.n_images), es, a);
+    if (nbr)                   // bottom tile rows
+        launch_one(hgi_tile_fast_part_kernel<MODE, INTERP, IDENTITY, EXTRA, NLEV, ALIGNED, 3>, dim3(tiles_x, nbr, a.n_images), es, a);
     if (fork) {
         cudaError_t e = cudaEventRecord(a.ev_join, a.side_stream);
         if (e == cudaSuccess) e = cudaStreamWaitEvent(stream, a.ev_join, 0);
@@ -489,15 +486,16 @@ cudaError_t launch_fast_n(const PassArgs& args, cudaStream_t stream)
     if (tiles_x == 0 || tiles_y == 0 || args.n_images == 0) return cudaSuccess;
     if (tiles_y > 65535u) return cudaErrorInvalidConfiguration;
     const size_t plane = (size_t)args.pitch * args.h;
+    // interior tile columns / rows (tile + halo inside the plane), for the bodies without in-image predicates
+    const uint32_t itx = args.w >= (uint32_t)(FMAX + 1) ? min(tiles_x, (args.w - (FMAX + 1)) / TW) : 0u;
+    const uint32_t ity = args.h >= (uint32_t)(FMAX + 1) ? min(tiles_y, (args.h - (FMAX + 1)) / TH) : 0u;
     // L2 prefetch distance of the interior tiles of the quantizing encode, in residencies (148 SMs x 10 CTAs): that
     // kernel is bound by its instruction stream, so the DRAM latency of a tile's first loads is the one stall it cannot
     // cover with other work; fetching the tile into L2 about one residency earlier takes it away (-2..3 %, A/B sweep:
     // k = 0.5..2 alike, beyond k = 2.5 the lines are evicted before use and the kernel loses 8 %).  The DRAM-bound light
     // kernels lose with any distance (+20 % at k = 2) and do not carry the code.  HGI_B200_PREFETCH=<k> overrides, 0 = off.
     static const double pf_k = [] { const char* e = getenv("HGI_B200_PREFETCH"); return e ? atof(e) : 1.0; }();
-    const bool split = (MODE == kModeEncode && args.quant_error != 0 && ALIGNED && NLEV == 4 &&
-                        (uint64_t)tiles_x * tiles_y * args.n_images >= kSplitMinTiles);   // only the split launch has interior-only CTAs
-    const double pf_tiles = split ? pf_k * 1480.0 : 0.0;
+    const double pf_tiles = pf_k * 1480.0;
     const uint64_t tiles_img = (uint64_t)tiles_x * tiles_y;
     uint32_t pf_images = 0, pf_rows = 0;
     if (pf_tiles > 0.0) {
@@ -508,38 +506,38 @@ cudaError_t launch_fast_n(const PassArgs& args, cudaStream_t stream)
         PassArgs a = args;
         a.n_images = args.n_images - first < 65535u ? args.n_images - first : 65535u;
         a.src = args.src + (size_t)first * plane;
-        // bounds against this launch's grid: planes [0, n - pf_images) / interior tile rows [0, fast_ity - pf_rows)
-        const uint32_t ity = a.h >= (uint32_t)(FMAX + 1) ? min(tiles_y, (a.h - (FMAX + 1)) / TH) : 0u;
-        a.pf_zlim = pf_images ? (a.n_images > pf_images ? a.n_images - pf_images : 0u) : (pf_rows ? a.n_images : 0u);
-        a.pf_ylim = pf_rows ? (ity > pf_rows ? ity - pf_rows : 0u) : 0xFFFFFFFFu;
-        a.pf_src = a.src + ((uint64_t)pf_images * args.h + (uint64_t)pf_rows * TH) * args.pitch;
         if (args.grid_out) a.grid_out = args.grid_out + (size_t)first * plane;
         if (args.recon_out) a.recon_out = args.recon_out + (size_t)first * plane;
         if (args.c_recon) a.c_recon = args.c_recon + (size_t)first * args.cpitch * args.ch;
         if (args.c_q) a.c_q = args.c_q + (size_t)first * args.cpitch * args.ch;
+        a.fast_itx = itx;
+        a.fast_ity = ity;
+        a.fast_rcol = (itx + 1 == tiles_x && a.w == tiles_x * (uint32_t)TW) ? 1u : 0u;   // ONE right column, exactly TW wide
+        const bool extra = (a.recon_out != nullptr);
+        // a large slice of the quantizing encode runs as split launches (interior / edges); only their interior-only
+        // CTAs prefetch.  Small slices: one launch, less latency
+        const bool split = MODE == kModeEncode && a.quant_error != 0 && ALIGNED && NLEV == 4 &&
+                           tiles_img * a.n_images >= split_min_tiles();
+        // prefetch bounds against this slice's grid: planes [0, n - pf_images) / interior tile rows [0, ity - pf_rows)
+        const uint32_t zi = split ? pf_images : 0u, zr = split ? pf_rows : 0u;
+        a.pf_zlim = zi ? (a.n_images > zi ? a.n_images - zi : 0u) : (zr ? a.n_images : 0u);
+        a.pf_ylim = zr ? (ity > zr ? ity - zr : 0u) : 0xFFFFFFFFu;
+        a.pf_src = a.src + ((uint64_t)zi * args.h + (uint64_t)zr * TH) * args.pitch;
         const dim3 nb(tiles_x, tiles_y, a.n_images);
-        // interior tile columns / rows (tile + halo inside the plane), for the bodies without in-image predicates
-        a.fast_itx = a.w >= (uint32_t)(FMAX + 1) ? min(tiles_x, (a.w - (FMAX + 1)) / TW) : 0u;
-        a.fast_ity = a.h >= (uint32_t)(FMAX + 1) ? min(tiles_y, (a.h - (FMAX + 1)) / TH) : 0u;
-        a.fast_rcol = (a.fast_itx + 1 == tiles_x && a.w == tiles_x * (uint32_t)TW) ? 1u : 0u;   // ONE right column, exactly TW wide
         if (MODE == kModeDecode) {
-            hgi_tile_fast_kernel<kModeDecode, INTERP, true, false, NLEV, ALIGNED><<<nb, NT, 0, stream>>>(a); ++launch_count();
-        } else {
-            const bool extra = (a.recon_out != nullptr);
-            const bool ident = (a.quant_error == 0);
-            if (ident && !extra) { hgi_tile_fast_kernel<kModeEncode, INTERP, true, false, NLEV, ALIGNED><<<nb, NT, 0, stream>>>(a); ++launch_count(); }
-            else if (ident) { hgi_tile_fast_kernel<kModeEncode, INTERP, true, true, NLEV, ALIGNED><<<nb, NT, 0, stream>>>(a); ++launch_count(); }
-            else if constexpr (ALIGNED && NLEV == 4 && MODE == kModeEncode) {
-                if ((uint64_t)tiles_x * tiles_y * a.n_images >= kSplitMinTiles) {
-                    const cudaError_t es = extra ? launch_fast_split<kModeEncode, INTERP, false, true, NLEV, ALIGNED>(a, tiles_x, tiles_y, stream)
-                                                 : launch_fast_split<kModeEncode, INTERP, false, false, NLEV, ALIGNED>(a, tiles_x, tiles_y, stream);
-                    if (es != cudaSuccess) return es;
-                }   // small jobs: one launch, less latency
-                else if (!extra) { hgi_tile_fast_kernel<kModeEncode, INTERP, false, false, NLEV, ALIGNED><<<nb, NT, 0, stream>>>(a); ++launch_count(); }
-                else { hgi_tile_fast_kernel<kModeEncode, INTERP, false, true, NLEV, ALIGNED><<<nb, NT, 0, stream>>>(a); ++launch_count(); }
+            launch_one(hgi_tile_fast_kernel<kModeDecode, INTERP, true, false, NLEV, ALIGNED>, nb, stream, a);
+        } else if (a.quant_error == 0) {
+            launch_one(!extra ? hgi_tile_fast_kernel<kModeEncode, INTERP, true, false, NLEV, ALIGNED>
+                              : hgi_tile_fast_kernel<kModeEncode, INTERP, true, true, NLEV, ALIGNED>, nb, stream, a);
+        } else if (split) {
+            if constexpr (MODE == kModeEncode && ALIGNED && NLEV == 4) {
+                const cudaError_t es = extra ? launch_fast_split<kModeEncode, INTERP, false, true, NLEV, ALIGNED>(a, tiles_x, tiles_y, stream)
+                                             : launch_fast_split<kModeEncode, INTERP, false, false, NLEV, ALIGNED>(a, tiles_x, tiles_y, stream);
+                if (es != cudaSuccess) return es;
             }
-            else if (!extra) { hgi_tile_fast_kernel<kModeEncode, INTERP, false, false, NLEV, ALIGNED><<<nb, NT, 0, stream>>>(a); ++launch_count(); }
-            else { hgi_tile_fast_kernel<kModeEncode, INTERP, false, true, NLEV, ALIGNED><<<nb, NT, 0, stream>>>(a); ++launch_count(); }
+        } else {
+            launch_one(!extra ? hgi_tile_fast_kernel<kModeEncode, INTERP, false, false, NLEV, ALIGNED>
+                              : hgi_tile_fast_kernel<kModeEncode, INTERP, false, true, NLEV, ALIGNED>, nb, stream, a);
         }
         const cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return e;
