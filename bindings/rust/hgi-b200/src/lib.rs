@@ -166,3 +166,15 @@ pub fn plan_region(width: u32, height: u32, levels: u32, scale_log2: u32, region
     if rc != HGI_OK { return Err(format!("hgi_plan_region: {}", strerror(rc))); }
     Ok(plan)
 }
+
+/// `hgi_plan_crop`: the window every plane of a batched crop of this size decodes, placed for the origin `crop.0, crop.1`
+/// (pure host arithmetic).  Its width and height depend on the crop's size only.
+pub fn plan_crop(width: u32, height: u32, levels: u32, scale_log2: u32, crop: (u32, u32, u32, u32))
+                 -> Result<hgi_region_plan_t, String> {
+    let rect = hgi_rect_t { x: crop.0, y: crop.1, width: crop.2, height: crop.3 };
+    let mut plan = hgi_region_plan_t { scaled_width: 0, scaled_height: 0, levels: 0,
+                                       window: hgi_rect_t { x: 0, y: 0, width: 0, height: 0 }, crop_x: 0, crop_y: 0 };
+    let rc = unsafe { hgi_plan_crop(width, height, levels, scale_log2, &rect, &mut plan) };
+    if rc != HGI_OK { return Err(format!("hgi_plan_crop: {}", strerror(rc))); }
+    Ok(plan)
+}

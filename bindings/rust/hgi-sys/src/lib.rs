@@ -132,6 +132,12 @@ extern "C" {
     pub fn hgi_decode_region_u8(ctx: *mut hgi_ctx_t, grid: *const u8, width: u32, height: u32,
                                 params: *const hgi_params_t, scale_log2: u32, region: *const hgi_rect_t,
                                 image_out: *mut u8) -> c_int;
+    pub fn hgi_plan_crop(width: u32, height: u32, levels: u32, scale_log2: u32, crop: *const hgi_rect_t,
+                         plan_out: *mut hgi_region_plan_t) -> c_int;
+    pub fn hgi_decode_crops_dev(ctx: *mut hgi_ctx_t, d_grids: *const u8, n_images: u32, width: u32, height: u32,
+                                pitch: u32, params: *const hgi_params_t, scale_log2: u32, crop_width: u32,
+                                crop_height: u32, d_origins: *const i32, d_out: *mut u8, out_pitch: u32,
+                                stream: *mut c_void) -> c_int;
     pub fn hgi_pool_create(devices: *const c_int, n_devices: c_int, pool_out: *mut *mut hgi_pool_t) -> c_int;
     pub fn hgi_pool_destroy(pool: *mut hgi_pool_t);
     pub fn hgi_pool_size(pool: *const hgi_pool_t) -> c_int;

@@ -234,6 +234,26 @@ int hgi_decode_region_u8(hgi_ctx_t *ctx, const uint8_t *grid, uint32_t width, ui
                          const hgi_params_t *params, uint32_t scale_log2, const hgi_rect_t *region,
                          uint8_t *image_out);
 
+/* ---- batched crops: a same-sized rectangle at its own origin from every plane --------------- */
+/* The uniform window of a crop (DESIGN.md "Batched crops"), per axis with n = ws (hs), c = crop width (height), S' and
+   A as above: need = c + 2 S' + A - 1; D = n if need >= n, else n - floor((n - need) / A) * A; the window is
+   [min(floor(u / A) * A, n - D), + D).  It contains hgi_plan_region's window of the same rectangle, and its width and
+   height do not depend on crop->x, crop->y.  Pure host arithmetic.  HGI_ERR_INVALID_ARG as hgi_plan_region, and for a
+   NULL crop. */
+int hgi_plan_crop(uint32_t width, uint32_t height, uint32_t levels, uint32_t scale_log2, const hgi_rect_t *crop,
+                  hgi_region_plan_t *plan_out);
+/* `n_images` grid planes (as hgi_decode_region_dev) -> a crop_width x crop_height rectangle of each one's scaled image,
+   at that plane's own origin: d_origins[i] = {x, y} (int32, device memory, 4-byte aligned) is read on the device, when
+   the chain runs, and clamped to [0, ws - crop_width] x [0, hs - crop_height].  Output layout as hgi_decode_region_dev.
+   Enqueued on `stream`, no host synchronisation; once a first call has sized the scratch, a call of the same shapes
+   allocates nothing and may be captured into a caller's CUDA graph (origins rewritten in place before each replay).
+   HGI_ERR_INVALID_ARG: a crop of size 0 or larger than the scaled image, out_pitch < crop_width, NULL or misaligned
+   pointers (n_images > 0); HGI_ERR_UNSUPPORTED on HGI_PATH_PER_LEVEL. */
+int hgi_decode_crops_dev(hgi_ctx_t *ctx, const uint8_t *d_grids, uint32_t n_images, uint32_t width, uint32_t height,
+                         uint32_t pitch, const hgi_params_t *params, uint32_t scale_log2, uint32_t crop_width,
+                         uint32_t crop_height, const int32_t *d_origins, uint8_t *d_out, uint32_t out_pitch,
+                         void *stream);
+
 /* ---- pool: the GPUs of one box behind one handle ------------------------------------------ */
 /* The reference encodes one image per call on one thread (benches/bench.rs:54-110, src/main.rs:41-71); the path
    shards with no exchange between the shards (SURVEY.md 8e), so a pool drives one context per GPU from the calling

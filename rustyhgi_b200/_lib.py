@@ -82,6 +82,8 @@ PROTOTYPES = {
     "hgi_plan_region": (_int, [_u32, _u32, _u32, _u32, _pr, ctypes.POINTER(RegionPlanStruct)]),
     "hgi_decode_region_dev": (_int, [_vp, _vp, _u32, _u32, _u32, _u32, _pp, _u32, _pr, _vp, _u32, _vp]),
     "hgi_decode_region_u8": (_int, [_vp, _vp, _u32, _u32, _pp, _u32, _pr, _vp]),
+    "hgi_plan_crop": (_int, [_u32, _u32, _u32, _u32, _pr, ctypes.POINTER(RegionPlanStruct)]),
+    "hgi_decode_crops_dev": (_int, [_vp, _vp, _u32, _u32, _u32, _u32, _pp, _u32, _u32, _u32, _vp, _vp, _u32, _vp]),
     "hgi_pool_create": (_int, [_vp, _int, ctypes.POINTER(_vp)]),
     "hgi_pool_destroy": (None, [_vp]),
     "hgi_pool_size": (_int, [_vp]),

@@ -464,6 +464,35 @@ class Decoder:
         ctx.check(rc, "hgi_decode_region_dev")
         return out
 
+    def decode_crops_device(self, levels, grids, origins, size, scale_log2=0, out=None, stream=None):
+        """Batched crops (hgi_decode_crops_dev): for CUDA grids (n, h, w), packed or with padded rows, and a CUDA int32
+        tensor `origins` (n, 2) of (x, y) on their device, plane i's crop_w x crop_h rectangle of its scaled image at
+        origins[i] (clamped into it), byte-identical to `decode_device(levels, grids)[i, ::2^k, ::2^k]` sliced there.
+        `size` = (crop_w, crop_h).  The origins are read on the device when the chain runs, so they may come from device
+        code.  The result is (n, crop_h, crop_w); `out` may be such a tensor with padded rows, whose padding is left
+        untouched."""
+        import torch
+        t, n, h, w, pitch = _dev_planes(grids, "grids")
+        ctx = _ctx_for(self._ctx, t)
+        cw, ch = (int(v) for v in size)
+        if not isinstance(origins, torch.Tensor) or origins.dtype != torch.int32 or origins.device != t.device:
+            raise ValueError(f"origins must be an int32 tensor on {t.device}")
+        if tuple(origins.shape) != (n, 2) or not origins.is_contiguous():
+            raise ValueError(f"origins must be a contiguous ({n}, 2) tensor")
+        if min(cw, ch) < 0:
+            raise ValueError("size must be (crop_w, crop_h) with non-negative values")
+        if out is None:
+            out = torch.empty((n, ch, cw) if grids.dim() == 3 else (ch, cw), dtype=torch.uint8, device=t.device)
+        o, on, oh, ow, out_pitch = _dev_planes(out, "out")
+        if (on, oh, ow) != (n, ch, cw) or o.device != t.device:
+            raise ValueError(f"out must be ({n}, {ch}, {cw}) on {t.device}")
+        st = _stream_handle(stream, t.device)
+        p = _params(levels, self._interp)
+        rc = _lib.lib().hgi_decode_crops_dev(ctx._h, t.data_ptr(), n, w, h, pitch, ctypes.byref(p), int(scale_log2), cw, ch,
+                                             origins.data_ptr(), o.data_ptr(), out_pitch, st)
+        ctx.check(rc, "hgi_decode_crops_dev")
+        return out
+
 
 RegionPlan = collections.namedtuple("RegionPlan", "scaled_width scaled_height levels window crop_x crop_y")
 RegionPlan.__doc__ = """hgi_region_plan_t: the scaled image's size, the levels decoded on the window (L' = max(L - k, 0)),
@@ -487,6 +516,17 @@ def plan_region(width, height, levels, scale_log2=0, region=None):
     rc = _lib.lib().hgi_plan_region(int(width), int(height), int(levels), int(scale_log2), _rect(region), ctypes.byref(p))
     if rc:
         raise HgiError(rc, "hgi_plan_region")
+    w = p.window
+    return RegionPlan(p.scaled_width, p.scaled_height, p.levels, (w.x, w.y, w.width, w.height), p.crop_x, p.crop_y)
+
+
+def plan_crop(width, height, levels, scale_log2, crop):
+    """hgi_plan_crop: the window a batched crop of `crop` = (x, y, width, height) (scaled coordinates) decodes.  Its
+    size depends on the crop's size only; the window of every plane of a batch has that size.  Pure host arithmetic."""
+    p = RegionPlanStruct()
+    rc = _lib.lib().hgi_plan_crop(int(width), int(height), int(levels), int(scale_log2), _rect(crop), ctypes.byref(p))
+    if rc:
+        raise HgiError(rc, "hgi_plan_crop")
     w = p.window
     return RegionPlan(p.scaled_width, p.scaled_height, p.levels, (w.x, w.y, w.width, w.height), p.crop_x, p.crop_y)
 

@@ -733,13 +733,33 @@ int plan_region(uint32_t w, uint32_t h, uint32_t levels, uint32_t k, const hgi_r
     return HGI_OK;
 }
 
-// Argument checks shared by the region entry points: decode's, plus the region.
+// Window of a batched crop (DESIGN.md "Batched crops"): hgi::crop_axis on each axis, so the window's extent depends on
+// the crop's size only and every plane of a batch decodes a window of that extent.  `crop` is required.
+int plan_crop(uint32_t w, uint32_t h, uint32_t levels, uint32_t k, const hgi_rect_t* crop, hgi_region_plan_t* p,
+              hgi_rect_t* r_out)
+{
+    if (!crop) return HGI_ERR_INVALID_ARG;
+    hgi_region_plan_t tight;
+    hgi_rect_t r;
+    if (int rc = plan_region(w, h, levels, k, crop, &tight, &r)) return rc;   // the same limits as a region
+    const uint32_t lp = tight.levels;
+    const hgi::CropAxis x = hgi::crop_axis(tight.scaled_width, r.width, lp, lp > 4 ? lp : 4, r.x);
+    const hgi::CropAxis y = hgi::crop_axis(tight.scaled_height, r.height, lp, lp, r.y);
+    *p = hgi_region_plan_t{tight.scaled_width, tight.scaled_height, lp, hgi_rect_t{x.start, y.start, x.extent, y.extent},
+                           r.x - x.start, r.y - y.start};
+    *r_out = r;
+    return HGI_OK;
+}
+
+using PlanFn = int (*)(uint32_t, uint32_t, uint32_t, uint32_t, const hgi_rect_t*, hgi_region_plan_t*, hgi_rect_t*);
+
+// Argument checks shared by the region and crop entry points: decode's, plus the rectangle (`plan`: its window rule).
 int check_region(hgi_ctx* ctx, const hgi_params_t* prm, uint32_t w, uint32_t h, uint32_t n_images, uint32_t pitch,
-                 uint32_t k, const hgi_rect_t* region, hgi_region_plan_t* pl, hgi_rect_t* r)
+                 uint32_t k, const hgi_rect_t* region, hgi_region_plan_t* pl, hgi_rect_t* r, PlanFn plan = plan_region)
 {
     int rc = check_job(ctx, prm, false, w, h, n_images, pitch, {});
     if (rc < 0) return rc;   // an empty job is the region rules' to judge
-    rc = plan_region(w, h, prm->levels, k, region, pl, r);
+    rc = plan(w, h, prm->levels, k, region, pl, r);
     if (rc) return rc;
     if (ctx->path == HGI_PATH_PER_LEVEL) return HGI_ERR_UNSUPPORTED;   // the window decode is a tile path
     return HGI_OK;
@@ -747,10 +767,12 @@ int check_region(hgi_ctx* ctx, const hgi_params_t* prm, uint32_t w, uint32_t h, 
 
 // Scalable decode of `n_images` planes: gather the window lattice (src + img * plane_stride + v * row_step + (u << k),
 // see launch_region_gather) into dense planes, decode them on the tile path with L' levels, crop the region into
-// d_out.  Launches plainly: region chains are not graph-cached.
+// d_out.  Launches plainly: region chains are not graph-cached.  With `crops.xy` every plane gathers and crops at its
+// own origin (hgi::launch_region_gather); `pl` is then the uniform window of plan_crop, whose origin is not used.
 int run_region(hgi_ctx* ctx, Scratch& sc, const uint8_t* src, uint64_t row_step, uint64_t plane_stride, bool vec,
                uint64_t row_avail, uint32_t k, uint32_t n_images, const hgi_region_plan_t& pl, const hgi_rect_t& r,
-               const hgi_params_t* prm, uint8_t* d_out, uint32_t out_pitch, cudaStream_t st)
+               const hgi_params_t* prm, uint8_t* d_out, uint32_t out_pitch, cudaStream_t st,
+               const hgi::CropOrigins& crops = hgi::CropOrigins{})
 {
     const uint32_t ww = pl.window.width, wh = pl.window.height, wpitch = align16(ww);
     const size_t bytes = (size_t)n_images * wpitch * wh;
@@ -759,7 +781,7 @@ int run_region(hgi_ctx* ctx, Scratch& sc, const uint8_t* src, uint64_t row_step,
     if (!rc && levels) rc = reserve(ctx, sc, sc.region_out, bytes);
     if (rc) return rc;
     HGI_CUDA(ctx, hgi::launch_region_gather(src, row_step, plane_stride, k, ww, wh, wpitch, n_images, vec, row_avail,
-                                            sc.region_in.p, st));
+                                            sc.region_in.p, st, crops));
     const uint8_t* win = sc.region_in.p;
     if (levels) {
         rc = run_tile_path(ctx, sc, hgi::kModeDecode, sc.region_in.p, n_images, ww, wh, wpitch, levels, prm, nullptr,
@@ -768,7 +790,7 @@ int run_region(hgi_ctx* ctx, Scratch& sc, const uint8_t* src, uint64_t row_step,
         win = sc.region_out.p;
     }
     HGI_CUDA(ctx, hgi::launch_region_crop(win, wpitch, wh, pl.crop_x, pl.crop_y, r.width, r.height, n_images, d_out,
-                                          out_pitch, st));
+                                          out_pitch, st, crops));
     return HGI_OK;
 }
 
@@ -1191,6 +1213,37 @@ int hgi_decode_region_u8(hgi_ctx_t* ctx, const uint8_t* grid, uint32_t width, ui
     if (!rc) rc = run_region(ctx, sl.scratch, sl.in.p, spitch, 0, true, spitch, k, 1, pl, r, params, sl.out.p, r.width, sl.stream);
     if (!rc) rc = cuda_rc(ctx, cudaMemcpyAsync(image_out, sl.out.p, out_bytes, cudaMemcpyDeviceToHost, sl.stream));
     return drain(ctx, 1, rc);
+}
+
+int hgi_plan_crop(uint32_t width, uint32_t height, uint32_t levels, uint32_t scale_log2, const hgi_rect_t* crop,
+                  hgi_region_plan_t* plan_out)
+{
+    if (!plan_out) return HGI_ERR_INVALID_ARG;
+    hgi_rect_t r;
+    return plan_crop(width, height, levels, scale_log2, crop, plan_out, &r);
+}
+
+int hgi_decode_crops_dev(hgi_ctx_t* ctx, const uint8_t* d_grids, uint32_t n_images, uint32_t width, uint32_t height,
+                         uint32_t pitch, const hgi_params_t* params, uint32_t scale_log2, uint32_t crop_width,
+                         uint32_t crop_height, const int32_t* d_origins, uint8_t* d_out, uint32_t out_pitch, void* stream)
+{
+    hgi_region_plan_t pl;
+    hgi_rect_t r;
+    const hgi_rect_t crop{0, 0, crop_width, crop_height};
+    int rc = check_region(ctx, params, width, height, n_images, pitch, scale_log2, &crop, &pl, &r, plan_crop);
+    if (rc) return rc;
+    if (out_pitch < crop_width) return HGI_ERR_INVALID_ARG;
+    if (n_images == 0) return HGI_OK;
+    if (!d_grids || !d_out || !d_origins || ((uintptr_t)d_origins & 3u)) return HGI_ERR_INVALID_ARG;
+    DevCall dc(ctx, stream, true);
+    if (dc.rc) return dc.rc;
+    const uint32_t k = scale_log2;
+    const uint64_t row_step = (uint64_t)pitch << k, plane_stride = (uint64_t)pitch * height;
+    // each plane's window starts at a multiple of 16 bytes of its row (U0 << k, U0 a multiple of max(S', 16))
+    const bool vec = aligned16(d_grids) && row_step % 16 == 0 && (n_images == 1 || plane_stride % 16 == 0);
+    const hgi::CropOrigins crops{d_origins, pl.scaled_width, pl.scaled_height, crop_width, crop_height, pl.levels};
+    return run_region(ctx, *dc.sc, d_grids, row_step, plane_stride, vec, pitch, k, n_images, pl, r, params, d_out, out_pitch,
+                      dc.st, crops);
 }
 
 /* ---- pool: several GPUs behind one handle -------------------------------------------------------------------- */

@@ -80,13 +80,40 @@ cudaError_t launch_decimate(const uint8_t* src, uint32_t pitch, uint32_t h, uint
 // Scalable decode (hgi_region.cu).  Gather: dst[img][v][u] = src[img * plane_stride + v * row_step + (u << k)] for the
 // ww x wh window of `n_images` planes, rows of dst `dpitch` (16-byte multiple) apart, zero padded; `vec`: src, row_step
 // and plane_stride are 16-byte aligned and every source row is readable for `row_avail` bytes (128-bit loads).
+// Batched crops (DESIGN.md "Batched crops"): every plane decodes a window of the same extent at its own origin.  One
+// axis of the rule: n = scaled extent, c = crop extent (1 <= c <= n), coarse step S' = 2^s_log2, start alignment
+// A = 2^a_log2 (max(S', 16) on columns, S' on rows), u = the crop's origin.  The tight window of a region needs at most
+// need = c + 2 S' + A - 1 cells; the extent is n, or else the one in [need, need + A) that leaves n - extent a multiple
+// of A, so that the start min(floor(u / A) * A, n - extent) is A-aligned and the window never leaves the image.
+struct CropAxis {
+    uint32_t start, extent;
+};
+__host__ __device__ inline CropAxis crop_axis(uint32_t n, uint32_t c, uint32_t s_log2, uint32_t a_log2, uint32_t u)
+{
+    const uint64_t need = (uint64_t)c + (2ull << s_log2) + (1ull << a_log2) - 1;
+    const uint32_t extent = need >= n ? n : n - (uint32_t)(((n - need) >> a_log2) << a_log2);
+    const uint32_t start = (uint32_t)(((uint64_t)u >> a_log2) << a_log2), last = n - extent;
+    return CropAxis{start < last ? start : last, extent};
+}
+// The per-plane origins of a crop batch: xy[img] = (x, y), read on the device and clamped to [0, ws - cw] x [0, hs - ch].
+struct CropOrigins {
+    const int32_t* xy;       // null: every plane uses the window of the launch (hgi_decode_region_*)
+    uint32_t ws, hs;         // scaled image
+    uint32_t cw, ch;         // crop size
+    uint32_t lp;             // L' = log2 of the coarse step S'
+};
+
 cudaError_t launch_region_gather(const uint8_t* src, uint64_t row_step, uint64_t plane_stride, uint32_t k, uint32_t ww,
                                  uint32_t wh, uint32_t dpitch, uint32_t n_images, bool vec, uint64_t row_avail,
-                                 uint8_t* dst, cudaStream_t stream);
+                                 uint8_t* dst, cudaStream_t stream, const CropOrigins& crops = CropOrigins{});
 // Crop: out[img][r][j] = win[img][cy + r][cx + j] (window planes wpitch x wh) for the rw x rh rectangle; output rows
 // out_pitch apart, planes out_pitch * rh apart; no byte outside the rectangle is written.
+// With `crops.xy`: plane img's window starts at (U0, V0) = crop_axis(...).start of its clamped origin (x, y), the gather
+// reads from src + V0 * row_step + (U0 << k) with row_avail - (U0 << k) readable bytes, and the crop takes (cx, cy) =
+// (x - U0, y - V0) instead of the arguments.
 cudaError_t launch_region_crop(const uint8_t* win, uint32_t wpitch, uint32_t wh, uint32_t cx, uint32_t cy, uint32_t rw,
-                               uint32_t rh, uint32_t n_images, uint8_t* out, uint32_t out_pitch, cudaStream_t stream);
+                               uint32_t rh, uint32_t n_images, uint8_t* out, uint32_t out_pitch, cudaStream_t stream,
+                               const CropOrigins& crops = CropOrigins{});
 cudaError_t launch_seed(int mode, const uint8_t* src, uint8_t* dst, uint32_t w, uint32_t h,
                         uint32_t levels, uint32_t n_images, cudaStream_t stream);
 cudaError_t launch_level(int mode, int interp, const LevelArgs& args, cudaStream_t stream);

@@ -62,16 +62,31 @@ __device__ __forceinline__ uint4 gather_vec(const uint8_t* __restrict__ srow, ui
     }
 }
 
+// Plane img of a crop batch: its origin (x, y) clamped into the scaled image, and the start (x0, y0) of its window.
+struct CropWindow {
+    uint32_t x, y, x0, y0;
+};
+__device__ __forceinline__ CropWindow crop_window(const CropOrigins& co, uint64_t img)
+{
+    const int32_t ox = __ldg(co.xy + 2 * img), oy = __ldg(co.xy + 2 * img + 1);   // 4-byte aligned only
+    const uint32_t mx = co.ws - co.cw, my = co.hs - co.ch;
+    const uint32_t x = ox < 0 ? 0u : ((uint32_t)ox > mx ? mx : (uint32_t)ox);
+    const uint32_t y = oy < 0 ? 0u : ((uint32_t)oy > my ? my : (uint32_t)oy);
+    const uint32_t ax = co.lp > 4u ? co.lp : 4u;
+    return CropWindow{x, y, crop_axis(co.ws, co.cw, co.lp, ax, x).start, crop_axis(co.hs, co.ch, co.lp, co.lp, y).start};
+}
+
 // dst[img][v][u] = src[img * plane_stride + v * row_step + (u << k)] for u < ww, zero for ww <= u < dpitch.
 // One thread writes 16 output bytes; a flat grid-stride loop over (window row, chunk) has no limit on the number of
 // rows.  `vec`: the source rows are 16-byte aligned and readable for `row_avail` bytes, so chunks whose whole source
 // run lies inside that take the 128-bit path (k <= 3); the others, and k >= 4 (one point per 16-byte chunk: a warp
-// reads a contiguous run of every sector as in hgi_decimate_kernel), load point by point.
-template <int K>
+// reads a contiguous run of every sector as in hgi_decimate_kernel), load point by point.  CROPS: plane img reads its
+// own window, see launch_region_gather.
+template <int K, bool CROPS>
 __global__ void __launch_bounds__(kCopyThreads)
 hgi_region_gather_kernel(const uint8_t* __restrict__ src, uint64_t row_step, uint64_t plane_stride, uint32_t kshift,
                          uint32_t ww, uint32_t wh, uint32_t dpitch, uint64_t n_rows, uint32_t vec, uint64_t row_avail,
-                         uint8_t* __restrict__ dst)
+                         uint8_t* __restrict__ dst, CropOrigins co)
 {
     const uint32_t cpr = dpitch / 16u;
     const uint64_t total = n_rows * cpr;
@@ -80,8 +95,15 @@ hgi_region_gather_kernel(const uint8_t* __restrict__ src, uint64_t row_step, uin
         const uint32_t c = (uint32_t)(it - row * cpr);
         const uint64_t img = row / wh, v = row - img * wh;
         const uint8_t* srow = src + img * plane_stride + v * row_step;
+        uint64_t avail = row_avail;
+        if constexpr (CROPS) {
+            const CropWindow cw = crop_window(co, img);
+            const uint64_t x0 = (uint64_t)cw.x0 << kshift;   // a multiple of 16: the start is aligned to max(S', 16)
+            srow += cw.y0 * row_step + x0;
+            avail -= x0;
+        }
         uint4 out;
-        if (K >= 0 && vec && 16u * c + 16u <= ww && ((uint64_t)(c + 1) << (4 + K)) <= row_avail) {
+        if (K >= 0 && vec && 16u * c + 16u <= ww && ((uint64_t)(c + 1) << (4 + K)) <= avail) {
             out = gather_vec<K < 0 ? 0 : K>(srow, c);
         } else {
             uint32_t o[4] = {0u, 0u, 0u, 0u};
@@ -100,9 +122,12 @@ hgi_region_gather_kernel(const uint8_t* __restrict__ src, uint64_t row_step, uin
 // out_pitch * rh.  Threads own 16-byte-aligned chunks of the output address space: whole chunks inside the
 // rectangle row are one 128-bit store built from two aligned 128-bit loads of the window row (funnel shift by the
 // misalignment); the chunks at the two ends of a row store byte by byte, so nothing outside the rectangle is written.
+// CROPS: (cx, cy) is plane img's own, from its origin and window start.
+template <bool CROPS>
 __global__ void __launch_bounds__(kCopyThreads)
 hgi_region_crop_kernel(const uint8_t* __restrict__ win, uint32_t wpitch, uint32_t wh, uint32_t cx, uint32_t cy,
-                       uint32_t rw, uint32_t rh, uint64_t n_rows, uint8_t* __restrict__ out, uint32_t out_pitch)
+                       uint32_t rw, uint32_t rh, uint64_t n_rows, uint8_t* __restrict__ out, uint32_t out_pitch,
+                       CropOrigins co)
 {
     const uint32_t cpr = (rw + 30u) / 16u + 1u;   // most chunks a row of rw bytes can touch
     const uint64_t total = n_rows * cpr;
@@ -111,7 +136,13 @@ hgi_region_crop_kernel(const uint8_t* __restrict__ win, uint32_t wpitch, uint32_
         const uint32_t c = (uint32_t)(it - row * cpr);
         const uint64_t img = row / rh, r = row - img * rh;
         uint8_t* drow = out + row * out_pitch;
-        const uint8_t* srow = win + (img * wh + cy + r) * wpitch + cx;
+        uint32_t ox = cx, oy = cy;
+        if constexpr (CROPS) {
+            const CropWindow cw = crop_window(co, img);
+            ox = cw.x - cw.x0;
+            oy = cw.y - cw.y0;
+        }
+        const uint8_t* srow = win + (img * wh + oy + r) * wpitch + ox;
         const int64_t j0 = 16 * (int64_t)c - (int64_t)((uintptr_t)drow & 15u);
         if (j0 >= (int64_t)rw) continue;
         if (j0 >= 0 && j0 + 16 <= (int64_t)rw) {
@@ -136,33 +167,46 @@ hgi_region_crop_kernel(const uint8_t* __restrict__ win, uint32_t wpitch, uint32_
     }
 }
 
+template <bool CROPS>
+void gather(const uint8_t* src, uint64_t row_step, uint64_t plane_stride, uint32_t k, uint32_t ww, uint32_t wh,
+            uint32_t dpitch, uint64_t n_rows, bool vec, uint64_t row_avail, uint8_t* dst, cudaStream_t stream,
+            const CropOrigins& co)
+{
+    const uint32_t nb = copy_blocks(n_rows * (dpitch / 16u));
+    switch (k) {
+        case 0: hgi_region_gather_kernel<0, CROPS><<<nb, kCopyThreads, 0, stream>>>(src, row_step, plane_stride, k, ww, wh, dpitch, n_rows, vec, row_avail, dst, co); break;
+        case 1: hgi_region_gather_kernel<1, CROPS><<<nb, kCopyThreads, 0, stream>>>(src, row_step, plane_stride, k, ww, wh, dpitch, n_rows, vec, row_avail, dst, co); break;
+        case 2: hgi_region_gather_kernel<2, CROPS><<<nb, kCopyThreads, 0, stream>>>(src, row_step, plane_stride, k, ww, wh, dpitch, n_rows, vec, row_avail, dst, co); break;
+        case 3: hgi_region_gather_kernel<3, CROPS><<<nb, kCopyThreads, 0, stream>>>(src, row_step, plane_stride, k, ww, wh, dpitch, n_rows, vec, row_avail, dst, co); break;
+        default: hgi_region_gather_kernel<-1, CROPS><<<nb, kCopyThreads, 0, stream>>>(src, row_step, plane_stride, k, ww, wh, dpitch, n_rows, 0u, 0u, dst, co); break;
+    }
+}
+
 }  // namespace
 
 cudaError_t launch_region_gather(const uint8_t* src, uint64_t row_step, uint64_t plane_stride, uint32_t k, uint32_t ww,
                                  uint32_t wh, uint32_t dpitch, uint32_t n_images, bool vec, uint64_t row_avail,
-                                 uint8_t* dst, cudaStream_t stream)
+                                 uint8_t* dst, cudaStream_t stream, const CropOrigins& crops)
 {
     if (ww == 0 || wh == 0 || n_images == 0) return cudaSuccess;
     const uint64_t n_rows = (uint64_t)n_images * wh;
-    const uint32_t nb = copy_blocks(n_rows * (dpitch / 16u));
-    switch (k) {
-        case 0: hgi_region_gather_kernel<0><<<nb, kCopyThreads, 0, stream>>>(src, row_step, plane_stride, k, ww, wh, dpitch, n_rows, vec, row_avail, dst); break;
-        case 1: hgi_region_gather_kernel<1><<<nb, kCopyThreads, 0, stream>>>(src, row_step, plane_stride, k, ww, wh, dpitch, n_rows, vec, row_avail, dst); break;
-        case 2: hgi_region_gather_kernel<2><<<nb, kCopyThreads, 0, stream>>>(src, row_step, plane_stride, k, ww, wh, dpitch, n_rows, vec, row_avail, dst); break;
-        case 3: hgi_region_gather_kernel<3><<<nb, kCopyThreads, 0, stream>>>(src, row_step, plane_stride, k, ww, wh, dpitch, n_rows, vec, row_avail, dst); break;
-        default: hgi_region_gather_kernel<-1><<<nb, kCopyThreads, 0, stream>>>(src, row_step, plane_stride, k, ww, wh, dpitch, n_rows, 0u, 0u, dst); break;
-    }
+    if (crops.xy) gather<true>(src, row_step, plane_stride, k, ww, wh, dpitch, n_rows, vec, row_avail, dst, stream, crops);
+    else gather<false>(src, row_step, plane_stride, k, ww, wh, dpitch, n_rows, vec, row_avail, dst, stream, crops);
     ++launch_count();
     return cudaGetLastError();
 }
 
 cudaError_t launch_region_crop(const uint8_t* win, uint32_t wpitch, uint32_t wh, uint32_t cx, uint32_t cy, uint32_t rw,
-                               uint32_t rh, uint32_t n_images, uint8_t* out, uint32_t out_pitch, cudaStream_t stream)
+                               uint32_t rh, uint32_t n_images, uint8_t* out, uint32_t out_pitch, cudaStream_t stream,
+                               const CropOrigins& crops)
 {
     if (rw == 0 || rh == 0 || n_images == 0) return cudaSuccess;
     const uint64_t n_rows = (uint64_t)n_images * rh;
     const uint32_t nb = copy_blocks(n_rows * ((rw + 30u) / 16u + 1u));
-    hgi_region_crop_kernel<<<nb, kCopyThreads, 0, stream>>>(win, wpitch, wh, cx, cy, rw, rh, n_rows, out, out_pitch);
+    if (crops.xy)
+        hgi_region_crop_kernel<true><<<nb, kCopyThreads, 0, stream>>>(win, wpitch, wh, cx, cy, rw, rh, n_rows, out, out_pitch, crops);
+    else
+        hgi_region_crop_kernel<false><<<nb, kCopyThreads, 0, stream>>>(win, wpitch, wh, cx, cy, rw, rh, n_rows, out, out_pitch, crops);
     ++launch_count();
     return cudaGetLastError();
 }
