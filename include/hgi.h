@@ -105,7 +105,8 @@ int hgi_ctx_set_path(hgi_ctx_t *ctx, int path /* hgi_path_t */);
    kernels and D2H of different chunks overlap).  0 = the default (64 MiB, 3 slots; HGI_B200_CHUNK_MB and
    HGI_B200_SLOTS in the environment override the default).  A non-zero `chunk_mb` is also the chunk of
    hgi_histogram_u8 / hgi_error_metrics_u8 (MiB) and hgi_rgb_to_luma_u8 (Mi pixels), which alternate their chunks
-   between two slots (defaults: 1024 / 256 MiB / 64 Mi pixels). */
+   between two slots (defaults: 1024 / 256 MiB / 64 Mi pixels; hgi_histogram_u8 counts at most 4095 MiB per chunk,
+   so that its 32-bit device bins cannot overflow). */
 int hgi_ctx_set_pipeline(hgi_ctx_t *ctx, uint32_t chunk_mb, uint32_t slots);
 int hgi_ctx_synchronize(hgi_ctx_t *ctx);
 /* cudaError_t of the last failing runtime call (0 if none) and its string. */
@@ -181,6 +182,9 @@ int hgi_decode_dev(hgi_ctx_t *ctx, const uint8_t *d_grids, uint32_t n_images, ui
                    void *stream);
 int hgi_rgb_to_luma_dev(hgi_ctx_t *ctx, const uint8_t *d_rgb, size_t n_pixels, uint8_t *d_luma_out,
                         void *stream);
+/* `n_images` packed planes of `n_per_image` bytes each.  The bins are 32-bit and the count is one launch with a block
+   or more per image: n_per_image >= 2^32 or n_images >= 2^31 is HGI_ERR_INVALID_ARG (so is d_hist_out with
+   width * height >= 2^32 or n_images >= 2^31 in the encode entry points). */
 int hgi_histogram_dev(hgi_ctx_t *ctx, const uint8_t *d_grid, size_t n_per_image,
                       uint32_t n_images, uint32_t *d_hist_out /* [n_images][256], overwritten */,
                       void *stream);

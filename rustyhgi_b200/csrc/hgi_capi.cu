@@ -590,6 +590,9 @@ int run_dev_cached(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint
 // Limits of the kernels' 32-bit offset arithmetic (tile-relative offsets up to 64 rows * pitch): rows shorter than 2^26
 // bytes; the per-image residual histogram has 32-bit bins.
 constexpr uint32_t kMaxPitch = 1u << 26;
+// The residual histogram is one launch with at least one block per image, and a grid holds at most 2^31 - 1 blocks
+// (its bins for that many images would take 2 TiB, more than any device has).
+constexpr uint32_t kMaxHistImages = 0x7FFFFFFFu;
 
 int cuda_rc(hgi_ctx* ctx, cudaError_t e) { return e == cudaSuccess ? HGI_OK : fail(ctx, e); }
 
@@ -954,7 +957,7 @@ int hgi_encode_dev_pitched(hgi_ctx_t* ctx, const uint8_t* d_images, uint32_t n_i
                            uint32_t pitch, const hgi_params_t* params, uint8_t* d_grids_out, uint8_t* d_recon_out,
                            uint32_t* d_hist_out, void* stream)
 {
-    const bool bins_ok = !d_hist_out || (uint64_t)width * height < (1ull << 32);   // u32 bins
+    const bool bins_ok = !d_hist_out || ((uint64_t)width * height < (1ull << 32) && n_images <= kMaxHistImages);   // u32 bins
     if (int rc = check_job(ctx, params, true, width, height, n_images, pitch, {d_images, d_grids_out}, bins_ok))
         return rc == kEmptyJob ? HGI_OK : rc;
     DevCall dc(ctx, stream, true);
@@ -992,6 +995,7 @@ int hgi_histogram_dev(hgi_ctx_t* ctx, const uint8_t* d_grid, size_t n_per_image,
 {
     if (!ctx || !d_hist_out) return HGI_ERR_INVALID_ARG;
     if (n_per_image >= ((size_t)1 << 32)) return HGI_ERR_INVALID_ARG;  // u32 bins
+    if (n_images > kMaxHistImages) return HGI_ERR_INVALID_ARG;
     if (n_images == 0) return HGI_OK;
     if (!d_grid && n_per_image) return HGI_ERR_INVALID_ARG;
     DevCall dc(ctx, stream);
@@ -1109,8 +1113,10 @@ int hgi_histogram_u8(hgi_ctx_t* ctx, const uint8_t* grid, size_t n, uint64_t his
     if (!grid) return HGI_ERR_INVALID_ARG;
     DeviceGuard g(ctx);
     if (!g.ok) return HGI_ERR_CUDA;
-    // keeps the u32 device bins far from overflow (and the length a uint32_t)
-    const size_t chunk = ctx->chunk_bytes ? ctx->chunk_bytes : ((size_t)1 << 30);
+    // A chunk shorter than 2^32 bytes cannot overflow the u32 device bins and its length fits the launch's uint32_t;
+    // the default stays far below that, a larger pipeline chunk (up to 4096 MiB) is cut to 4095 MiB.
+    size_t chunk = ctx->chunk_bytes ? ctx->chunk_bytes : ((size_t)1 << 30);
+    if (chunk > ((size_t)4095 << 20)) chunk = (size_t)4095 << 20;
     uint32_t part[2][256];
     return run_chunks(ctx, n, chunk, 1, 0, sizeof(part[0]), [&](int k, Slot& sl, size_t off, size_t len) -> int {
         HGI_CUDA(ctx, cudaMemcpyAsync(sl.in.p, grid + off, len, cudaMemcpyHostToDevice, sl.stream));
