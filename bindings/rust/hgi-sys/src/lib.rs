@@ -83,6 +83,7 @@ extern "C" {
     pub fn hgi_strerror(status: c_int) -> *const c_char;
     pub fn hgi_ctx_create(device: c_int, ctx_out: *mut *mut hgi_ctx_t) -> c_int;
     pub fn hgi_ctx_destroy(ctx: *mut hgi_ctx_t);
+    /// Accepts 0..=3 (hgi_path_t); every value runs the fused tile path, the others are kept for compatibility.
     pub fn hgi_ctx_set_path(ctx: *mut hgi_ctx_t, path: c_int) -> c_int;
     pub fn hgi_ctx_set_pipeline(ctx: *mut hgi_ctx_t, chunk_mb: u32, slots: u32) -> c_int;
     pub fn hgi_ctx_synchronize(ctx: *mut hgi_ctx_t) -> c_int;

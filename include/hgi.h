@@ -70,13 +70,13 @@ typedef enum {
     HGI_QLEVEL_HIGH = 3
 } hgi_quant_level_t;
 
-/* Which CUDA path a context uses.  All produce identical bytes. */
+/* Which CUDA path a context uses (hgi_ctx_set_path).  There is one: the other values are kept so that callers which
+   set them still work. */
 typedef enum {
-    HGI_PATH_TILE = 0,         /* default: fused multi-level tile kernels (register-prefetch SWAR kernel where eligible) */
-    HGI_PATH_PER_LEVEL = 1,    /* one kernel per level over HBM (north_star's literal shape) */
-    HGI_PATH_TILE_GENERIC = 2, /* fused tiles, always the generic (scalar, any alignment) kernel */
-    HGI_PATH_TILE_TMA = 3      /* accepted for compatibility: runs exactly what HGI_PATH_TILE runs (the TMA kernel it
-                                  once selected has been removed) */
+    HGI_PATH_TILE = 0,         /* fused multi-level tile kernels, every plane size and layout */
+    HGI_PATH_PER_LEVEL = 1,    /* accepted for compatibility: runs exactly what HGI_PATH_TILE runs */
+    HGI_PATH_TILE_GENERIC = 2, /* accepted for compatibility: runs exactly what HGI_PATH_TILE runs */
+    HGI_PATH_TILE_TMA = 3      /* accepted for compatibility: runs exactly what HGI_PATH_TILE runs */
 } hgi_path_t;
 
 #define HGI_MAX_LEVELS 31u
@@ -192,7 +192,7 @@ int hgi_histogram_dev(hgi_ctx_t *ctx, const uint8_t *d_grid, size_t n_per_image,
    every plane argument, all planes share the pitch).  A pitch that is a multiple of 16 with 16-byte-aligned bases
    puts any width on the 128-bit path: pad the rows of odd-width planes instead of packing them.  Input bytes in
    the padding are ignored; output bytes in the padding are unspecified.  pitch == width is hgi_encode_dev /
-   hgi_decode_dev.  Not available on HGI_PATH_PER_LEVEL (-> HGI_ERR_UNSUPPORTED). */
+   hgi_decode_dev. */
 int hgi_encode_dev_pitched(hgi_ctx_t *ctx, const uint8_t *d_images, uint32_t n_images, uint32_t width,
                            uint32_t height, uint32_t pitch, const hgi_params_t *params,
                            uint8_t *d_grids_out, uint8_t *d_recon_out /* nullable */,
@@ -227,8 +227,7 @@ int hgi_plan_region(uint32_t width, uint32_t height, uint32_t levels, uint32_t s
                     hgi_region_plan_t *plan_out);
 /* `n_images` grid planes (rows `pitch` bytes apart, as hgi_decode_dev_pitched) -> the region of each one's scaled
    image: d_out rows are `out_pitch` bytes apart (>= region width), planes out_pitch * region height apart, and no byte
-   outside the rectangles is written.  Enqueued on `stream` like every *_dev call.  Not on HGI_PATH_PER_LEVEL
-   (-> HGI_ERR_UNSUPPORTED). */
+   outside the rectangles is written.  Enqueued on `stream` like every *_dev call. */
 int hgi_decode_region_dev(hgi_ctx_t *ctx, const uint8_t *d_grids, uint32_t n_images, uint32_t width, uint32_t height,
                           uint32_t pitch, const hgi_params_t *params, uint32_t scale_log2, const hgi_rect_t *region,
                           uint8_t *d_out, uint32_t out_pitch, void *stream);
@@ -252,7 +251,7 @@ int hgi_plan_crop(uint32_t width, uint32_t height, uint32_t levels, uint32_t sca
    Enqueued on `stream`, no host synchronisation; once a first call has sized the scratch, a call of the same shapes
    allocates nothing and may be captured into a caller's CUDA graph (origins rewritten in place before each replay).
    HGI_ERR_INVALID_ARG: a crop of size 0 or larger than the scaled image, out_pitch < crop_width, NULL or misaligned
-   pointers (n_images > 0); HGI_ERR_UNSUPPORTED on HGI_PATH_PER_LEVEL. */
+   pointers (n_images > 0). */
 int hgi_decode_crops_dev(hgi_ctx_t *ctx, const uint8_t *d_grids, uint32_t n_images, uint32_t width, uint32_t height,
                          uint32_t pitch, const hgi_params_t *params, uint32_t scale_log2, uint32_t crop_width,
                          uint32_t crop_height, const int32_t *d_origins, uint8_t *d_out, uint32_t out_pitch,

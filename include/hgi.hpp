@@ -76,6 +76,7 @@ public:
     Context(const Context&) = delete;
     Context& operator=(const Context&) = delete;
     hgi_ctx_t* get() const { return ctx_; }
+    // every hgi_path_t value runs the fused tile path (the others are accepted for compatibility)
     void set_path(hgi_path_t path) { check(hgi_ctx_set_path(ctx_, path), "hgi_ctx_set_path"); }
     uint64_t kernel_launches() const { return hgi_ctx_kernel_launches(ctx_); }
     static std::shared_ptr<Context> shared(int device = 0)

@@ -42,6 +42,8 @@ class InterpolationType(enum.IntEnum):      # src/interpolator.rs:4-9 (serialisa
 
 _INTERP_LEFTTOP = 3
 _QUANT_NOOP, _QUANT_LINEAR = 0, 1
+# hgi_path_t: every value runs the fused tile path; PATH_PER_LEVEL, PATH_TILE_GENERIC and PATH_TILE_TMA are accepted
+# for compatibility
 PATH_TILE, PATH_PER_LEVEL, PATH_TILE_GENERIC, PATH_TILE_TMA = 0, 1, 2, 3
 
 

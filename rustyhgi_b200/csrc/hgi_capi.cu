@@ -58,7 +58,6 @@ struct Scratch {
     uint64_t gen = 0;    // bumped whenever one of the buffers moves: cached launch chains that point into them are stale
     DevBuf compact[4];   // ping-pong {recon, q} compact planes of the coarse passes
     DevBuf dec_in;       // decimated source of a coarse pass
-    DevBuf level_recon;  // per-level path: reconstruction planes when the caller gives none
     DevBuf region_in, region_out;   // scalable decode: the gathered window of the grid, and the decoded window
     // fork/join of the independent split launches of the quantizing encode (hgi_kernels.h PassArgs::side_stream)
     cudaStream_t side = nullptr;
@@ -80,7 +79,7 @@ struct StreamScratch {
 // once and replayed with one cudaGraphLaunch: what a caller with fixed buffers -- a frame loop, the band driver of
 // the pool -- pays per call on the host drops from one launch per kernel to one launch per call.
 struct ChainKey {
-    int mode, path, interp, quant_kind, quant_level;
+    int mode, interp, quant_kind, quant_level;
     const uint8_t* src;
     uint8_t *grid_out, *recon_out;
     uint32_t* hist;
@@ -89,7 +88,7 @@ struct ChainKey {
     uint64_t scratch_gen;
     bool operator==(const ChainKey& o) const
     {
-        return mode == o.mode && path == o.path && interp == o.interp && quant_kind == o.quant_kind &&
+        return mode == o.mode && interp == o.interp && quant_kind == o.quant_kind &&
                quant_level == o.quant_level && src == o.src && grid_out == o.grid_out && recon_out == o.recon_out &&
                hist == o.hist && n_images == o.n_images && w == o.w && h == o.h && pitch == o.pitch &&
                levels == o.levels && scratch == o.scratch && scratch_gen == o.scratch_gen;
@@ -117,7 +116,6 @@ constexpr size_t kMaxCallerStreams = 32;   // scratch sets kept for device-API c
 
 struct hgi_ctx {
     int device = 0;
-    int path = HGI_PATH_TILE;
     cudaStream_t stream = nullptr;
     cudaError_t last_err = cudaSuccess;
     uint64_t launches = 0;
@@ -212,8 +210,7 @@ void destroy_side(Scratch& sc)
 
 void free_scratch(Scratch& sc)
 {
-    free_bufs({&sc.compact[0], &sc.compact[1], &sc.compact[2], &sc.compact[3], &sc.dec_in, &sc.level_recon, &sc.region_in,
-               &sc.region_out});
+    free_bufs({&sc.compact[0], &sc.compact[1], &sc.compact[2], &sc.compact[3], &sc.dec_in, &sc.region_in, &sc.region_out});
     destroy_side(sc);
 }
 
@@ -385,7 +382,7 @@ int run_tile_path(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint3
     }
     const uint8_t* c_recon = nullptr;
     const uint8_t* c_q = nullptr;
-    uint32_t cw = 0, ch = 0, cpitch = 0;
+    uint32_t ch = 0, cpitch = 0;
     for (size_t i = 0; i < passes.size(); ++i) {
         const Pass& ps = passes[i];
         hgi::PassArgs a{};
@@ -398,13 +395,10 @@ int run_tile_path(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint3
         a.wD = ceil_shift(w, ps.d_log2);
         a.hD = ceil_shift(h, ps.d_log2);
         a.dpitch = align16(a.wD);
-        a.cw = cw;
         a.ch = ch;
         a.cpitch = cpitch;
         a.c_recon = c_recon;
         a.c_q = c_q;
-        a.tiles_x = (a.wD + hgi::kTileW - 1) / hgi::kTileW;
-        a.tiles_y = (a.hD + hgi::kTileH - 1) / hgi::kTileH;
         a.n_images = n_images;
         a.quant_error = qerr;
         if (ps.d_log2 == 0) {
@@ -424,61 +418,11 @@ int run_tile_path(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint3
             a.s_q = sc.compact[set + 1].p;
             a.dec_in = sc.dec_in.p;
         }
-        HGI_CUDA(ctx, hgi::launch_tile_pass(mode, prm->interp, a, st, ctx->path == HGI_PATH_TILE_GENERIC));
+        HGI_CUDA(ctx, hgi::launch_tile_pass(mode, prm->interp, a, st));
         c_recon = a.s_recon;
         c_q = a.s_q;
-        cw = a.wD;
         ch = a.hD;
         cpitch = a.dpitch;
-    }
-    return HGI_OK;
-}
-
-int run_level_path(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint32_t n_images, uint32_t w, uint32_t h,
-                   uint32_t levels, const hgi_params_t* prm, uint8_t* grid_out, uint8_t* recon_out,
-                   cudaStream_t st)
-{
-    const size_t plane = (size_t)w * h;
-    const uint32_t qerr = (mode == hgi::kModeEncode) ? hgi::level_error(prm->quant_kind, prm->quant_level) : 0u;
-    // images per sub-batch so that a private reconstruction scratch stays bounded
-    uint32_t per = n_images;
-    uint8_t* recon = recon_out;
-    if (mode == hgi::kModeEncode && recon == nullptr) {
-        const size_t budget = 1ull << 30;
-        per = (uint32_t)(budget / plane);
-        if (per < 1) per = 1;
-        if (per > n_images) per = n_images;
-        int rc = reserve(ctx, sc, sc.level_recon, (size_t)per * plane);
-        if (rc) return rc;
-        recon = sc.level_recon.p;
-    }
-    for (uint32_t first = 0; first < n_images; first += per) {
-        const uint32_t cnt = (n_images - first < per) ? n_images - first : per;
-        const uint8_t* s = src + (size_t)first * plane;
-        uint8_t* r = (recon == recon_out) ? recon + (size_t)first * plane : recon;
-        uint8_t* g = grid_out ? grid_out + (size_t)first * plane : nullptr;
-        if (mode == hgi::kModeEncode) {
-            // `mut input: GrayImage` by value (src/encoder.rs:39): the reconstruction starts as the image
-            HGI_CUDA(ctx, cudaMemcpyAsync(r, s, (size_t)cnt * plane, cudaMemcpyDeviceToDevice, st));
-            HGI_CUDA(ctx, hgi::launch_seed(mode, s, g, w, h, levels, cnt, st));
-        } else {
-            // GrayImage::new is zero-filled (src/decoder.rs:19); every byte is overwritten below, but
-            // keep the reference's initial state so partial lattices can never leak stale data
-            HGI_CUDA(ctx, cudaMemsetAsync(r, 0, (size_t)cnt * plane, st));
-            HGI_CUDA(ctx, hgi::launch_seed(mode, s, r, w, h, levels, cnt, st));
-        }
-        for (uint32_t level = 0; level < levels; ++level) {
-            hgi::LevelArgs a{};
-            a.grid_in = s;
-            a.grid_out = g;
-            a.recon = r;
-            a.w = w;
-            a.h = h;
-            a.step_log2 = levels - level;
-            a.n_images = cnt;
-            a.quant_error = qerr;
-            HGI_CUDA(ctx, hgi::launch_level(mode, prm->interp, a, st));
-        }
     }
     return HGI_OK;
 }
@@ -489,16 +433,11 @@ int run_dev(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint32_t n_
     if (n_images == 0 || (size_t)w * h == 0) return HGI_OK;
     const uint32_t levels = effective_levels(prm->levels, w, h);
     uint8_t* primary = (mode == hgi::kModeEncode) ? grid_out : recon_out;
-    const bool packed = (pitch == w);
     if (levels == 0) {
         // L = 0: grid == image (src/encoder.rs:26-37 copies every pixel, the level loop is empty)
         HGI_CUDA(ctx, cudaMemcpy2DAsync(primary, pitch, src, pitch, w, (size_t)h * n_images, cudaMemcpyDeviceToDevice, st));
         if (mode == hgi::kModeEncode && recon_out)
             HGI_CUDA(ctx, cudaMemcpy2DAsync(recon_out, pitch, src, pitch, w, (size_t)h * n_images, cudaMemcpyDeviceToDevice, st));
-    } else if (ctx->path == HGI_PATH_PER_LEVEL) {  // all other paths are tile variants
-        if (!packed) return HGI_ERR_UNSUPPORTED;    // the per-level kernels address packed planes only
-        int rc = run_level_path(ctx, sc, mode, src, n_images, w, h, levels, prm, grid_out, recon_out, st);
-        if (rc) return rc;
     } else {
         int rc = run_tile_path(ctx, sc, mode, src, n_images, w, h, pitch, levels, prm, grid_out, recon_out, st);
         if (rc) return rc;
@@ -525,7 +464,7 @@ int run_dev_cached(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint
                    cudaStream_t st)
 {
     const uint32_t levels = effective_levels(prm->levels, w, h);
-    const bool multi = levels > (uint32_t)hgi::kMaxPassLevels || ctx->path == HGI_PATH_PER_LEVEL;   // >= 3 launches
+    const bool multi = levels > (uint32_t)hgi::kMaxPassLevels;   // >= 3 launches
     auto plain = [&] {   // plain launches: the chain is not worth a graph, or its stream cannot be captured
         (void)cudaGetLastError();
         return run_dev(ctx, sc, mode, src, n_images, w, h, pitch, prm, grid_out, recon_out, hist, st);
@@ -534,7 +473,7 @@ int run_dev_cached(hgi_ctx* ctx, Scratch& sc, int mode, const uint8_t* src, uint
     if (!multi || !graphs_enabled() || st == cudaStreamLegacy || st == cudaStreamPerThread ||
         cudaStreamIsCapturing(st, &cap) != cudaSuccess || cap != cudaStreamCaptureStatusNone)
         return plain();
-    ChainKey key{mode, ctx->path, prm->interp, prm->quant_kind, prm->quant_level, src, grid_out, recon_out, hist,
+    ChainKey key{mode, prm->interp, prm->quant_kind, prm->quant_level, src, grid_out, recon_out, hist,
                  n_images, w, h, pitch, levels, &sc, sc.gen};
     ChainGraph* hit = nullptr;
     for (ChainGraph& g : ctx->chains)
@@ -762,10 +701,7 @@ int check_region(hgi_ctx* ctx, const hgi_params_t* prm, uint32_t w, uint32_t h, 
 {
     int rc = check_job(ctx, prm, false, w, h, n_images, pitch, {});
     if (rc < 0) return rc;   // an empty job is the region rules' to judge
-    rc = plan(w, h, prm->levels, k, region, pl, r);
-    if (rc) return rc;
-    if (ctx->path == HGI_PATH_PER_LEVEL) return HGI_ERR_UNSUPPORTED;   // the window decode is a tile path
-    return HGI_OK;
+    return plan(w, h, prm->levels, k, region, pl, r);
 }
 
 // Scalable decode of `n_images` planes: gather the window lattice (src + img * plane_stride + v * row_step + (u << k),
@@ -875,8 +811,8 @@ void hgi_ctx_destroy(hgi_ctx_t* ctx)
 
 int hgi_ctx_set_path(hgi_ctx_t* ctx, int path)
 {
+    // every path value runs the tile path (hgi.h): only the range is checked
     if (!ctx || path < HGI_PATH_TILE || path > HGI_PATH_TILE_TMA) return HGI_ERR_INVALID_ARG;
-    ctx->path = path;
     return HGI_OK;
 }
 

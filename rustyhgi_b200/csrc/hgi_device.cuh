@@ -3,7 +3,6 @@
 // Arithmetic restated from the reference (paths relative to the reference tree):
 //   prediction  src/interpolator.rs:43-54 (Crossed), :19-26 (LeftTop)
 //   quantizer   src/quantizator.rs:50-60 (Linear table), :27-29 (NoOp)
-//   fix-up      src/encoder.rs:56-60
 // Everything is u8 / small unsigned integer arithmetic; there is no floating point.
 #pragma once
 #include <cstdint>
@@ -37,23 +36,6 @@ __host__ __device__ __forceinline__ uint32_t quant_entry(uint32_t v, uint32_t er
 {
     const uint32_t scale = 2u * error + 1u;
     return (((v + error) / scale) * scale) & 0xFFu;
-}
-
-// One encoder step (src/encoder.rs:52-64).  Returns the stored symbol; *recon gets the value the
-// decoder will reconstruct.  `lut` may be null for the identity quantizer (NoOp / Lossless).
-template <bool IDENTITY>
-__device__ __forceinline__ uint32_t encode_point(uint32_t actual, uint32_t pred, const uint8_t* lut,
-                                                 uint32_t* recon)
-{
-    const uint32_t diff = (actual - pred) & 0xFFu;          // :53 wrapping_sub
-    uint32_t q = IDENTITY ? diff : (uint32_t)lut[diff];     // :54
-    if (!IDENTITY) {
-        const bool overflow = (pred + q) > 255u;            // :56
-        const bool expected = (pred + diff) > 255u;         // :57
-        if (overflow != expected) q = diff;                 // :58-60
-    }
-    *recon = (pred + q) & 0xFFu;                            // :63 wrapping_add
-    return q;
 }
 
 }  // namespace hgi

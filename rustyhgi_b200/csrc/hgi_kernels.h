@@ -9,9 +9,6 @@ namespace hgi {
 // ---- fused tile path ----------------------------------------------------------------------
 // One *pass* runs `nlev` (1..4) consecutive levels of the hierarchy for every tile of the
 // lattice {(x,y) : x,y multiples of D = 2^d_log2}; see DESIGN.md "Pass decomposition".
-constexpr int kTileW = 128;   // lattice points per tile row
-constexpr int kTileH = 64;    // lattice rows per tile
-constexpr int kTileThreads = 256;
 constexpr int kMaxPassLevels = 4;
 
 struct PassArgs {
@@ -28,11 +25,10 @@ struct PassArgs {
     uint32_t cpitch;         // bytes per row of c_recon / c_q
     uint32_t dpitch;         // D>1: bytes per row of s_recon / s_q / dec_in (16-byte multiple)
     uint32_t wD, hD;         // lattice size of this pass: ceil(w/D), ceil(h/D)
-    uint32_t cw, ch;         // size of the coarser pass's compact planes
+    uint32_t ch;             // rows of the coarser pass's compact planes
     uint32_t d_log2;         // log2(D)
     uint32_t nlev;           // levels fused in this pass (1..4); coarse step F = 2^nlev
-    uint32_t tiles_x, tiles_y;
-    uint32_t fast_tx, fast_itx, fast_ity;   // fast tile kernel: tiles per row, interior tile columns / rows (tile + halo inside the plane)
+    uint32_t fast_itx, fast_ity;            // interior tile columns / rows (tile + halo inside the plane)
     uint32_t fast_rcol;                     // 1: there is exactly one non-interior tile column and it is a whole tile wide
     uint32_t n_images;
     // fast kernel, quantizing encode, interior tiles: L2 prefetch of the tile at pf_src = src + distance (the same tile of a later
@@ -52,27 +48,14 @@ struct PassArgs {
     cudaEvent_t ev_fork, ev_join;
 };
 
-// Dispatch of one pass.  By default every pass of a plane up to 65535 tiles tall goes to the register-prefetch SWAR
-// kernel (hgi_tile_fast.cu), taller planes to the generic kernel (hgi_tile_kernels.cu); `generic` forces the generic
-// kernel, the independent formulation the tests cross-check against.
 // Kernels the calling thread's launch_* calls have launched and no context has been charged for yet: every launcher
 // adds one per kernel it launches, and the context whose work it was takes them (hgi_ctx_kernel_launches).
 uint64_t& launch_count();
 
-cudaError_t launch_tile_pass(int mode, int interp, const PassArgs& args, cudaStream_t stream, bool generic);
-cudaError_t launch_tile_pass_fast(int mode, int interp, const PassArgs& args, cudaStream_t stream);
+// One pass, on the SWAR tile kernel (hgi_tile_fast.cu).
+cudaError_t launch_tile_pass(int mode, int interp, const PassArgs& args, cudaStream_t stream);
 bool quant_swar_self_check();
 
-// ---- per-level path -----------------------------------------------------------------------
-struct LevelArgs {
-    const uint8_t* grid_in;  // decode: residual planes
-    uint8_t* grid_out;       // encode: residual planes
-    uint8_t* recon;          // reconstruction planes, updated in place (encode: starts as image)
-    uint32_t w, h;
-    uint32_t step_log2;      // coarse step of this level = 2^step_log2 (sub-step = step/2)
-    uint32_t n_images;
-    uint32_t quant_error;
-};
 // D>1 passes of the SWAR kernels: gather the pass's lattice {multiples of 2^d_log2} of `n_images` pitched planes into
 // dense planes (dpitch x hD each, zero padded), so that the pass itself runs on contiguous rows.
 cudaError_t launch_decimate(const uint8_t* src, uint32_t pitch, uint32_t h, uint32_t d_log2, uint32_t wD, uint32_t hD,
@@ -114,9 +97,6 @@ cudaError_t launch_region_gather(const uint8_t* src, uint64_t row_step, uint64_t
 cudaError_t launch_region_crop(const uint8_t* win, uint32_t wpitch, uint32_t wh, uint32_t cx, uint32_t cy, uint32_t rw,
                                uint32_t rh, uint32_t n_images, uint8_t* out, uint32_t out_pitch, cudaStream_t stream,
                                const CropOrigins& crops = CropOrigins{});
-cudaError_t launch_seed(int mode, const uint8_t* src, uint8_t* dst, uint32_t w, uint32_t h,
-                        uint32_t levels, uint32_t n_images, cudaStream_t stream);
-cudaError_t launch_level(int mode, int interp, const LevelArgs& args, cudaStream_t stream);
 
 // ---- reductions ---------------------------------------------------------------------------
 // `n_images` planes of `h` rows of `w` bytes, `pitch` bytes apart (pitch == w: one contiguous run of w * h bytes per

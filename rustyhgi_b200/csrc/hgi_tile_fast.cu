@@ -1,7 +1,6 @@
-// hgi_tile_fast.cu -- the fast fused HGI tile kernel (sm_100a), register-prefetch variant: the default for
-// every pass.  Same pass/tile/halo decomposition as hgi_tile_kernels.cu (the generic scalar kernel, now only
-// used for planes taller than 4 M rows and as a test cross-check), restructured so the work per pixel drops ~4x
-// (shared device code: hgi_tile_swar.cuh):
+// hgi_tile_fast.cu -- the fused HGI tile kernel (sm_100a), register-prefetch variant: it runs every pass of every
+// plane.  The pass/tile/halo decomposition is the one tests/tile_model.py states plainly, restructured so the work per
+// pixel is ~4x below a byte-wise formulation (shared device code: hgi_tile_swar.cuh):
 //
 //  * every level s in {2,4,8,16} of the tile lives in its own DENSE shared-memory plane P_s (lattice-s points
 //    only, one byte each), so each level is "the finest level of a half-size image": even rows read
@@ -451,7 +450,6 @@ inline void launch_one(void (*kernel)(PassArgs), dim3 nb, cudaStream_t stream, c
 template <int MODE, int INTERP, bool IDENTITY, bool EXTRA, int NLEV, bool ALIGNED>
 cudaError_t launch_fast_split(PassArgs& a, uint32_t tiles_x, uint32_t tiles_y, cudaStream_t stream)
 {
-    a.fast_tx = tiles_x;
     if (a.fast_itx == 0 || a.fast_ity == 0) a.fast_itx = a.fast_ity = 0;
     // the edge launches depend on nothing the interior launch writes: fork them onto the side stream when there is one
     const bool fork = a.fast_itx && a.side_stream && a.ev_fork && a.ev_join;
@@ -479,16 +477,14 @@ cudaError_t launch_fast_split(PassArgs& a, uint32_t tiles_x, uint32_t tiles_y, c
     return cudaGetLastError();
 }
 
+// One grid of a pass: `a` holds the slice's planes -- its images, or one image from the slice's first tile row down, so
+// that a.h still covers the halo rows below the slice -- and `rows` the slice's tile rows (gridDim.y).
 template <int MODE, int INTERP, int NLEV, bool ALIGNED>
-cudaError_t launch_fast_n(const PassArgs& args, cudaStream_t stream)
+cudaError_t launch_fast_slice(PassArgs a, uint32_t tiles_x, uint32_t rows, cudaStream_t stream)
 {
-    const uint32_t tiles_x = (args.w + TW - 1) / TW, tiles_y = (args.h + TH - 1) / TH;
-    if (tiles_x == 0 || tiles_y == 0 || args.n_images == 0) return cudaSuccess;
-    if (tiles_y > 65535u) return cudaErrorInvalidConfiguration;
-    const size_t plane = (size_t)args.pitch * args.h;
     // interior tile columns / rows (tile + halo inside the plane), for the bodies without in-image predicates
-    const uint32_t itx = args.w >= (uint32_t)(FMAX + 1) ? min(tiles_x, (args.w - (FMAX + 1)) / TW) : 0u;
-    const uint32_t ity = args.h >= (uint32_t)(FMAX + 1) ? min(tiles_y, (args.h - (FMAX + 1)) / TH) : 0u;
+    const uint32_t itx = a.w >= (uint32_t)(FMAX + 1) ? min(tiles_x, (a.w - (FMAX + 1)) / TW) : 0u;
+    const uint32_t ity = a.h >= (uint32_t)(FMAX + 1) ? min(rows, (a.h - (FMAX + 1)) / TH) : 0u;
     // L2 prefetch distance of the interior tiles of the quantizing encode, in residencies (148 SMs x 10 CTAs): that
     // kernel is bound by its instruction stream, so the DRAM latency of a tile's first loads is the one stall it cannot
     // cover with other work; fetching the tile into L2 about one residency earlier takes it away (-2..3 %, A/B sweep:
@@ -496,51 +492,72 @@ cudaError_t launch_fast_n(const PassArgs& args, cudaStream_t stream)
     // kernels lose with any distance (+20 % at k = 2) and do not carry the code.  HGI_B200_PREFETCH=<k> overrides, 0 = off.
     static const double pf_k = [] { const char* e = getenv("HGI_B200_PREFETCH"); return e ? atof(e) : 1.0; }();
     const double pf_tiles = pf_k * 1480.0;
-    const uint64_t tiles_img = (uint64_t)tiles_x * tiles_y;
+    const uint64_t tiles_img = (uint64_t)tiles_x * rows;
     uint32_t pf_images = 0, pf_rows = 0;
     if (pf_tiles > 0.0) {
         if ((double)tiles_img <= pf_tiles) pf_images = (uint32_t)((pf_tiles + (double)tiles_img - 1.0) / (double)tiles_img);
         else pf_rows = (uint32_t)((pf_tiles + (double)tiles_x - 1.0) / (double)tiles_x);
     }
-    for (uint32_t first = 0; first < args.n_images; first += 65535u) {   // gridDim.z limit
-        PassArgs a = args;
-        a.n_images = args.n_images - first < 65535u ? args.n_images - first : 65535u;
-        a.src = args.src + (size_t)first * plane;
-        if (args.grid_out) a.grid_out = args.grid_out + (size_t)first * plane;
-        if (args.recon_out) a.recon_out = args.recon_out + (size_t)first * plane;
-        if (args.c_recon) a.c_recon = args.c_recon + (size_t)first * args.cpitch * args.ch;
-        if (args.c_q) a.c_q = args.c_q + (size_t)first * args.cpitch * args.ch;
-        a.fast_itx = itx;
-        a.fast_ity = ity;
-        a.fast_rcol = (itx + 1 == tiles_x && a.w == tiles_x * (uint32_t)TW) ? 1u : 0u;   // ONE right column, exactly TW wide
-        const bool extra = (a.recon_out != nullptr);
-        // a large slice of the quantizing encode runs as split launches (interior / edges); only their interior-only
-        // CTAs prefetch.  Small slices: one launch, less latency
-        const bool split = MODE == kModeEncode && a.quant_error != 0 && ALIGNED && NLEV == 4 &&
-                           tiles_img * a.n_images >= split_min_tiles();
-        // prefetch bounds against this slice's grid: planes [0, n - pf_images) / interior tile rows [0, ity - pf_rows)
-        const uint32_t zi = split ? pf_images : 0u, zr = split ? pf_rows : 0u;
-        a.pf_zlim = zi ? (a.n_images > zi ? a.n_images - zi : 0u) : (zr ? a.n_images : 0u);
-        a.pf_ylim = zr ? (ity > zr ? ity - zr : 0u) : 0xFFFFFFFFu;
-        a.pf_src = a.src + ((uint64_t)zi * args.h + (uint64_t)zr * TH) * args.pitch;
-        const dim3 nb(tiles_x, tiles_y, a.n_images);
-        if (MODE == kModeDecode) {
-            launch_one(hgi_tile_fast_kernel<kModeDecode, INTERP, true, false, NLEV, ALIGNED>, nb, stream, a);
-        } else if (a.quant_error == 0) {
-            launch_one(!extra ? hgi_tile_fast_kernel<kModeEncode, INTERP, true, false, NLEV, ALIGNED>
-                              : hgi_tile_fast_kernel<kModeEncode, INTERP, true, true, NLEV, ALIGNED>, nb, stream, a);
-        } else if (split) {
-            if constexpr (MODE == kModeEncode && ALIGNED && NLEV == 4) {
-                const cudaError_t es = extra ? launch_fast_split<kModeEncode, INTERP, false, true, NLEV, ALIGNED>(a, tiles_x, tiles_y, stream)
-                                             : launch_fast_split<kModeEncode, INTERP, false, false, NLEV, ALIGNED>(a, tiles_x, tiles_y, stream);
-                if (es != cudaSuccess) return es;
-            }
-        } else {
-            launch_one(!extra ? hgi_tile_fast_kernel<kModeEncode, INTERP, false, false, NLEV, ALIGNED>
-                              : hgi_tile_fast_kernel<kModeEncode, INTERP, false, true, NLEV, ALIGNED>, nb, stream, a);
+    a.fast_itx = itx;
+    a.fast_ity = ity;
+    a.fast_rcol = (itx + 1 == tiles_x && a.w == tiles_x * (uint32_t)TW) ? 1u : 0u;   // ONE right column, exactly TW wide
+    const bool extra = (a.recon_out != nullptr);
+    // a large slice of the quantizing encode runs as split launches (interior / edges); only their interior-only
+    // CTAs prefetch.  Small slices: one launch, less latency
+    const bool split = MODE == kModeEncode && a.quant_error != 0 && ALIGNED && NLEV == 4 &&
+                       tiles_img * a.n_images >= split_min_tiles();
+    // prefetch bounds against this slice's grid: planes [0, n - pf_images) / interior tile rows [0, ity - pf_rows)
+    const uint32_t zi = split ? pf_images : 0u, zr = split ? pf_rows : 0u;
+    a.pf_zlim = zi ? (a.n_images > zi ? a.n_images - zi : 0u) : (zr ? a.n_images : 0u);
+    a.pf_ylim = zr ? (ity > zr ? ity - zr : 0u) : 0xFFFFFFFFu;
+    a.pf_src = a.src + ((uint64_t)zi * a.h + (uint64_t)zr * TH) * a.pitch;
+    const dim3 nb(tiles_x, rows, a.n_images);
+    if (MODE == kModeDecode) {
+        launch_one(hgi_tile_fast_kernel<kModeDecode, INTERP, true, false, NLEV, ALIGNED>, nb, stream, a);
+    } else if (a.quant_error == 0) {
+        launch_one(!extra ? hgi_tile_fast_kernel<kModeEncode, INTERP, true, false, NLEV, ALIGNED>
+                          : hgi_tile_fast_kernel<kModeEncode, INTERP, true, true, NLEV, ALIGNED>, nb, stream, a);
+    } else if (split) {
+        if constexpr (MODE == kModeEncode && ALIGNED && NLEV == 4) {
+            const cudaError_t es = extra ? launch_fast_split<kModeEncode, INTERP, false, true, NLEV, ALIGNED>(a, tiles_x, rows, stream)
+                                         : launch_fast_split<kModeEncode, INTERP, false, false, NLEV, ALIGNED>(a, tiles_x, rows, stream);
+            if (es != cudaSuccess) return es;
         }
-        const cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) return e;
+    } else {
+        launch_one(!extra ? hgi_tile_fast_kernel<kModeEncode, INTERP, false, false, NLEV, ALIGNED>
+                          : hgi_tile_fast_kernel<kModeEncode, INTERP, false, true, NLEV, ALIGNED>, nb, stream, a);
+    }
+    return cudaGetLastError();
+}
+
+// gridDim.y and gridDim.z hold at most 65535 tile rows and images: a pass runs in slices of up to 65535 whole images or,
+// for a plane of more than 65535 tile rows, one image at a time in bands of up to 65535 tile rows (the kernel steps
+// from image to image by h * pitch, so a band must be the only image of its grid).
+template <int MODE, int INTERP, int NLEV, bool ALIGNED>
+cudaError_t launch_fast_n(const PassArgs& args, cudaStream_t stream)
+{
+    const uint32_t tiles_x = (args.w + TW - 1) / TW, tiles_y = (args.h + TH - 1) / TH;
+    if (tiles_x == 0 || tiles_y == 0 || args.n_images == 0) return cudaSuccess;
+    const size_t plane = (size_t)args.pitch * args.h, cplane = (size_t)args.cpitch * args.ch;
+    const uint32_t per = tiles_y <= 65535u ? 65535u : 1u;
+    for (uint32_t first = 0; first < args.n_images; first += per) {
+        for (uint32_t ty0 = 0; ty0 < tiles_y; ty0 += 65535u) {
+            const size_t y0 = (size_t)ty0 * TH, off = (size_t)first * plane + y0 * args.pitch;
+            const size_t coff = (size_t)first * cplane + (y0 >> NLEV) * args.cpitch;   // y0 is a multiple of 2^NLEV
+            PassArgs a = args;
+            a.n_images = args.n_images - first < per ? args.n_images - first : per;
+            a.h = args.h - (uint32_t)y0;
+            a.src = args.src + off;
+            if (args.grid_out) a.grid_out = args.grid_out + off;
+            if (args.recon_out) a.recon_out = args.recon_out + off;
+            if (args.c_recon) {
+                a.c_recon = args.c_recon + coff;
+                a.ch = args.ch - (uint32_t)(y0 >> NLEV);
+            }
+            if (args.c_q) a.c_q = args.c_q + coff;
+            const cudaError_t e = launch_fast_slice<MODE, INTERP, NLEV, ALIGNED>(a, tiles_x, min(65535u, tiles_y - ty0), stream);
+            if (e != cudaSuccess) return e;
+        }
     }
     return cudaSuccess;
 }
@@ -627,19 +644,27 @@ cudaError_t launch_decimate(const uint8_t* src, uint32_t pitch, uint32_t h, uint
                             uint32_t dpitch, uint32_t n_images, uint8_t* dst, cudaStream_t stream)
 {
     if (wD == 0 || hD == 0 || n_images == 0) return cudaSuccess;
-    if (hD > 65535u) return cudaErrorInvalidConfiguration;
     const uint32_t words = dpitch / 4, bx = words < 256u ? ((words + 31u) / 32u) * 32u : 256u;
+    // slices of up to 65535 images x 65535 rows (gridDim.z / gridDim.y); the kernel uses h and hD as plane strides only
     for (uint32_t first = 0; first < n_images; first += 65535u) {
         const uint32_t cnt = n_images - first < 65535u ? n_images - first : 65535u;
-        const dim3 nb((words + bx - 1) / bx, hD, cnt);
-        hgi_decimate_kernel<<<nb, bx, 0, stream>>>(src + (size_t)first * pitch * h, pitch, h, d_log2, wD, hD, dpitch,
-                                                   dst + (size_t)first * dpitch * hD);
-        ++launch_count();
+        for (uint32_t y0 = 0; y0 < hD; y0 += 65535u) {
+            const dim3 nb((words + bx - 1) / bx, min(65535u, hD - y0), cnt);
+            hgi_decimate_kernel<<<nb, bx, 0, stream>>>(src + ((size_t)first * h + ((size_t)y0 << d_log2)) * pitch, pitch, h,
+                                                       d_log2, wD, hD, dpitch, dst + ((size_t)first * hD + y0) * dpitch);
+            ++launch_count();
+        }
     }
     return cudaGetLastError();
 }
 
-cudaError_t launch_tile_pass_fast(int mode, int interp, const PassArgs& a, cudaStream_t stream)
+uint64_t& launch_count()
+{
+    static thread_local uint64_t n = 0;
+    return n;
+}
+
+cudaError_t launch_tile_pass(int mode, int interp, const PassArgs& a, cudaStream_t stream)
 {
     if (mode == kModeEncode)
         return interp == kInterpLeftTop ? launch_fast_t<kModeEncode, kInterpLeftTop>(a, stream)

@@ -1,5 +1,5 @@
 """Batched crops on the B200 (-m gpu): hgi_decode_crops_dev against the oracle's full decode, decimated by 2^k and
-sliced at each plane's own origin -- golden planes at every scale on both tile paths and interpolators, 1080p frames
+sliced at each plane's own origin -- golden planes at every scale with both interpolators, 1080p frames
 with random crops, padded rows, clamped origins, two streams, a caller's CUDA graph with origins rewritten in place,
 more than 65 535 planes, launch counts and every error code."""
 import ctypes
@@ -12,7 +12,7 @@ from conftest import get_plane, photo_like
 from oracle import c as oc
 
 pytestmark = pytest.mark.gpu
-PATHS = {"tile": hgi.PATH_TILE, "generic": hgi.PATH_TILE_GENERIC}
+PATHS = {"tile": hgi.PATH_TILE}
 INTERPS = {"crossed": (hgi.Crossed, oc.INTERP_CROSSED), "lefttop": (hgi.LeftTop, oc.INTERP_LEFTTOP)}
 
 
@@ -275,8 +275,22 @@ def test_error_codes():
     assert dev(ctx_h=None) == -1
     assert dev(interp=1) == -8 and dev(interp=2) == -8                 # Line / Previous
     assert dev(interp=7) == -1
+    # every path value runs the tile path: crops on a PATH_PER_LEVEL context are the oracle's
+    imgs = np.stack([photo_like(48, 64, 9 + i) for i in range(2)])
+    grids = oc.encode_batch(imgs, 4, qlevel=oc.MEDIUM)
+    fulls = oc.decode_batch(grids, 4)
+    gg = torch.from_numpy(grids).cuda()
+    xy = np.array([[3, 5], [40, 60]], np.int32)          # the second origin is clamped
+    d_xy = dev_origins(xy)
     per_level = hgi.Context(0, path=hgi.PATH_PER_LEVEL)
-    assert dev(ctx_h=per_level._h) == -8 and dev(5, 5, 2, ctx_h=per_level._h) == -8
+    for cw, ch, k in ((8, 8, 0), (5, 5, 2)):
+        ws, hs = scaled_size(48, 64, k)
+        clamped = np.minimum(xy, [ws - cw, hs - ch])
+        o.fill_(0x5A)
+        assert dev(cw, ch, k, ctx_h=per_level._h, grids=gg.data_ptr(), origins=d_xy.data_ptr()) == 0
+        torch.cuda.synchronize()
+        got = o.cpu().numpy().reshape(-1)[:2 * 48 * ch].reshape(2, ch, 48)[:, :, :cw]
+        assert np.array_equal(got, want_crops(fulls, k, clamped, cw, ch)), (cw, ch, k)
     per_level.close()
     # n == 0 launches nothing
     before = ctx.kernel_launches

@@ -138,14 +138,14 @@ def test_status_codes(env):
     case("region_dev: region outside, no images", L.hgi_decode_region_dev(ctx, None, 0, W, H, W, prm(), 0, bad, None, 64, None), INVALID)
     case("region_u8: region outside", L.hgi_decode_region_u8(ctx, hb, W, H, prm(), 0, bad, hb), INVALID)
     case("region_dev: scale 32", L.hgi_decode_region_dev(ctx, db, 1, W, H, W, prm(), 32, None, do, 64, None), INVALID)
-    for k, path in ((0, hgi.PATH_PER_LEVEL), (1, hgi.PATH_PER_LEVEL)):
-        pl = ctxs[path]._h
-        case(("per-level region", k), L.hgi_decode_region_dev(pl, db, 1, W, H, W, prm(), k, rect, do, 64, None), UNSUPPORTED)
-        case(("per-level region u8", k), L.hgi_decode_region_u8(pl, hb, W, H, prm(), k, rect, hb), UNSUPPORTED)
+    # every path value runs the tile path, which takes regions and padded rows
     pl = ctxs[hgi.PATH_PER_LEVEL]._h
-    case("per-level pitched encode", L.hgi_encode_dev_pitched(pl, db, 1, W, H, W + 16, prm(), do, None, None, None), UNSUPPORTED)
-    case("per-level pitched decode", L.hgi_decode_dev_pitched(pl, db, 1, W, H, W + 16, prm(), do, None), UNSUPPORTED)
-    case("per-level packed encode", L.hgi_encode_dev_pitched(pl, db, 1, W, H, W, prm(), do, None, None, None), 0)
+    for k in (0, 1):
+        case(("path 1 region", k), L.hgi_decode_region_dev(pl, db, 1, W, H, W, prm(), k, rect, do, 64, None), 0)
+        case(("path 1 region u8", k), L.hgi_decode_region_u8(pl, hb, W, H, prm(), k, rect, hout.ctypes.data), 0)
+    case("path 1 pitched encode", L.hgi_encode_dev_pitched(pl, db, 1, W, H, W + 16, prm(), do, None, None, None), 0)
+    case("path 1 pitched decode", L.hgi_decode_dev_pitched(pl, db, 1, W, H, W + 16, prm(), do, None), 0)
+    case("path 1 packed encode", L.hgi_encode_dev_pitched(pl, db, 1, W, H, W, prm(), do, None, None, None), 0)
     # histograms, reductions, colour conversion
     keep = [np.zeros(256, np.uint64), np.zeros(4 * 288, np.uint32)] + [np.zeros(1, np.uint64) for _ in range(3)]
     hist64, rle_out, *mp = [a.ctypes.data for a in keep]
@@ -264,9 +264,10 @@ def test_launch_counts(env):
         ("region_dev, scale 4", [ctx], lambda: L.hgi_decode_region_dev(ctx, db, N, W, H, W, prm(), 4, None, do, 4, None), 2),
         ("region_dev, whole plane", [ctx], lambda: L.hgi_decode_region_dev(ctx, db, N, W, H, W, prm(), 0, None, do, W, None), 1),
         ("region_u8, scale 1", [ctx], lambda: L.hgi_decode_region_u8(ctx, hb, W, H, prm(), 1, None, ho), 3),
-        ("per-level encode_u8", [plv], lambda: L.hgi_encode_u8(plv, hb, W, H, prm(), ho, None), 5),
-        ("per-level decode_batch_u8", [plv], lambda: L.hgi_decode_batch_u8(plv, hb, N, W, H, prm(), ho), 5),
-        ("generic encode_u8 L6", [gen], lambda: L.hgi_encode_u8(gen, hb, W, H, prm(6), ho, None), 2),
+        # paths 1 and 2 run what path 0 runs
+        ("path 1 encode_u8", [plv], lambda: L.hgi_encode_u8(plv, hb, W, H, prm(), ho, None), 1),
+        ("path 1 decode_batch_u8", [plv], lambda: L.hgi_decode_batch_u8(plv, hb, N, W, H, prm(), ho), 1),
+        ("path 2 encode_u8 L6", [gen], lambda: L.hgi_encode_u8(gen, hb, W, H, prm(6), ho, None), 3),
         ("pool encode_batch_u8 + hist", members, lambda: L.hgi_pool_encode_batch_u8(pool._h, hb, N, W, H, prm(), ho, hh), 2),
         ("pool decode_batch_u8", members, lambda: L.hgi_pool_decode_batch_u8(pool._h, hb, N, W, H, prm(), ho), 1),
         ("pool encode_plane_u8", members, lambda: L.hgi_pool_encode_plane_u8(pool._h, hb, W, H, prm(), ho), 1),
@@ -280,7 +281,7 @@ def test_launch_counts(env):
         torch.cuda.synchronize()
         want[tag] = tuple(n for _ in cs)
     # launch chains of the device API: run plainly, then captured, then replayed -- each call counts its kernels once
-    for tag, c, lv, n in (("encode_dev L6 + hist", ctx, 6, 4), ("per-level encode_dev + hist", plv, 4, 6)):
+    for tag, c, lv, n in (("encode_dev L6 + hist", ctx, 6, 4), ("path 1 encode_dev L6 + hist", plv, 6, 4)):
         fn = (lambda c=c, lv=lv: L.hgi_encode_dev(c, db, N, W, H, prm(lv), do, None, dh, None))
         got[tag] = tuple(_delta(L, [c], fn) for _ in range(3))
         want[tag] = (((n,), (0,)), ((n,), (1,)), ((n,), (1,)))

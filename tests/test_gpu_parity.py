@@ -1,8 +1,8 @@
 """Parity of the CUDA path (through the C ABI) with the oracle -- runs on the GPU box (-m gpu).
 
-Bit-exact on grid bytes, reconstruction and decoded pixels for every golden config, both CUDA
-paths (fused tiles / per level), both interpolators, all quantizers, ragged and degenerate sizes,
-batches, the device-pointer API, histograms and the `hgi test` metrics.  Nothing here reads
+Bit-exact on grid bytes, reconstruction and decoded pixels for every golden config, both
+interpolators, all quantizers, ragged and degenerate sizes, batches, the device-pointer API, histograms
+and the `hgi test` metrics; every hgi_path_t value runs the same kernels.  Nothing here reads
 /root/reference."""
 import ctypes
 import io
@@ -21,6 +21,8 @@ Q = hgi.QuantizationLevel
 
 @pytest.fixture(scope="module")
 def ctxs():
+    # one context per hgi_path_t value: each runs the tile path, and the tests that take a path pin that it gives the
+    # oracle's bytes whichever value a caller has set
     tile = hgi.Context(0, hgi.PATH_TILE)
     lvl = hgi.Context(0, hgi.PATH_PER_LEVEL)
     gen = hgi.Context(0, hgi.PATH_TILE_GENERIC)
@@ -224,10 +226,11 @@ def test_device_api_misaligned_bases_and_odd_widths(ctxs):
                 assert bool((t[:off] == fill).all()) and bool((t[off + size:] == fill).all())
 
 
-@pytest.mark.parametrize("path", ["tile", "tma"])
+@pytest.mark.parametrize("path", ["tile", "level", "generic", "tma"])
 def test_random_cases(ctxs, path):
     """Seeded random sweep over sizes (aligned and ragged), levels, quantizers, interpolators and image
-    statistics: every byte of grid, reconstruction and decoded image must equal the oracle."""
+    statistics: every byte of grid, reconstruction and decoded image must equal the oracle, on every hgi_path_t value,
+    with as many kernels as HGI_PATH_TILE launches for the same calls."""
     rng = np.random.default_rng(20261018)
     kinds = ("noise", "smooth", "const", "extremes", "ramp")
     for case in range(70):
@@ -248,7 +251,14 @@ def test_random_cases(ctxs, path):
         else:
             yy, xx = np.mgrid[0:h, 0:w]
             img = ((xx * 5 + yy * 3) & 255).astype(np.uint8)
-        check_case(ctxs[path], img, levels, q, interp=interp)
+        ctx, ref = ctxs[path], ctxs["tile"]
+        launches = ctx.kernel_launches
+        check_case(ctx, img, levels, q, interp=interp)
+        launches = ctx.kernel_launches - launches
+        if ctx is not ref:
+            want = ref.kernel_launches
+            check_case(ref, img, levels, q, interp=interp)
+            assert launches == ref.kernel_launches - want, (case, w, h, levels)
 
 
 def test_more_images_than_grid_z(ctxs):

@@ -13,7 +13,7 @@ from oracle import c as oc
 from rustyhgi_b200 import cli
 
 pytestmark = pytest.mark.gpu
-PATHS = {"tile": hgi.PATH_TILE, "generic": hgi.PATH_TILE_GENERIC}
+PATHS = {"tile": hgi.PATH_TILE}
 INTERPS = {"crossed": (hgi.Crossed, oc.INTERP_CROSSED), "lefttop": (hgi.LeftTop, oc.INTERP_LEFTTOP)}
 
 
@@ -212,8 +212,18 @@ def test_error_codes():
     assert dev(n=0, grids=None, out=None) == 0                          # nothing to do
     assert dev(interp=1) == -8 and dev(interp=2) == -8 and host(interp=1) == -8   # Line / Previous
     assert dev(interp=7) == -1
+    # every path value runs the tile path: regions on a PATH_PER_LEVEL context are the oracle's
+    img = photo_like(48, 64, 9)
+    grid = oc.encode(img, 4, qlevel=oc.MEDIUM)
+    full = oc.decode(grid, 4)
+    gg = torch.from_numpy(grid).cuda()
     per_level = hgi.Context(0, path=hgi.PATH_PER_LEVEL)
-    assert dev(ctx_h=per_level._h) == -8 and dev((0, 0, 5, 5), 2, ctx_h=per_level._h) == -8
+    for region, k in ((None, 0), ((0, 0, 5, 5), 2), ((3, 7, 9, 5), 1)):
+        o.fill_(0x5A)
+        assert dev(region, k, ctx_h=per_level._h, grids=gg.data_ptr()) == 0
+        torch.cuda.synchronize()
+        want = cut(full, k, region)
+        assert np.array_equal(o.cpu().numpy()[:want.shape[0], :want.shape[1]], want), (region, k)
     per_level.close()
     with pytest.raises(hgi.HgiError):
         hgi.Decoder(hgi.Crossed, ctx=ctx).decode_region_device(4, g, region=(40, 0, 9, 1))

@@ -59,16 +59,6 @@ def test_pitched_planes_any_width(path):
     c.close()
 
 
-def test_pitched_is_rejected_where_it_has_no_kernel():
-    import torch
-    c = hgi.Context(0, hgi.PATH_PER_LEVEL)
-    buf = torch.zeros((1, 32, 48), dtype=torch.uint8, device="cuda")
-    with pytest.raises(hgi.HgiError) as e:
-        hgi.Encoder(hgi.Crossed, hgi.Linear(Q.Low), 3, ctx=c).encode_device(buf[:, :, :40])
-    assert e.value.status == -8
-    c.close()
-
-
 def test_deep_hierarchies_take_the_decimated_coarse_passes(ctx):
     """levels 5..12 on planes large enough for two and three passes: the coarse passes run on the gathered lattice."""
     rng = np.random.default_rng(8)

@@ -55,6 +55,14 @@ def test_small_tiles_many_passes():
     (("enc", 20, 160, 96, True, 0, 3), {}, 0),                     # L = 0 is a copy
     (("enc", 20, 160, 96, True, 0, 3), {"hist": True}, 1),
     (("enc", 20, 0, 96, True, 4, 3), {"hist": True}, 0),
+    # tall planes: the L5 coarse pass of 1048577 rows decimates 65537 lattice rows in two launches, 1025 tile rows
+    (("dec", 0, 16, 1048577, True, 5, 1), {}, 2 + 1 + 1),
+    # 65537 tile rows: per image a band of 65535 (no interior column: the bottom-row launch) and one of 2
+    (("enc", 20, 16, 4194305, True, 4, 2), {"hist": True}, 2 * (1 + 1) + 1),
+    (("enc", 20, 160, 4194305, True, 4, 1), {}, 2 + 1),           # band 0: interior + right column, band 1: 4 tiles, one launch
+    # 131073 tile rows, three bands; the coarse pass decimates 524290 lattice rows in nine launches
+    (("enc", 20, 16, 8388625, True, 8, 1), {}, 9 + 1 + 3),
+    (("enc", 20, 160, 8388625, True, 4, 2), {}, 2 * (2 + 2 + 1)),
 ])
 def test_expected_launches(args, kw, want):
     """The plain statement of the launch dispatch (tile_model.expected_launches) on hand-worked shapes."""

@@ -1,5 +1,5 @@
 """Executable model of the fused tile-pass decomposition used by the CUDA library
-(rustyhgi_b200/csrc/hgi_tile_kernels.cu + plan_passes in hgi_capi.cu).
+(the tile kernel of rustyhgi_b200/csrc/hgi_tile_fast.cu + plan_passes in hgi_capi.cu), stated byte by byte.
 
 Test infrastructure: it mirrors, tile by tile, *which* bytes a CTA stages, which coarse values it
 takes from the previous pass, which cells/points it processes per level (the `need_limit`
@@ -32,34 +32,40 @@ def plan_passes(levels):
 
 
 SPLIT_MIN_TILES = 4 * 1480      # split_min_tiles() in hgi_tile_fast.cu (HGI_B200_SPLIT_MIN overrides it)
-MAX_GRID_Z = 65535               # images per launch (gridDim.z)
+MAX_GRID = 65535                 # images (gridDim.z) and rows (gridDim.y) per launch
 
 
 def expected_launches(mode, qerr, w, h, pitch_aligned, levels, n, split_min=SPLIT_MIN_TILES, hist=False):
     """Kernels one device-API call of the tile path launches (hgi_ctx_kernel_launches), stated plainly: per pass of
-    plan_passes(L), one decimate launch per 65535-image chunk for a coarse pass, then per chunk either one launch or,
-    for a split quantizing encode, the interior / right-column / bottom-row launches that have tiles; plus one for the
-    histogram.  `mode` is "enc" or "dec", `qerr` the quantizer's error (0: Lossless / NoOp), `pitch_aligned` whether
-    the fine pass runs the 128-bit instantiation (16-byte rows and bases; coarse passes always do)."""
+    plan_passes(L), for a coarse pass one decimate launch per 65535 images x 65535 lattice rows; then per slice -- up to
+    65535 whole images, or, in a plane of more than 65535 tile rows, one image's band of up to 65535 tile rows -- either
+    one launch or, for a split quantizing encode, the interior / right-column / bottom-row launches that have tiles;
+    plus one for the histogram.  `mode` is "enc" or "dec", `qerr` the quantizer's error (0: Lossless / NoOp),
+    `pitch_aligned` whether the fine pass runs the 128-bit instantiation (16-byte rows and bases; coarse passes always
+    do)."""
     if n == 0 or w * h == 0:
         return 0
     total = 1 if hist else 0
-    chunks = [min(MAX_GRID_Z, n - first) for first in range(0, n, MAX_GRID_Z)]
+    chunks = [min(MAX_GRID, n - first) for first in range(0, n, MAX_GRID)]
     for (d, nlev) in plan_passes(effective_levels(levels, w, h)):
         wD, hD = -(-w >> d), -(-h >> d)
         tx, ty = -(-wD // TW), -(-hD // TH)
         if d > 0:
-            total += len(chunks)
-        for cnt in chunks:
-            split = mode == "enc" and qerr != 0 and (pitch_aligned or d > 0) and nlev == 4 and tx * ty * cnt >= split_min
+            total += len(chunks) * -(-hD // MAX_GRID)
+        if ty <= MAX_GRID:   # (images, tile rows, rows from the slice's first row to the bottom of the plane)
+            slices = [(cnt, ty, hD) for cnt in chunks]
+        else:
+            slices = [(1, min(MAX_GRID, ty - t0), hD - t0 * TH) for _ in range(n) for t0 in range(0, ty, MAX_GRID)]
+        for cnt, rows, hr in slices:
+            split = mode == "enc" and qerr != 0 and (pitch_aligned or d > 0) and nlev == 4 and tx * rows * cnt >= split_min
             if not split:
                 total += 1
                 continue
             itx = min(tx, (wD - (FMAX + 1)) // TW) if wD >= FMAX + 1 else 0
-            ity = min(ty, (hD - (FMAX + 1)) // TH) if hD >= FMAX + 1 else 0
+            ity = min(rows, (hr - (FMAX + 1)) // TH) if hr >= FMAX + 1 else 0
             if itx == 0 or ity == 0:
                 itx = ity = 0
-            total += (itx > 0) + (tx - itx > 0 and ity > 0) + (ty - ity > 0)
+            total += (itx > 0) + (tx - itx > 0 and ity > 0) + (rows - ity > 0)
     return total
 
 

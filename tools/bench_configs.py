@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Times every BASELINE.json config on one B200 (device-resident planes, CUDA events, criterion-style
-25 samples after warm-up: median and best) for the three CUDA paths, next to the single-thread CPU
+25 samples after warm-up: median and best) on the tile path, next to the single-thread CPU
 oracle.  Prints a markdown table; `bench.py` remains the contract benchmark (config 5).
 
     python tools/bench_configs.py [--samples 25] > profiles/rNN_configs.md
@@ -61,8 +61,7 @@ def main():
         ("C4 synthetic 16384x16384", ((x[None, :] * x[:, None]) & 255).to(torch.uint8).contiguous(), 8, [2]),
     ]
     qn = ["Lossless", "Low", "Medium", "High"]
-    ctxs = {"fast tile": hgi.Context(0, hgi.PATH_TILE), "generic tile": hgi.Context(0, hgi.PATH_TILE_GENERIC),
-            "per level": hgi.Context(0, hgi.PATH_PER_LEVEL)}
+    ctxs = {"tile": hgi.Context(0, hgi.PATH_TILE)}
     print(f"# Per-config timings, one B200, planes resident in HBM, {args.samples} samples (median / best), "
           f"peak {PEAK:.1f} GB/s measured\n")
     print("| config | L | quant | path | encode us (med/best) | decode us (med/best) | enc+dec Mpixel/s | "
@@ -77,8 +76,6 @@ def main():
             oc.decode(g, levels)
             cpu = npx / (time.perf_counter() - t0) / 1e6
             for pname, ctx in ctxs.items():
-                if pname != "fast tile" and npx > (1 << 27) and pname == "per level":
-                    pass
                 enc = hgi.Encoder(hgi.Crossed, hgi.Linear(hgi.QuantizationLevel(q)), levels, ctx=ctx)
                 dec = hgi.Decoder(hgi.Crossed, ctx=ctx)
                 grid = torch.empty_like(img)

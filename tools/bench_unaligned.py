@@ -24,7 +24,7 @@ def t(fn, n=20):
     return a.elapsed_time(b) / n
 
 
-print("| width | layout | kernel | encode ms | decode ms | enc+dec Mpixel/s |\n|---|---|---|---|---|---|")
+print("| width | layout | encode ms | decode ms | enc+dec Mpixel/s |\n|---|---|---|---|---|")
 for w in (1920, 1916, 1918, 1919, 1000):
     pitch = (w + 15) // 16 * 16
     for layout in ("packed", "rows padded to %d" % pitch):
@@ -37,13 +37,10 @@ for w in (1920, 1916, 1918, 1919, 1000):
             buf = torch.randint(0, 256, (256, 1080, pitch), dtype=torch.uint8, device="cuda")
             frames = buf[:, :, :w]
             g, o = torch.empty_like(buf)[:, :, :w], torch.empty_like(buf)[:, :, :w]
-        for name, path in (("swar", hgi.PATH_TILE), ("generic", hgi.PATH_TILE_GENERIC)):
-            if name == "generic" and layout != "packed":
-                continue
-            ctx = hgi.Context(0, path)
-            enc = hgi.Encoder(hgi.Crossed, hgi.Linear(hgi.QuantizationLevel.Medium), 4, ctx=ctx)
-            dec = hgi.Decoder(hgi.Crossed, ctx=ctx)
-            te = t(lambda: enc.encode_device(frames, grids_out=g))
-            td = t(lambda: dec.decode_device(4, g, images_out=o))
-            print(f"| {w} | {layout} | {name} | {te:.3f} | {td:.3f} | {256 * 1080 * w / (te + td) / 1e3:.0f} |")
-            ctx.close()
+        ctx = hgi.Context(0)
+        enc = hgi.Encoder(hgi.Crossed, hgi.Linear(hgi.QuantizationLevel.Medium), 4, ctx=ctx)
+        dec = hgi.Decoder(hgi.Crossed, ctx=ctx)
+        te = t(lambda: enc.encode_device(frames, grids_out=g))
+        td = t(lambda: dec.decode_device(4, g, images_out=o))
+        print(f"| {w} | {layout} | {te:.3f} | {td:.3f} | {256 * 1080 * w / (te + td) / 1e3:.0f} |")
+        ctx.close()

@@ -11,5 +11,5 @@ name=$1; shift
 out=../../build/$name; mkdir -p $out
 NV="/usr/local/cuda/bin/nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -Xcompiler -fPIC -fmad=false"
 $NV "$@" -c -o $out/hgi_tile_fast.o hgi_tile_fast.cu
-$NV -shared -cudart static -o ../../build/libhgi_$name.so $out/hgi_tile_fast.o hgi_capi.o hgi_tile_kernels.o hgi_level_kernels.o hgi_reduce_kernels.o hgi_region.o hgi_archive.o -lz
+$NV -shared -cudart static -o ../../build/libhgi_$name.so $out/hgi_tile_fast.o hgi_capi.o hgi_reduce_kernels.o hgi_region.o hgi_archive.o -lz
 echo built build/libhgi_$name.so

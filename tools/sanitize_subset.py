@@ -4,7 +4,7 @@
     compute-sanitizer --tool memcheck|racecheck|initcheck python tools/sanitize_subset.py [--light]
 
 Touches every kernel of libhgi_b200.so through the C ABI -- fast tile kernel (interior + edge launches, all level
-counts, aligned / unaligned / pitched planes), generic kernel, per-level kernels, decimated coarse passes,
+counts, aligned / unaligned / pitched planes), decimated coarse passes,
 histogram, RLE token table, RGB->luma, error metrics -- and checks each result against the oracle."""
 import argparse
 import os
@@ -41,7 +41,7 @@ def check(ctx, img, levels, q, interp=hgi.Crossed):
     n_checked += 1
 
 
-paths = {"tile": hgi.PATH_TILE, "generic": hgi.PATH_TILE_GENERIC, "level": hgi.PATH_PER_LEVEL}
+paths = {"tile": hgi.PATH_TILE}
 ctxs = {k: hgi.Context(0, v) for k, v in paths.items()}
 lena = get_plane("lena_tif")
 for name, ctx in ctxs.items():
